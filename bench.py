@@ -26,6 +26,12 @@ parameters (protopformer_b200/synth.py).  Prints ONE JSON line (rank 0).
                timed on this box's host cores on a bounded sample (rank 0, N=1 only).
   --impl reference : that CPU port as its own arm (the reference is pure Python over ATen; /root/reference does not
                exist on the GPU box, so the port stands in: cpu_baseline.kind = "port").
+
+  --dump-outputs DIR  after the timed device-resident steps, writes what the last of them returned to the caller as
+               DIR/<name>.npy (float32): logits, and in training loss, ppc_cov, ppc_mean, dtokens and the parameter
+               gradients grad_P, grad_Pg, grad_Wa, grad_ba (rank 0).  The inputs depend only on the arguments, so two
+               builds run with the same arguments can be compared output for output.  Above DUMP_BYTES in all, the
+               largest arrays are cut to a fixed seeded sample of their leading-dimension rows (the same rows every run).
 """
 from __future__ import annotations
 
@@ -47,6 +53,7 @@ METRIC = "prototype_head_train_images_per_sec"
 METRIC_EVAL = "prototype_head_forward_images_per_sec"
 UNIT = "images/s"
 DEFAULT_WORKLOAD = "cub_b64"    # BASELINE.json configs[1]: deit_tiny CUB shape, training step, batch 64 per GPU
+DUMP_BYTES = 60 * 2 ** 20       # --dump-outputs: data bytes written in all (headroom under 64 MB for the .npy headers)
 
 
 def parse_workload(name: str, mode_flag: str | None):
@@ -167,6 +174,33 @@ def graph_time_us(fn, per_graph: int, replays: int = 10) -> float:
     b.record()
     torch.cuda.synchronize()
     return 1e3 * a.elapsed_time(b) / (replays * per_graph)
+
+
+def step_outputs(step, slot: int, train: bool) -> dict:
+    """Host copies of what a caller of the graphed step receives from the replay just run on `slot`."""
+    out = {"logits": step.logits[slot]}
+    if train:
+        out.update(loss=step.loss[slot], ppc_cov=step.ppc[slot][0], ppc_mean=step.ppc[slot][1], dtokens=step.dtokens[slot])
+        out.update({f"grad_{k}": g for k, g in step.grads.items()})
+    return {k: v.detach().float().cpu() for k, v in out.items()}
+
+
+def dump_outputs(out_dir: str, arrays: dict, budget: int = DUMP_BYTES):
+    """Writes every array as out_dir/<name>.npy (float32), smallest first.  An array larger than an equal share of the
+    budget left keeps a sample of its leading-dimension rows drawn from a fixed seed (sorted, so the same rows of the same
+    shape in every run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    order = sorted(arrays, key=lambda k: arrays[k].numel())
+    for i, name in enumerate(order):
+        t = arrays[name]
+        share = budget // (len(order) - i)
+        if t.dim() > 0 and t.shape[0] > 1 and 4 * t.numel() > share:
+            keep = max(1, share // (4 * (t.numel() // t.shape[0])))
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+        budget -= 4 * t.numel()
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -418,7 +452,13 @@ def main():
                          "available / plain peer pointers) or NCCL")
     ap.add_argument("--eager-allreduce", action="store_true",
                     help="N>1: issue the NCCL gradient all-reduce after each graph replay instead of inside the graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA step: use it with --impl ours")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -515,6 +555,8 @@ def main():
     barrier()
     t_w1 = time.perf_counter()
     sampler.window = (t_w0, t_w1)
+    # copied out now: the legs below replay the step again
+    outputs = step_outputs(step, (args.steps - 1) % nbuf, train) if args.dump_outputs and rank == 0 else None
     ms = ev0.elapsed_time(ev1)
     if world > 1:
         t = torch.tensor([ms], device=dev)
@@ -633,13 +675,12 @@ def main():
                 fstep.run(i % nbuf)
             torch.cuda.synchronize()
             f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            nf = max(200, args.steps // 2)
             f0.record()
-            for i in range(nf):
+            for i in range(args.steps):
                 fstep.run(i % nbuf)
             f1.record()
             torch.cuda.synchronize()
-            fms = f0.elapsed_time(f1) / nf
+            fms = f0.elapsed_time(f1) / args.steps
             ff = step_flops(shape, False)
             forward_only = {"metric": METRIC_EVAL, "value": shape.B / (fms * 1e-3), "unit": UNIT, "ms_per_step": fms,
                             "gpu_launches_per_step": fstep.kernel_launches_per_step,
@@ -661,7 +702,7 @@ def main():
             next_rows = {"error": str(exc)}
         if train:
             try:
-                dropin = measure_dropin(shape, mode, params, step, nbuf, 200)
+                dropin = measure_dropin(shape, mode, params, step, nbuf, args.steps)
             except Exception as exc:
                 dropin = {"error": f"{type(exc).__name__}: {exc}"}
 
@@ -714,6 +755,8 @@ def main():
             "next_rows": next_rows,
             "cpu_baseline": cpu,
         }
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         # graphs that recorded NCCL kernels keep the communicator busy: drop them first, and never let a stuck teardown

@@ -10,17 +10,17 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "multigpu: needs >= 2 CUDA devices on one box (deselected otherwise)")
+    config.addinivalue_line("markers", "multigpu: needs >= 2 CUDA devices on one box (skipped otherwise)")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
     n_dev = torch.cuda.device_count() if torch.cuda.is_available() else 0
-    if n_dev < 2:           # multi-GPU tests are not skipped but left out: a one-GPU box reports no skips
-        gone = [it for it in items if "multigpu" in it.keywords]
-        if gone:
-            items[:] = [it for it in items if "multigpu" not in it.keywords]
-            config.hook.pytest_deselected(items=gone)
+    if n_dev < 2:
+        skip_multi = pytest.mark.skip(reason=f"needs >= 2 CUDA devices ({n_dev} present)")
+        for item in items:
+            if "multigpu" in item.keywords:
+                item.add_marker(skip_multi)
     if torch.cuda.is_available():
         return
     skip = pytest.mark.skip(reason="no CUDA device")

@@ -37,8 +37,11 @@ def test_library_builds_loads_and_exports_every_declared_symbol():
 
 
 def test_sass_contains_blackwell_tensor_and_tma_instructions():
-    from protopformer_b200 import _lib
-    sass = subprocess.run(["cuobjdump", "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    from protopformer_b200 import _lib, build
+    cuobjdump = os.path.join(os.path.dirname(build._nvcc()), "cuobjdump")      # the toolkit that built the library
+    sass = ""
+    if os.path.exists(cuobjdump):
+        sass = subprocess.run([cuobjdump, "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
     if not sass:
         pytest.skip("cuobjdump unavailable")
     for mnemonic in ("UTCHMMA", "UTMALDG", "LDTM"):
@@ -254,6 +257,31 @@ def test_bench_arms_build_identical_config_objects():
     assert not train and shape.D == 384 and mode == "fp32"
     assert bench.parse_workload("cars_b64_bf16", None)[2] == "bf16"
     assert bench.step_flops(shape, False) < bench.step_flops(shape, True)
+
+
+def test_bench_dump_outputs_stays_in_budget_with_a_fixed_row_sample(tmp_path):
+    """--dump-outputs: small arrays are written whole, a large one is cut to the same seeded rows on every call, and the
+    data written stays within the budget."""
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    g = torch.Generator().manual_seed(3)
+    arrays = {"loss": torch.tensor(1.5), "logits": torch.randn(8, 5, generator=g), "dtokens": torch.randn(300, 7, 4, generator=g)}
+    budget = 4 * (1 + 40 + 100 * 28)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays, budget)
+    got = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in arrays}
+    assert got["loss"].dtype == np.float32 and float(got["loss"]) == 1.5
+    assert np.array_equal(got["logits"], arrays["logits"].numpy())
+    assert sum(a.nbytes for a in got.values()) <= budget and 1 <= got["dtokens"].shape[0] < 300
+    assert np.array_equal(got["dtokens"], np.load(tmp_path / "b" / "dtokens.npy"))
+    rows = [int(np.argmax((arrays["dtokens"].numpy() == r).all(axis=(1, 2)))) for r in got["dtokens"]]
+    assert rows == sorted(set(rows))                       # distinct rows of the input, in their original order
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                       timeout=600, cwd=ROOT)
+    assert r.returncode == 2 and "--steps" in r.stderr
 
 
 def test_round2_entry_points_validate_arguments_before_touching_the_device():

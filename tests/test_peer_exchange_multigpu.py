@@ -1,6 +1,6 @@
 """The gradient exchange over peer memory on two ranks of one box (one process per GPU, torch.distributed.run on 127.0.0.1):
 scripts/ddp_check.py holds the graphed step with the exchange recorded in its CUDA graph -- multicast, plain peer pointers
-and NCCL -- to the averaged per-rank gradients of the same step without the exchange.  Collected only where >= 2 GPUs exist."""
+and NCCL -- to the averaged per-rank gradients of the same step without the exchange.  Skipped where fewer than 2 GPUs exist."""
 import os
 import subprocess
 import sys
