@@ -288,7 +288,10 @@ int pph_head_prep(const float* scores, const float* tokens, const float* Wa, con
  * writes losses[0] -- lets the PPC loss overlap the last layers instead of lengthening the launch.  Adding 4 to use_ppc
  * makes dZs_ppc leave as the pre-activation gradient (times Z (1 - Z)): the form pph_addon_bwd3's dpre_add_s takes.
  * workspace: pph_head_mid_ws_bytes() bytes, ZERO-FILLED once before first use (grid-barrier and ticket counters, all
- * self-resetting).  C <= 256; B <= 64 * (SM count / 2).  Out-of-range labels are clamped. */
+ * self-resetting).  C <= 256; B <= 64 * (SM count / 2).  Out-of-range labels are clamped.
+ * When pph_last_layer_pattern, run on the same workspace before this call, found both Wl and Wg in the class-connection
+ * pattern, the last layers take their class-sum form (O(B P) instead of O(B P C), same results up to summation order);
+ * otherwise the general product.  The launch clears the verdicts it used: each call needs a check of its own. */
 int pph_head_mid_ws_bytes(int B, int K, int D, int P, int Pg, int C, int m, long long* bytes /* host */);
 int pph_head_mid(const float* act_l, const float* act_g, const float* dmin_l, const float* dmin_g,
                  const int32_t* argmin_l, const float* Wl, const float* Wg, const int64_t* labels,
@@ -303,6 +306,15 @@ int pph_head_mid(const float* act_l, const float* act_g, const float* dmin_l, co
                                          (total, ce, ppc_cov, ppc_mean) with the same store that completes losses[0]: the
                                          caller's device->host read of the step result without a copy node */,
                  pph_stream_t stream);
+
+/* Device-side check of the last layers Wl [C,P] and Wg [C,Pg] (Wg may be NULL when Pg = 0) against the pattern of
+ * PPNet.set_last_layer_incorrect_connection (protopformer.py:367-386): with m = n / C, W[c,p] == a where p / m == c and
+ * == b elsewhere, a = W[0,0], b = W[1,0] (b = a when C = 1), by exact float equality; n % C != 0 fails.  Writes its
+ * verdicts into the first PPH_LL_PATTERN_BYTES of `workspace` (a pph_head_mid workspace) for the pph_head_mid call that
+ * follows on the stream: two records {int32 ok; float a; float b; int32 unused}, Wl then Wg (Pg = 0: ok, a = b = 0).
+ * One launch, integer atomics only, no host synchronisation -- meant to run inside the captured step, every step. */
+#define PPH_LL_PATTERN_BYTES 32
+int pph_last_layer_pattern(const float* Wl, int P, const float* Wg, int Pg, int C, void* workspace, pph_stream_t stream);
 
 /* (a8 part 2), second implementation: same results as pph_similarity_bwd(PPH_BWD_GRADS) from operands staged in shared
  * memory by feature slices (no L2 row gathers), every row summed in a fixed order (no atomics on data).  Three kernels,

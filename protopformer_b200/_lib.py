@@ -51,6 +51,7 @@ SIGNATURES = {
     "pph_head_prep": [_p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _f] + [_p] * 14 + [_p, _i, _p, _p, _p, _p, _p] * 2 + [_p],
     "pph_head_mid_ws_bytes": [_i, _i, _i, _i, _i, _i, _i, C.POINTER(C.c_longlong)],
     "pph_head_mid": [_p] * 8 + [_i] * 8 + [_f, _i, _f, _f, _i, _i] + [_p] * 5 + [_f] * 4 + [_p] * 14,
+    "pph_last_layer_pattern": [_p, _i, _p, _i, _i, _p, _p],
     "pph_similarity_bwd2_supported": [_i, _i, _i, _i, _i],
     "pph_similarity_bwd2_ws_bytes": [_i, _i, _i, _i, C.POINTER(C.c_longlong)],
     "pph_similarity_bwd2": [_i] + [_p] * 8 + [_i] * 6 + [_p, _p, _i] + [_p] * 5,
@@ -76,7 +77,7 @@ _RESTYPES = {"pph_last_error_string": C.c_char_p}
 KERNELS_PER_CALL = {
     "pph_select_topk": 1, "pph_addon_fwd": 1, "pph_split_rows": 1, "pph_logits_fwd": 1, "pph_ppc_fwd": 1,
     "pph_ppc_bwd": 1, "pph_logits_bwd": 1, "pph_similarity_bwd": 2, "pph_addon_bwd": 3, "pph_loss_tail": 1, "pph_loss_combine": 1, "pph_rollout_scores": 2, "pph_adamw_step": 1, "pph_class_maps": 1, "pph_rollout_cls_rows": 1,
-    "pph_head_prep": 1, "pph_head_mid": 1, "pph_similarity_bwd_fused": 1, "pph_addon_bwd2": 1, "pph_addon_fwd2": 1,
+    "pph_head_prep": 1, "pph_head_mid": 1, "pph_last_layer_pattern": 1, "pph_similarity_bwd_fused": 1, "pph_addon_bwd2": 1, "pph_addon_fwd2": 1,
     "pph_peer_allreduce": 1, "pph_gather_rows_host": 1,
     "pph_ppc_dense_fwd": 1, "pph_ppc_dense_bwd": 1, "pph_select_addon_fwd": 1,
 }

@@ -17,7 +17,17 @@
 //            prototype-gradient kernel walks it row by row).
 // FP32 FMA throughout: 2 x 102 MFLOP at the CUB shape, far too skinny (64 x 200 outputs) for a tensor-core tile
 // grid -- what matters here is that every SM has a CTA and that no intermediate leaves L2.
+//
+// Role LL has a second, class-sum form for last layers that hold the class-connection pattern of
+// set_last_layer_incorrect_connection (protopformer.py:367-386: W[c,p] = a on the prototype's own class p / m, b
+// elsewhere -- the frozen init of every run).  Then logit_c = b T + (a - b) s_c with s_c the sum of class c's m
+// activations and T their total, and (dlogits W)[p] = b sum_c dlogits[c] + (a - b) dlogits[p / m]: O(B P) instead of
+// O(B P C), one CTA per image, no grid barrier.  pph_last_layer_pattern checks both matrices on the device (every
+// step, inside the graph: a host-side decision would go stale after W.data.copy_) and leaves its verdict at the start
+// of the workspace; the launch reads it and runs the class-sum form only when both pass, the three phases otherwise.
 #include <math.h>
+
+#include <algorithm>
 
 #include "pph_bins.cuh"
 #include "pph_common.cuh"
@@ -29,6 +39,20 @@ constexpr int kMidThreads = 256;
 constexpr int kMidTB = 64;       // images per tile
 constexpr int kMidPS = 32;       // prototypes per slice
 constexpr int kMidAST = 68;      // row stride of the [*][64-image] shared tiles (16-byte aligned, 4 mod 32 banks)
+
+// Verdict of pph_last_layer_pattern on one last layer (layout documented at PPH_LL_PATTERN_BYTES in protohead.h).
+struct LLPattern {
+    int ok;          // every entry is a on its own class and b elsewhere (exact float equality)
+    float a, b;
+    int unused;
+};
+// First bytes of the pph_head_mid workspace: the verdicts for Wl and Wg, then the check's own counters.  All zero at
+// first use (ok = 0: the three-phase role); the launch that reads the verdicts clears `ok` again.
+struct LLPatternWs {
+    LLPattern rec[2];
+    unsigned int bad, ticket;
+};
+static_assert(sizeof(LLPattern) * 2 == PPH_LL_PATTERN_BYTES, "protohead.h documents two 16-byte records");
 
 struct MidArgs {
     int B, Bp, K, D, P, Pg, C, Cp, m, N, side;
@@ -47,7 +71,8 @@ struct MidArgs {
     float2* pairT;
     // workspace
     float *part, *dlT, *ce_part, *ppc_part, *ppc_losses;
-    unsigned int* ctr;      // [0] barrier, [1] done, [2] fin, [3] ppc ticket
+    unsigned int* ctr;      // [0] barrier, [1] done, [2] fin, [3] ppc ticket, [4] class-sum LL ticket
+    LLPatternWs* pattern;
     int32_t *bin_start, *item_start, *bin_list;
     int4* item_desc;
     int32_t *cls_id, *cls_start, *cls_item, *cls_order;
@@ -348,6 +373,125 @@ __device__ __forceinline__ void ll_role(const MidArgs& a, float* sm) {
     grid_finish(a.ctr, a.ctr + 1, (unsigned int)a.n_ll);
 }
 
+__device__ __forceinline__ float block_max_mid(float v, float* red) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    __syncthreads();
+    if (lane == 0) red[warp] = v;
+    __syncthreads();
+    float s = red[0];
+#pragma unroll
+    for (int w = 1; w < kMidThreads / 32; ++w) s = fmaxf(s, red[w]);
+    return s;
+}
+
+// g[b,p] of one branch in the class-sum form (and its pairT column when the staged backward wants it)
+__device__ __forceinline__ void ll_class_grad(const MidArgs& a, int b, bool glob, const LLPattern& w, float Sdl,
+                                              const float* dls) {
+    const int np = glob ? a.Pg : a.P, m = np / a.C;
+    const float coef = glob ? a.gc : 1.0f - a.gc;
+    const float* dmin = glob ? a.dmin_g : a.dmin_l;
+    float* gout = glob ? a.g_g : a.g_l;
+    const float bS = w.b * Sdl, amb = w.a - w.b;
+    const size_t row = (size_t)b * np;
+    constexpr int U = 4;            // dmin loads in flight per thread before the first use
+    for (int p0 = threadIdx.x; p0 < np; p0 += U * kMidThreads) {
+        float d[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const int p = p0 + u * kMidThreads;
+            d[u] = p < np ? __ldg(dmin + row + p) : 0.f;
+        }
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const int p = p0 + u * kMidThreads;
+            if (p >= np) break;
+            const float g = coef * fmaf(amb, dls[p / m], bS) * dact_of_dist(d[u], a.act_fn, a.eps);
+            gout[row + p] = g;
+            if (a.pairT)
+                a.pairT[(size_t)(glob ? a.P + p : p) * a.Bp + b] =
+                    make_float2(g, __int_as_float(glob ? a.K : __ldg(a.argmin_l + row + p)));
+        }
+    }
+}
+
+// role LL, class-sum form (both last layers passed pph_last_layer_pattern): LL CTA r takes images r, r + n_ll, ...; a
+// thread owns one class (C <= 256).  Every sum runs in a fixed order (bit-identical replays).  The softmax and the
+// cross-entropy are taken over the class-dependent part of the logits only, z_c = (1-gc)(a_l-b_l) s_l,c +
+// gc (a_g-b_g) s_g,c: the b T terms are the same for every class and cancel, and at ~1e3 they would cost digits.
+__device__ void ll_class_role(const MidArgs& a, const LLPattern& wl, const LLPattern& wg, float* sm) {
+    const int tid = threadIdx.x, c = tid;
+    const int B = a.B, C = a.C, ml = a.P / C, mg = a.Pg / C;
+    float* dls = sm;                  // [256] dlogits of the image
+    float* zs = dls + kMidThreads;    // [256] class-dependent logits
+    float* red = zs + kMidThreads;    // [8]
+    const float kl = (1.0f - a.gc) * (wl.a - wl.b), kg = a.gc * (wg.a - wg.b);
+    for (int b = blockIdx.x; b < B; b += a.n_ll) {
+        float sl = 0.f, sg = 0.f;
+        if (c < C) {
+            const float* rl = a.act_l + (size_t)b * a.P + (size_t)c * ml;
+            const float* rg = a.act_g + (size_t)b * a.Pg + (size_t)c * mg;
+            for (int j = 0; j < ml; ++j) sl += __ldg(rl + j);
+            for (int j = 0; j < mg; ++j) sg += __ldg(rg + j);
+        }
+        const float Tl = block_sum_mid(sl, red), Tg = block_sum_mid(sg, red);
+        const float z = c < C ? fmaf(kl, sl, kg * sg) : -INFINITY;
+        zs[c] = z;
+        if (c < C) {
+            const float lv = fmaf(wl.a - wl.b, sl, wl.b * Tl), gv = fmaf(wg.a - wg.b, sg, wg.b * Tg);
+            a.logits_l[(size_t)b * C + c] = lv;
+            a.logits_g[(size_t)b * C + c] = gv;
+            a.logits[(size_t)b * C + c] = a.gc * gv + (1.0f - a.gc) * lv;
+        }
+        const float mx = block_max_mid(z, red);       // its barriers also publish zs[]
+        const float e = c < C ? expf(z - mx) : 0.f;
+        const float se = block_sum_mid(e, red);
+        long y = a.labels[b];
+        if (y < 0) y = 0;
+        if (y >= C) y = C - 1;
+        if (tid == 0) a.ce_part[b] = logf(se) + mx - zs[y];
+        if (a.train) {
+            const float dl = c < C ? (e / se - (c == (int)y ? 1.0f : 0.0f)) * (a.upstream / (float)B) : 0.f;
+            if (c < C) a.dlogits[(size_t)b * C + c] = dl;
+            dls[c] = dl;
+            const float Sdl = block_sum_mid(dl, red);      // its barriers also publish dls[]
+            ll_class_grad(a, b, false, wl, Sdl, dls);
+            ll_class_grad(a, b, true, wg, Sdl, dls);
+        }
+        __syncthreads();                                  // zs / dls / red are reused by the next image
+    }
+    if (a.train && a.pairT) {        // columns of the padded images are zeros, as the three-phase role writes them
+        for (int b = a.B + blockIdx.x; b < a.Bp; b += a.n_ll)
+            for (int p = tid; p < a.P + a.Pg; p += kMidThreads) a.pairT[(size_t)p * a.Bp + b] = make_float2(0.f, 0.f);
+    }
+    // every LL CTA takes the ticket (it read the verdicts first); the last one forms the batch mean of the CE terms in
+    // the same fixed order as the three-phase role and clears the verdicts: the next launch without a fresh check
+    // falls back to the general product
+    __shared__ int last;
+    __syncthreads();
+    if (tid == 0) {
+        __threadfence();
+        last = atomicAdd(a.ctr + 4, 1u) == (unsigned int)a.n_ll - 1u;
+        if (last) {
+            __threadfence();
+            a.pattern->rec[0].ok = 0;
+            a.pattern->rec[1].ok = 0;
+            a.ctr[4] = 0u;
+        }
+    }
+    __syncthreads();
+    if (last) {
+        float v = 0.f;
+        for (int i = tid; i < B; i += kMidThreads) v += __ldcg(a.ce_part + i);
+        const float ce = block_sum_mid(v, red) / (float)B;
+        if (tid == 0) {
+            a.losses[1] = ce;
+            role_finished(a);
+        }
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // role PPC: forward (restatement of SURVEY.md 8(d)(iii), same arithmetic as pph_ppc.cu) + backward in one CTA per image
 // ---------------------------------------------------------------------------------------------------------------
@@ -539,7 +683,11 @@ head_mid_kernel(const MidArgs a) {
     extern __shared__ __align__(16) float sm_mid[];
     const int bid = blockIdx.x;
     if (bid < a.n_ll) {
-        ll_role<CJ>(a, sm_mid);
+        // one decision for the whole grid: the verdicts were written by an earlier launch and change only in this
+        // launch's last class-sum CTA, after every LL CTA has read them
+        const LLPattern wl = a.pattern->rec[0], wg = a.pattern->rec[1];
+        if (wl.ok && wg.ok) ll_class_role(a, wl, wg, sm_mid);
+        else ll_role<CJ>(a, sm_mid);
     } else if (bid < a.n_ll + a.n_bin) {
         bin_tokens_body<false>(bid - a.n_ll, a.argmin_l, a.K, a.P, a.bin_start, a.item_start, a.bin_list,
                         reinterpret_cast<int*>(sm_mid), a.item_desc);
@@ -607,6 +755,7 @@ static MidPlan mid_plan(int B, int K, int D, int P, int Pg, int C, int m, int ma
 }
 
 struct MidWs {
+    LLPatternWs* pattern;
     unsigned int* ctr;
     float *part, *dlT, *ce_part, *ppc_part, *ppc_losses;
     size_t bytes;
@@ -617,7 +766,9 @@ static MidWs mid_carve(void* base, const MidPlan& p, int B) {
     char* q = static_cast<char*>(base);
     size_t off = 0;
     auto take = [&](size_t n) { char* r = q ? q + off : nullptr; off += (n + 255) / 256 * 256; return r; };
-    w.ctr = reinterpret_cast<unsigned int*>(take(sizeof(int) * 8));        // first: the part that must start zeroed
+    // first: the part that must start zeroed (pph_last_layer_pattern finds its records at offset 0 without the plan)
+    w.pattern = reinterpret_cast<LLPatternWs*>(take(sizeof(LLPatternWs)));
+    w.ctr = reinterpret_cast<unsigned int*>(take(sizeof(int) * 8));
     w.ppc_losses = reinterpret_cast<float*>(take(sizeof(float) * 2));
     w.ce_part = reinterpret_cast<float*>(take(sizeof(float) * (size_t)B));
     w.ppc_part = reinterpret_cast<float*>(take(sizeof(float) * 2 * (size_t)B));
@@ -632,7 +783,86 @@ static int mid_max_ctas() {
     return n > 0 ? n : 148;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// pph_last_layer_pattern: is W[c,p] == (p / m == c ? W[0,0] : W[1,0]) for every entry of a (C, n) matrix, m = n / C?
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int kPatThreads = 256, kPatVecPerThread = 4;
+
+// 1 if this thread's share of W holds an entry off the pattern.  vec4: n % 4 == 0 and W 16-byte aligned, so a float4
+// never straddles two rows.
+__device__ __forceinline__ unsigned int pattern_scan(const float* __restrict__ W, int C, int n, bool vec4) {
+    if (n == 0) return 0u;
+    if (n % C != 0) return 1u;
+    const int m = n / C, total = C * n;
+    const float a = __ldg(W), b = C > 1 ? __ldg(W + n) : a;
+    const int t0 = blockIdx.x * blockDim.x + threadIdx.x, stride = gridDim.x * blockDim.x;
+    bool bad = false;
+    if (vec4) {
+        const float4* W4 = reinterpret_cast<const float4*>(W);
+#pragma unroll 4
+        for (int i = t0; i < total / 4; i += stride) {
+            const float4 v = __ldg(W4 + i);
+            const int e = 4 * i, c = e / n, p = e - c * n;
+            bad |= v.x != ((p / m == c) ? a : b);
+            bad |= v.y != (((p + 1) / m == c) ? a : b);
+            bad |= v.z != (((p + 2) / m == c) ? a : b);
+            bad |= v.w != (((p + 3) / m == c) ? a : b);
+        }
+    } else {
+#pragma unroll 4
+        for (int e = t0; e < total; e += stride) {
+            const int c = e / n, p = e - c * n;
+            bad |= __ldg(W + e) != ((p / m == c) ? a : b);
+        }
+    }
+    return bad ? 1u : 0u;
+}
+
+__device__ __forceinline__ LLPattern pattern_record(const float* W, int C, int n, bool bad) {
+    LLPattern r;
+    r.ok = !bad;
+    r.a = n > 0 ? W[0] : 0.f;
+    r.b = n > 0 ? (C > 1 ? W[n] : r.a) : 0.f;
+    r.unused = 0;
+    return r;
+}
+
+// Integer flags only: CTAs that saw a mismatch OR a bit into `bad`; the last CTA to take the ticket writes both
+// verdicts and resets the counters (self-resetting under graph replay, no host sync).
+__global__ void __launch_bounds__(kPatThreads)
+last_layer_pattern_kernel(const float* __restrict__ Wl, int P, int vec_l, const float* __restrict__ Wg, int Pg, int vec_g,
+                          int C, LLPatternWs* ws) {
+    pdl_sync();
+    const unsigned int bits = pattern_scan(Wl, C, P, vec_l) | (pattern_scan(Wg, C, Pg, vec_g) << 1);
+    const int bad_l = __syncthreads_or(bits & 1u), bad_g = __syncthreads_or(bits & 2u);
+    if (threadIdx.x != 0) return;
+    if (bad_l || bad_g) atomicOr(&ws->bad, (bad_l ? 1u : 0u) | (bad_g ? 2u : 0u));
+    __threadfence();
+    if (atomicAdd(&ws->ticket, 1u) != gridDim.x - 1u) return;
+    __threadfence();
+    const unsigned int all = atomicExch(&ws->bad, 0u);
+    ws->rec[0] = pattern_record(Wl, C, P, all & 1u);
+    ws->rec[1] = pattern_record(Wg, C, Pg, all & 2u);
+    ws->ticket = 0u;
+}
+
 }  // namespace pph
+
+extern "C" int pph_last_layer_pattern(const float* Wl, int P, const float* Wg, int Pg, int C, void* workspace,
+                                      pph_stream_t stream) {
+    using namespace pph;
+    PPH_REQUIRE(Wl && workspace && (Pg == 0 || Wg), PPH_EINVAL, "pph_last_layer_pattern: null pointer");
+    PPH_REQUIRE(P >= 1 && Pg >= 0 && C >= 1, PPH_EINVAL, "pph_last_layer_pattern: bad dims");
+    PPH_REQUIRE((long long)C * P < (1LL << 31) && (long long)C * Pg < (1LL << 31), PPH_EUNSUP,
+                "pph_last_layer_pattern: C x P = %lld entries", (long long)C * (P > Pg ? P : Pg));
+    auto vec4 = [](const float* W, int n) { return (n % 4 == 0 && (reinterpret_cast<uintptr_t>(W) & 15) == 0) ? 1 : 0; };
+    const int vl = vec4(Wl, P), vg = vec4(Wg, Pg);
+    const int per_cta = kPatThreads * kPatVecPerThread * 4;             // entries a CTA covers with one pass
+    const int ctas = std::min(mid_max_ctas(), std::max(1, ceil_div(C * std::max(P, Pg), per_cta)));
+    launch_k(last_layer_pattern_kernel, dim3(ctas), dim3(kPatThreads), 0, as_stream(stream), Wl, P, vl, Wg, Pg, vg, C,
+             static_cast<LLPatternWs*>(workspace));
+    return launch_status("pph_last_layer_pattern");
+}
 
 extern "C" int pph_head_mid_ws_bytes(int B, int K, int D, int P, int Pg, int C, int m, long long* bytes) {
     using namespace pph;
@@ -691,6 +921,7 @@ extern "C" int pph_head_mid(const float* act_l, const float* act_g, const float*
     a.g_l = g_l; a.g_g = g_g; a.pairT = reinterpret_cast<float2*>(pairT);
     a.part = w.part; a.dlT = w.dlT; a.ce_part = w.ce_part; a.ppc_part = w.ppc_part; a.ppc_losses = w.ppc_losses;
     a.ctr = w.ctr;
+    a.pattern = w.pattern;
     a.bin_start = a.item_start = a.bin_list = nullptr;
     a.item_desc = nullptr;
     a.cls_id = a.cls_start = a.cls_item = a.cls_order = nullptr;

@@ -1,7 +1,7 @@
 """Static-shape training / inference step of the prototype head captured in CUDA graphs.
 
 At the CUB shape the whole head costs tens of microseconds on a B200, i.e. it is launch-bound from Python; the
-idiomatic B200 answer is to record the step once (forward + PPC loss + cross-entropy + backward, 10 kernels) and
+idiomatic B200 answer is to record the step once (forward + PPC loss + cross-entropy + backward, 11 kernels) and
 replay it.  The step goes through exactly the public operators of ``ops`` (nothing is bypassed), reads its inputs
 from static device buffers ("slots") and leaves its results in static tensors:
 
@@ -72,7 +72,7 @@ class GraphedHeadStep:
         if fused:
             # one set of intermediate buffers shared by all slots (replays are serial on one stream)
             D, P, Pg = params["Wa"].shape[0], params["P"].shape[0], params["Pg"].shape[0]
-            # impl: "v2" = the round-2 launch sequence (10 launches), "v1" = the round-1 sequence (fallback / A-B arm), "auto" = v2 if the
+            # impl: "v2" = the round-2 launch sequence (11 launches), "v1" = the round-1 sequence (fallback / A-B arm), "auto" = v2 if the
             # shape is inside what those kernels were built for
             if impl == "auto":
                 impl = "v2" if ops.fused_step_supported(B, N, Din, D, cfg.K, P, Pg, C, m) else "v1"

@@ -708,13 +708,15 @@ def fused_step_supported(B, N, Din, D, K, P, Pg, C, m) -> bool:
 
 
 class FusedHeadStep:
-    """forward (+ PPC + cross-entropy + backward) of the head for a fixed shape: 10 launches over the current stream and two
+    """forward (+ PPC + cross-entropy + backward) of the head for a fixed shape: 11 launches over the current stream and two
     side branches (default variants; DESIGN.md section 4.0):
 
       pph_select_addon_fwd      selection + gather + add-on + sigmoid + bf16 operands (tcgen05, single shot)
         || pph_split_rows x2    bf16 operands / norms of both prototype tensors, memset of dtokens           (side branch)
+        || pph_last_layer_pattern  do Wl, Wg still hold the class-connection pattern? (verdict for pph_head_mid)
       pph_similarity_fwd        tcgen05 distances, log similarity, min / argmin over tokens (the (B,P,K) map stays in TMEM)
-      pph_head_mid (LL)         last layers + cross-entropy + last-layer backward, token bins, class lists
+      pph_head_mid (LL)         last layers (class-sum form when the verdict allows) + cross-entropy + last-layer backward,
+                                token bins, class lists
         || pph_head_mid (PPC)   PPC loss forward + backward                                        [training, side branch]
       pph_similarity_bwd_fused  argmin-routed gradients: dP, dPg, pre-activation gradients of the tokens      [training]
         || ppc rows add         PPC prototype rows onto dP                                          [training, side branch]
@@ -786,7 +788,7 @@ class FusedHeadStep:
         self.ws_tc = _ws("pph_addon_tc2_ws_bytes", B, N, Din, D, K, zero=True, device=device)
         self.side = torch.cuda.Stream(device=device)
         self.side2 = torch.cuda.Stream(device=device)
-        self.ev = [torch.cuda.Event() for _ in range(8)]
+        self.ev = [torch.cuda.Event() for _ in range(9)]
         self.dlogits = self.g_l = self.g_g = self.pairT = self.ws_bins = None
         self.dZs_ppc = self.dP_img = None
         if train:
@@ -820,6 +822,13 @@ class FusedHeadStep:
         c = _lib.call
         main, side, side2, ev = torch.cuda.current_stream(), self.side, self.side2, self.ev
         hook = reduce_hook or (lambda which: None)
+
+        def last_layer_pattern():
+            # do both last layers still hold the class-connection pattern?  Decided on the device every step (a weight
+            # copy through .data leaves no trace on the host); pph_head_mid reads the verdict (joined through ev[8])
+            c("pph_last_layer_pattern", Wl, Pn, Wg, Pgn, C, self.ws_mid)
+            ev[8].record(side)
+
         if self.variants["prep"] in ("tc", "tc1"):
             # selection -> tcgen05 add-on || operand split of both prototype tensors (side branch)
             ev[3].record(main)
@@ -830,6 +839,7 @@ class FusedHeadStep:
                 if self.train and self.variants["addon_bwd"] == "tc":
                     self.dtokens.zero_()            # rows of unselected tokens: a memset node off the critical path
                 ev[4].record(side)
+                last_layer_pattern()
             if self.variants["prep"] == "tc1":
                 if idx32 is None:
                     c("pph_select_topk", scores, B, max(H, 1), N, K, sel_idx, None)
@@ -849,12 +859,13 @@ class FusedHeadStep:
                   self.Zc_hi, self.Zc_lo, self.ws_tc)
             main.wait_event(ev[4])
         else:
-            if self.train and self.variants["addon_bwd"] == "tc":
-                ev[3].record(main)
-                side.wait_event(ev[3])
-                with torch.cuda.stream(side):
+            ev[3].record(main)
+            side.wait_event(ev[3])
+            with torch.cuda.stream(side):
+                if self.train and self.variants["addon_bwd"] == "tc":
                     self.dtokens.zero_()
                     ev[4].record(side)
+                last_layer_pattern()
             c("pph_head_prep", scores, tokens, Wa, ba, B, max(H, 1), N, Din, D, K, float(cfg.center), sel_idx, None,
               self.Zs, self.Zc, self.z2s, self.z2c, self.z2s_ctr, self.z2c_ctr, self.z2s_hi, self.z2c_hi,
               self.Zs_hi, self.Zs_lo, self.Zc_hi, self.Zc_lo,
@@ -863,6 +874,7 @@ class FusedHeadStep:
             if self.train and self.variants["addon_bwd"] == "tc":
                 main.wait_event(ev[4])
         if self.stop_after == 1:
+            main.wait_event(ev[8])
             return self.losses
         mode = cfg.mode_id
         sel = {_lib.MODE_FP32_FMA: 0, _lib.MODE_BF16X3: 1, _lib.MODE_BF16: 2}[mode]
@@ -872,6 +884,7 @@ class FusedHeadStep:
           (self.p2, self.p2_ctr, self.p2_hi)[sel], (self.pg2, self.pg2_ctr, self.pg2_hi)[sel],
           self.P_hi, self.P_lo, self.Pg_hi, self.Pg_lo,
           self.dmin_l, self.argmin, self.act_l, self.dmin_g, self.act_g, None, None)
+        main.wait_event(ev[8])
         if self.stop_after == 2:
             return self.losses
         ppc = self.use_ppc and self.train
