@@ -150,6 +150,18 @@ int pph_logits_bwd(const float* dlogits, const float* dlogits_g, const float* dl
                    int B, int P, int Pg, int C, float global_coe, int act_fn, float eps,
                    float* g_l, float* g_g, pph_stream_t stream);
 
+/* Weight gradients of the last layers, for callers that unfreeze them (the reference freezes them, protopformer.py:130-131,
+ * but its autograd would train them once `requires_grad` is set; main.py:370 then averages them with the rest): the
+ * derivative of protopformer.py:297-300 / 314-316 w.r.t. Wl and Wg,
+ *   dWl[c,p] = sum_b ((1-gc) dlogits[b,c] + dlogits_l[b,c]) act_l[b,p]      dWg[c,p] = sum_b (gc dlogits[b,c] + dlogits_g[b,c]) act_g[b,p]
+ * dlogits [B,C] (upstream gradient of the combined logits), dlogits_g / dlogits_l [B,C] or NULL (no upstream gradient on
+ * logits_global / logits_local), act_l [B,P], act_g [B,Pg] (pph_similarity_fwd).  dWl [C,P], dWg [C,Pg] are OVERWRITTEN;
+ * either may be NULL (not computed).  Every entry is one fixed-order sum over b (no atomics: bit-reproducible); the kernel
+ * never waits on another CTA, so it may share the device with the step's co-resident kernels.  B, P, C >= 1; no bound on C. */
+int pph_last_layer_wgrad(const float* dlogits, const float* dlogits_g, const float* dlogits_l,
+                         const float* act_l, const float* act_g, int B, int P, int Pg, int C, float global_coe,
+                         float* dWl, float* dWg, pph_stream_t stream);
+
 /* (a8, part 2) max-pool routing + distance backward (SURVEY.md 8(d)(iv)):
  *   dPl[p,:]   = 2 * sum_b g_l[b,p] * (Pl[p,:] - Zs[b,argmin[b,p],:])      dPg[p,:] = 2 * sum_b g_g[b,p] * (Pg[p,:] - Zc[b,:])
  *   dZs[b,k,:] = 2 * sum_{p: argmin[b,p]=k} g_l[b,p] * (Zs[b,k,:] - Pl[p,:])   dZc[b,:] = 2 * sum_p g_g[b,p] * (Zc[b,:] - Pg[p,:])

@@ -35,6 +35,7 @@ SIGNATURES = {
     "pph_ppc_fwd": [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _p, _p, _p, _p, _p, _p],
     "pph_ppc_bwd": [_p, _p, _p, _p, _p, _p, _p, _f, _f, _i, _i, _i, _i, _i, _i, _i, _f, _f, _f, _i, _p, _p, _p],
     "pph_logits_bwd": [_p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _f, _i, _f, _p, _p, _p],
+    "pph_last_layer_wgrad": [_p] * 5 + [_i] * 4 + [_f] + [_p] * 3,
     "pph_similarity_bwd_ws_bytes": [_i, _i, _i, _i, _i, C.POINTER(C.c_longlong)],
     "pph_similarity_bwd": [_p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _i, _p, _p, _p, _p, _p, _p, _p],
     "pph_loss_tail": [_p, _p, _p, _f, _f, _f, _i, _i, _p, _p, _p, _p, _p],
@@ -76,7 +77,7 @@ _RESTYPES = {"pph_last_error_string": C.c_char_p}
 # kernels launched per entry-point call (memset nodes are not counted); used for the bench's `gpu_launches` claim
 KERNELS_PER_CALL = {
     "pph_select_topk": 1, "pph_addon_fwd": 1, "pph_split_rows": 1, "pph_logits_fwd": 1, "pph_ppc_fwd": 1,
-    "pph_ppc_bwd": 1, "pph_logits_bwd": 1, "pph_similarity_bwd": 2, "pph_addon_bwd": 3, "pph_loss_tail": 1, "pph_loss_combine": 1, "pph_rollout_scores": 2, "pph_adamw_step": 1, "pph_class_maps": 1, "pph_rollout_cls_rows": 1,
+    "pph_ppc_bwd": 1, "pph_logits_bwd": 1, "pph_last_layer_wgrad": 1, "pph_similarity_bwd": 2, "pph_addon_bwd": 3, "pph_loss_tail": 1, "pph_loss_combine": 1, "pph_rollout_scores": 2, "pph_adamw_step": 1, "pph_class_maps": 1, "pph_rollout_cls_rows": 1,
     "pph_head_prep": 1, "pph_head_mid": 1, "pph_last_layer_pattern": 1, "pph_similarity_bwd_fused": 1, "pph_addon_bwd2": 1, "pph_addon_fwd2": 1,
     "pph_peer_allreduce": 1, "pph_gather_rows_host": 1,
     "pph_ppc_dense_fwd": 1, "pph_ppc_dense_bwd": 1, "pph_select_addon_fwd": 1,

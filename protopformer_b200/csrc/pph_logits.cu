@@ -1,6 +1,7 @@
 // (a6) prototype-to-class last layers + global/local combine (protopformer.py:297-300, 314-316) and the first
 // step of their backward, collapsed with the similarity derivative into one scalar per (image, prototype).
-// The last layers are frozen in the reference (protopformer.py:130-131) -> no weight gradient is produced.
+// The last layers are frozen in the reference (protopformer.py:130-131); a caller that unfreezes them gets their weight
+// gradients from pph_last_layer_wgrad (bottom of this file).
 //
 // Both are skinny FP32 contractions (B x C x (P+Pg) with B = 64): too small for a tensor-core tile grid, so they are
 // laid out for L2 traffic and determinism instead:
@@ -8,6 +9,7 @@
 //             register accumulators per thread, one block reduction -> every logit has ONE writer (deterministic).
 //   backward: transposed product G^T = W^T * upstream^T on tcgen05 through the manual-fill GEMM (pph_tcgemm.cuh).
 #include "pph_common.cuh"
+#include "pph_sgemm.cuh"
 #include "pph_tcgemm.cuh"
 
 namespace pph {
@@ -190,6 +192,49 @@ logits_bwd_fma_kernel(const float* __restrict__ dlogits, const float* __restrict
         }
 }
 
+// ---- last-layer weight gradients: dW[c,p] = sum_b (coef dlogits[b,c] + extra[b,c]) act[b,p], coef = 1-gc (local) | gc
+// (global).  ONE FP32 tile GEMM (pph_sgemm.cuh) over both layers: rows = classes, columns [0, nl) the local prototypes
+// (nl = P rounded up to the 64-wide column tile, so each CTA belongs to one layer), [nl, nl + Pg) the global ones,
+// contraction over the B images NOT split -> every entry is one fixed-order sum, no atomics (bit-reproducible).
+// Skinny-K (K = B) and bounded by the 4 C (P+Pg) bytes of output.
+struct LwAOp {      // (row = c, k = b) -> upstream gradient of the layer this CTA's columns belong to
+    static constexpr bool kContigK = false;
+    const float *dlogits, *dlogits_g, *dlogits_l;
+    int C, nl;
+    float gc;
+    __device__ __forceinline__ float operator()(int c, int b) const {
+        if (c >= C) return 0.f;
+        const bool global = (int)blockIdx.x * kGemmBN >= nl;
+        const float* extra = global ? dlogits_g : dlogits_l;
+        const size_t o = (size_t)b * C + c;
+        float x = (global ? gc : 1.0f - gc) * __ldg(dlogits + o);
+        if (extra) x += __ldg(extra + o);
+        return x;
+    }
+};
+// ng = Pg when dWg is computed, else 0: the loader's tail columns past the last requested one never touch act_g (which
+// may then be NULL)
+struct LwBOp {      // (row = column n, k = b) -> act[b, p]; consecutive columns are consecutive prototypes
+    static constexpr bool kContigK = false;
+    const float *act_l, *act_g;
+    int P, Pg, ng, nl;
+    __device__ __forceinline__ float operator()(int n, int b) const {
+        const bool global = n >= nl;
+        const int p = global ? n - nl : n;
+        if (p >= (global ? ng : P)) return 0.f;
+        return __ldg((global ? act_g : act_l) + (size_t)b * (global ? Pg : P) + p);
+    }
+};
+struct LwEpi {
+    float *dWl, *dWg;
+    int P, Pg, ng, nl;
+    __device__ __forceinline__ void operator()(int c, int n, float acc, float) const {
+        const bool global = n >= nl;
+        const int p = global ? n - nl : n;
+        if (p < (global ? ng : P)) (global ? dWg : dWl)[(size_t)c * (global ? Pg : P) + p] = acc;
+    }
+};
+
 }  // namespace pph
 
 extern "C" int pph_logits_fwd(const float* act_l, const float* act_g, const float* Wl, const float* Wg,
@@ -227,4 +272,27 @@ extern "C" int pph_logits_bwd(const float* dlogits, const float* dlogits_g, cons
     LbEpi e{dmin_l, dmin_g, g_l, g_g, B, P, Plpad, Pg, act_fn, eps};
     const int N = ceil_div(B, 2) * 2;           // the kernel walks columns in pairs
     return launch_tcgemm(Plpad + Pg, N, C, tcgemm_pick_bn(N), 1, a, b, e, as_stream(stream), "pph_logits_bwd(tcgen05)");
+}
+
+extern "C" int pph_last_layer_wgrad(const float* dlogits, const float* dlogits_g, const float* dlogits_l,
+                                    const float* act_l, const float* act_g, int B, int P, int Pg, int C, float global_coe,
+                                    float* dWl, float* dWg, pph_stream_t stream) {
+    using namespace pph;
+    PPH_REQUIRE(B >= 1 && P >= 1 && Pg >= 0 && C >= 1, PPH_EINVAL, "pph_last_layer_wgrad: bad dims");
+    if (Pg == 0) dWg = nullptr;                  // no global layer: nothing to write
+    PPH_REQUIRE((!dWl && !dWg) || dlogits, PPH_EINVAL, "pph_last_layer_wgrad: null pointer (dlogits)");
+    PPH_REQUIRE(!dWl || act_l, PPH_EINVAL, "pph_last_layer_wgrad: null pointer (act_l for dWl)");
+    PPH_REQUIRE(!dWg || act_g, PPH_EINVAL, "pph_last_layer_wgrad: null pointer (act_g for dWg)");
+    if (!dWl && !dWg) return 0;
+    const int nl = dWl ? (dWg ? ceil_div(P, kGemmBN) * kGemmBN : P) : 0;
+    const int ng = dWg ? Pg : 0;
+    LwAOp a{dlogits, dlogits_g, dlogits_l, C, nl, global_coe};
+    LwBOp b{act_l, act_g, P, Pg, ng, nl};
+    LwEpi e{dWl, dWg, P, Pg, ng, nl};
+    // maximum shared-memory carve-out, as every kernel of the training step asks for (pph_common.cuh, opt_in_smem): this
+    // launch runs on a branch beside the step's co-resident kernels
+    const cudaError_t err = opt_in_smem(sgemm_kernel<false, LwAOp, LwBOp, LwEpi>, 0);
+    PPH_REQUIRE(err == cudaSuccess, (int)err, "pph_last_layer_wgrad: %s", cudaGetErrorString(err));
+    launch_sgemm<false>(C, nl + ng, B, 1, a, b, e, as_stream(stream));
+    return launch_status("pph_last_layer_wgrad");
 }

@@ -1,10 +1,11 @@
 """Data-parallel plumbing of the head: one process per GPU, batch sharded, head parameters replicated.
 
 The only exchange step of the path is the gradient all-reduce of the trainable head parameters
-(`prototype_vectors`, `prototype_vectors_global`, `add_on_layers.*`; the last layers are frozen,
-protopformer.py:130-131) -- what DDP does implicitly in the reference (main.py:370).  Here the gradients of those
-parameters are views into ONE flat fp32 buffer, so a step issues a single NCCL all-reduce (3.2 MB at the CUB shape,
-latency-bound over NVLink/NVSwitch) on the backward stream right behind the prototype-gradient kernel.
+(`prototype_vectors`, `prototype_vectors_global`, `add_on_layers.*`, and `last_layer.weight` /
+`last_layer_global.weight` when the caller unfreezes them -- the reference freezes them, protopformer.py:130-131) --
+what DDP does implicitly in the reference (main.py:370).  Here the gradients of those parameters are views into ONE flat
+fp32 buffer (3.2 MB at the CUB shape, +3.2 MB with both last layers unfrozen), averaged over the ranks in segments
+that the graphed step exchanges as soon as each is final (latency-bound over NVLink/NVSwitch).
 """
 from __future__ import annotations
 
@@ -13,8 +14,10 @@ import torch.distributed as dist
 
 
 def head_parameters(module):
-    """Trainable head parameters in a fixed order (names follow tools/create_optimizer.py:31-39)."""
-    names = ["prototype_vectors", "prototype_vectors_global", "add_on_layers.0.weight", "add_on_layers.0.bias"]
+    """Trainable head parameters in a fixed order (names follow tools/create_optimizer.py:31-39); the last layers follow
+    the four others, and only when their weight requires grad (frozen by default, protopformer.py:130-131)."""
+    names = ["prototype_vectors", "prototype_vectors_global", "add_on_layers.0.weight", "add_on_layers.0.bias",
+             "last_layer.weight", "last_layer_global.weight"]
     params = dict(module.named_parameters())
     return [(n, params[n]) for n in names if n in params and params[n].requires_grad]
 

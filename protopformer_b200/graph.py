@@ -34,7 +34,9 @@ class GraphedHeadStep:
                  schedule: int | None = None, use_ppc: bool = True, impl: str = "auto", variants=None,
                  exchange: str = "nccl"):
         """params: dict with Wa (D,Din), ba (D), P (P,D), Pg (Pg,D) [leaf tensors, requires_grad in training] and
-        the frozen Wl (C,P), Wg (C,Pg).  ppc_*_coe follow scripts/train_cub.sh:43-44."""
+        the last layers Wl (C,P), Wg (C,Pg), frozen as in the reference unless their requires_grad is set: a training step
+        then also writes their gradients (appended to the flat buffer behind ba, Wl before Wg).  ppc_*_coe follow
+        scripts/train_cub.sh:43-44."""
         self.p, self.cfg, self.B, self.N, self.C, self.m = params, cfg, B, N, C, m
         self.train = train
         self.cov_coe, self.mean_coe = ppc_cov_coe, ppc_mean_coe
@@ -51,7 +53,9 @@ class GraphedHeadStep:
         self.graphs = [None] * n_slots
         self.reducer = None
         if train:
+            # unfrozen last layers go last: the existing segments keep their offsets and ("Wl", "Wg") is contiguous
             named = [(k, params[k]) for k in ("P", "Pg", "Wa", "ba")]
+            named += [(k, params[k]) for k in ("Wl", "Wg") if params[k].requires_grad]
             # exchange: "nccl" = NCCL all-reduce of the flat buffer, "peer" / "peer_nomc" = the library's own one-kernel
             # all-reduce over peer-mapped memory (with / without the NVLS multicast mapping)
             self.exchange, self.exchange_note = exchange, ""
@@ -82,28 +86,36 @@ class GraphedHeadStep:
             self.fused = cls(cfg, B, N, Din, D, P, Pg, C, m, dev, heads=heads, ppc_cov_coe=ppc_cov_coe,
                              ppc_mean_coe=ppc_mean_coe, train=train, use_ppc=use_ppc, schedule=schedule, **kw)
             if train:
-                self.grads = dict(zip(("P", "Pg", "Wa", "ba"), self.reducer.views))
+                self.grads = dict(zip((n for n, _ in self.reducer.named), self.reducer.views))
 
     # --------------------------------------------------------------------------------------------------------
     def _step_fused(self, slot: int, **extra):
         p, f = self.p, self.fused
         works = []
         hook = None
+        last, aligned = False, True
         if self.train and self.allreduce_in_graph and self.impl == "v2":
             # overlapped exchange: the prototype gradients (95 % of the flat buffer) are final before the add-on backward
             # starts, so their all-reduce is issued there (on the step's side branch) and runs under those kernels on
             # NCCL's stream; the add-on part follows the weight-gradient kernel.  Both join the step's stream below.
             seg = {"protos": self.reducer.segment(("P", "Pg")), "addon": self.reducer.segment(("Wa", "ba"))}
+            # unfrozen last layers: a third exchange ("last", peer slot 2) on their own branch, right behind their kernel
+            last = any(n in ("Wl", "Wg") for n, _ in self.reducer.named)
+            if last:
+                seg["last"] = self.reducer.segment(("Wl", "Wg"))
 
             aligned = all(v % 4 == 0 for v in seg["protos"])
+            if last:
+                aligned = aligned and all(v % 4 == 0 for v in seg["addon"])
 
             def hook(which):
                 lo, hi = seg[which]
                 if not aligned:           # odd sizes: one exchange of the whole buffer after the last gradient
-                    if which == "protos":
-                        return
+                    if which == "protos" or last:
+                        return            # (with the last-layer branch: below, once the step has joined it)
                     lo, hi = 0, None
-                w = self.reducer.allreduce(async_op=True, lo=lo, hi=hi, check=False, slot=0 if which == "protos" else 1)
+                peer_slot = {"protos": 0, "addon": 1, "last": 2}[which]
+                w = self.reducer.allreduce(async_op=True, lo=lo, hi=hi, check=False, slot=peer_slot)
                 if w is not None:
                     works.append(w)
         with torch.no_grad():
@@ -113,7 +125,7 @@ class GraphedHeadStep:
                    p["Wl"], p["Wg"], self.grads if self.train else None, **kw)
         for w in works:
             w.wait()                      # the capturing / current stream waits for NCCL's stream
-        if self.train and self.allreduce_in_graph and hook is None:
+        if self.train and self.allreduce_in_graph and (hook is None or (last and not aligned)):
             self.reducer.allreduce(check=False)
         self.loss[slot] = f.losses[0]
         self.logits[slot] = f.logits

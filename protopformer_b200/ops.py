@@ -300,7 +300,8 @@ def _similarity_raw(cfg: HeadConfig, tf: TokenFeatures, pl: ProtoOperands, pg: P
 
 
 class _SimilarityLogits(torch.autograd.Function):
-    """(Zs, Zc, P, Pg) -> logits.  Wl / Wg are the frozen last layers (protopformer.py:130-131): no gradient."""
+    """(Zs, Zc, P, Pg, Wl, Wg) -> logits.  Wl / Wg are frozen in the reference (protopformer.py:130-131); one that requires
+    grad gets its weight gradient from pph_last_layer_wgrad (the frozen default saves nothing extra and launches nothing)."""
 
     @staticmethod
     @torch.amp.custom_fwd(device_type="cuda", cast_inputs=torch.float32)
@@ -316,7 +317,8 @@ class _SimilarityLogits(torch.autograd.Function):
         logits = _empty((B, C), torch.float32, Zs)
         logits_g, logits_l = torch.empty_like(logits), torch.empty_like(logits)
         _lib.call("pph_logits_fwd", act_l, act_g, Wl, Wg, B, P, Pg, C, float(cfg.global_coe), logits, logits_g, logits_l)
-        ctx.save_for_backward(Zs, Zc, pl.P, pg.P, Wl, Wg, dmin_l, dmin_g, argmin)
+        want_w = ctx.needs_input_grad[4] or ctx.needs_input_grad[5]
+        ctx.save_for_backward(Zs, Zc, pl.P, pg.P, Wl, Wg, dmin_l, dmin_g, argmin, *((act_l, act_g) if want_w else ()))
         ctx.cfg = cfg
         ctx.mark_non_differentiable(act_l, act_g, dmin_l, dmin_g, argmin, pl.p2)
         return logits, logits_g, logits_l, act_l, act_g, dmin_l, dmin_g, argmin, pl.p2
@@ -324,7 +326,7 @@ class _SimilarityLogits(torch.autograd.Function):
     @staticmethod
     @torch.amp.custom_bwd(device_type="cuda")
     def backward(ctx, dlogits, dlogits_g, dlogits_l, *_unused):
-        Zs, Zc, Pl, Pgl, Wl, Wg, dmin_l, dmin_g, argmin = ctx.saved_tensors
+        Zs, Zc, Pl, Pgl, Wl, Wg, dmin_l, dmin_g, argmin, *acts = ctx.saved_tensors
         cfg = ctx.cfg
         B, K, D = Zs.shape
         P, Pg, C = Pl.shape[0], Pgl.shape[0], Wl.shape[0]
@@ -342,7 +344,13 @@ class _SimilarityLogits(torch.autograd.Function):
         ws = bwd_workspace(B, K, D, P, Pg, Zs.device)
         _lib.call("pph_similarity_bwd", g_l, g_g, argmin, Zs, Zc, Pl, Pgl, B, K, D, P, Pg, ws, 3, None, None,
                   dZs, dZc, dPl, dPg)
-        return dZs, dZc, dPl, dPg, None, None, None, None
+        dWl = torch.empty_like(Wl) if ctx.needs_input_grad[4] else None
+        dWg = torch.empty_like(Wg) if ctx.needs_input_grad[5] and Pg > 0 else None
+        if dWl is not None or dWg is not None:
+            act_l, act_g = acts
+            _lib.call("pph_last_layer_wgrad", dlogits, dlogits_g, dlogits_l, act_l, act_g, B, P, Pg, C,
+                      float(cfg.global_coe), dWl, dWg)
+        return dZs, dZc, dPl, dPg, dWl, dWg, None, None
 
 
 def addon_bwd_workspace(B, N, Din, D, K, device) -> torch.Tensor:
@@ -526,6 +534,20 @@ def ppc_loss_dense(cfg: HeadConfig, total_proto_act: torch.Tensor, cls_attn_roll
 # Fused training / inference step: the same entry points in a fixed sequence over pre-allocated buffers, no autograd
 # graph and no PyTorch glue kernels in between (what tools/engine_proto.py:49-76 amounts to for the head).
 # ------------------------------------------------------------------------------------------------------------------
+def _last_layer_grad_targets(train: bool, Wl, Wg, grads):
+    """(dWl, dWg) the training step writes, None for a frozen layer.  A last layer is trained iff its weight requires grad
+    (the reference's switch, protopformer.py:130-131); its gradient is OVERWRITTEN in grads["Wl"] / grads["Wg"]."""
+    if not train:
+        return None, None
+    out = []
+    for k, W in (("Wl", Wl), ("Wg", Wg)):
+        g = (grads or {}).get(k) if W.requires_grad else None
+        if W.requires_grad and g is None:
+            raise ValueError(f"the {k} last layer requires grad: pass grads[{k!r}] for the step to write its gradient into")
+        out.append(g)
+    return tuple(out)
+
+
 class FusedHeadStepV1:
     """Round-1 launch sequence (16 launches over three streams), kept as the fallback for shapes the round-2 step (FusedHeadStep)
     was not built for and as an A/B arm.  forward (+ PPC + cross-entropy + backward) of the head for a fixed shape.
@@ -535,7 +557,8 @@ class FusedHeadStepV1:
       [logits_bwd, similarity_bwd, ppc_bwd(accumulate), addon_bwd]
     Results live in attributes: losses (4,) = (total, ce, ppc_cov, ppc_mean), logits, logits_g, logits_l, act_l,
     dmin_l, argmin, idx32, dtokens; parameter gradients are OVERWRITTEN in the tensors of `grads`
-    (keys Wa, ba, P, Pg -- e.g. views of one flat all-reduce buffer)."""
+    (keys Wa, ba, P, Pg -- e.g. views of one flat all-reduce buffer -- and Wl / Wg for a last layer whose weight requires
+    grad: pph_last_layer_wgrad right after the loss tail)."""
 
     def __init__(self, cfg: HeadConfig, B, N, Din, D, P, Pg, C, m, device, heads: int = 0, ppc_cov_coe: float = 0.1,
                  ppc_mean_coe: float = 0.5, train: bool = True, use_ppc: bool = True, schedule: int | None = None):
@@ -662,6 +685,10 @@ class FusedHeadStepV1:
               float(upstream), B, C, self.ce_partial, self.ce_counter, self.losses, self.dlogits if self.train else None)
         if not self.train:
             return self.losses
+        dWl, dWg = _last_layer_grad_targets(self.train, Wl, Wg, grads)
+        if dWl is not None or dWg is not None:
+            c("pph_last_layer_wgrad", self.dlogits, None, None, self.act_l, self.act_g, B, Pn, Pgn, C,
+              float(cfg.global_coe), dWl, dWg)
         c("pph_logits_bwd", self.dlogits, None, None, Wl, Wg, self.dmin_l, self.dmin_g, B, Pn, Pgn, C,
           float(cfg.global_coe), cfg.act_id, float(cfg.eps), self.g_l, self.g_g)
         binned = ppc                                   # bins were produced on a side stream next to the PPC loss
@@ -718,6 +745,7 @@ class FusedHeadStep:
       pph_head_mid (LL)         last layers (class-sum form when the verdict allows) + cross-entropy + last-layer backward,
                                 token bins, class lists
         || pph_head_mid (PPC)   PPC loss forward + backward                                        [training, side branch]
+        || pph_last_layer_wgrad dWl, dWg (+ their exchange)        [training with an unfrozen last layer, own branch]
       pph_similarity_bwd_fused  argmin-routed gradients: dP, dPg, pre-activation gradients of the tokens      [training]
         || ppc rows add         PPC prototype rows onto dP                                          [training, side branch]
       pph_addon_bwd3 x2         dtokens, then dWa | dba (tcgen05, single shot)                                [training]
@@ -727,7 +755,8 @@ class FusedHeadStep:
 
     Same results interface as FusedHeadStepV1: losses (4,) = (total, ce, ppc_cov, ppc_mean), logits, logits_g, logits_l,
     act_l, dmin_l, argmin, idx32, dtokens; parameter gradients are OVERWRITTEN in the tensors of `grads`
-    (keys Wa, ba, P, Pg -- e.g. views of one flat all-reduce buffer).  Reference: tools/engine_proto.py:49-76."""
+    (keys Wa, ba, P, Pg -- e.g. views of one flat all-reduce buffer -- and Wl / Wg for a last layer whose weight requires
+    grad; with both frozen, the default, the step is exactly the 11 launches above).  Reference: tools/engine_proto.py:49-76."""
 
     def __init__(self, cfg: HeadConfig, B, N, Din, D, P, Pg, C, m, device, heads: int = 0, ppc_cov_coe: float = 0.1,
                  ppc_mean_coe: float = 0.5, train: bool = True, use_ppc: bool = True, schedule=None, variants=None):
@@ -789,6 +818,8 @@ class FusedHeadStep:
         self.side = torch.cuda.Stream(device=device)
         self.side2 = torch.cuda.Stream(device=device)
         self.ev = [torch.cuda.Event() for _ in range(9)]
+        self.side_ll = torch.cuda.Stream(device=device)         # last-layer weight gradients (unfrozen last layers only)
+        self.ev_ll = [torch.cuda.Event() for _ in range(2)]
         self.dlogits = self.g_l = self.g_g = self.pairT = self.ws_bins = None
         self.dZs_ppc = self.dP_img = None
         if train:
@@ -810,7 +841,8 @@ class FusedHeadStep:
              idx32=None, loss_mirror=None):
         """reduce_hook(which): called once with "protos" when grads["P"], grads["Pg"] are final (on the stream that
         produced them) and once with "addon" after grads["Wa"], grads["ba"]: the data-parallel caller issues its
-        asynchronous all-reduces there so that the first one overlaps the add-on backward.
+        asynchronous all-reduces there so that the first one overlaps the add-on backward.  With an unfrozen last layer
+        also once with "last", on the last-layer branch right after grads["Wl"] / grads["Wg"] are written.
         idx32: the ascending selected-token list (B,K) if the caller already ranked this batch's scores (the
         selection-first host transfer does): the step then skips its own selection launch and `self.idx32` is not
         updated.  loss_mirror: address of 4 floats (16-byte aligned, e.g. mapped pinned host memory) that receive
@@ -912,9 +944,27 @@ class FusedHeadStep:
                 main.wait_event(ev[1])
         else:
             mid(1 if ppc else 0)
+        dWl, dWg = _last_layer_grad_targets(self.train, Wl, Wg, grads)
+        train_ll = dWl is not None or dWg is not None
+        if train_ll:
+            # last-layer weight gradients need only dlogits (final after the LL role above) and act_l / act_g: their own
+            # branch beside the similarity backward, joined at the end -- the critical path never waits for it
+            self.ev_ll[0].record(main)
+            self.side_ll.wait_event(self.ev_ll[0])
+            with torch.cuda.stream(self.side_ll):
+                c("pph_last_layer_wgrad", self.dlogits, None, None, self.act_l, self.act_g, B, Pn, Pgn, C,
+                  float(cfg.global_coe), dWl, dWg)
+                hook("last")
+                self.ev_ll[1].record(self.side_ll)
+
+        def join_ll():
+            if train_ll:
+                main.wait_event(self.ev_ll[1])
+
         if not self.train or self.stop_after == 3:
             if late:
                 main.wait_event(ev[6])
+            join_ll()
             return self.losses
 
         def gather(parts, add, dpi):
@@ -958,6 +1008,7 @@ class FusedHeadStep:
                 hook("protos")
         if self.stop_after == 4:
             main.wait_event(ev[1])
+            join_ll()
             return self.losses
         if vr["addon_bwd"] == "tc":
             if late:
@@ -989,4 +1040,5 @@ class FusedHeadStep:
               self.ws_addon, grads["Wa"], grads["ba"], self.dtokens)
             hook("addon")
         main.wait_event(ev[1])
+        join_ll()
         return self.losses

@@ -23,6 +23,8 @@ MAX_TENSORS = 8
 def head_param_groups(ppnet, lrs: dict, weight_decay: float):
     """The head's part of ``split_weights`` (tools/create_optimizer.py:31-39): add-on layers with their own lr and a
     fixed 1e-3 weight decay, the two prototype tensors with the prototype lr and the optimizer-level weight decay.
+    Last layers whose weight requires grad (frozen by default, protopformer.py:130-131) form one more group with
+    ``lrs["last_layer"]`` and no weight decay, as ProtoPNet's last-layer optimizer.
     (The ``features`` group -- the backbone -- is outside this path.)"""
     groups = [{"params": list(ppnet.add_on_layers.parameters()), "lr": lrs["add_on_layers"], "weight_decay": 1e-3}]
     if hasattr(ppnet, "prototype_vectors"):
@@ -31,6 +33,12 @@ def head_param_groups(ppnet, lrs: dict, weight_decay: float):
     if hasattr(ppnet, "prototype_vectors_global"):
         groups.append({"params": [ppnet.prototype_vectors_global], "lr": lrs["prototype_vectors"],
                        "weight_decay": weight_decay})
+    last = [layer.weight for layer in (getattr(ppnet, "last_layer", None), getattr(ppnet, "last_layer_global", None))
+            if layer is not None and layer.weight.requires_grad]
+    if last:
+        if "last_layer" not in lrs:
+            raise KeyError("lrs['last_layer'] is missing: the last layers require grad, so they need a learning rate")
+        groups.append({"params": last, "lr": lrs["last_layer"], "weight_decay": 0.0})
     return groups
 
 

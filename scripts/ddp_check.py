@@ -1,6 +1,8 @@
 """N ranks, one per GPU: the step with the gradient all-reduce recorded inside the CUDA graph (overlapped with the
 add-on backward) must leave, on every rank, the average of the per-rank gradients of the same step run without the
-exchange.  Launch:  python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 scripts/ddp_check.py"""
+exchange.  Launch:  python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 scripts/ddp_check.py
+[--train-last-layers] [peer|peer_nomc|nccl ...]
+--train-last-layers unfreezes Wl and Wg: their gradients join the flat buffer and the step's third exchange ("last")."""
 import os
 import sys
 
@@ -17,6 +19,8 @@ def main():
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     dist.init_process_group("nccl", device_id=dev)
+    args = [a for a in sys.argv[1:] if a != "--train-last-layers"]
+    train_ll = len(args) != len(sys.argv) - 1
     shape = synth.SHAPES["cub_b64"]
     case = synth.make_case(shape, seed=1)
     batch = synth.make_case(shape, seed=50 + rank)
@@ -25,7 +29,7 @@ def main():
 
     def make(in_graph, exchange="nccl"):
         params = {k: case[k].to(dev) for k in ("Wa", "ba", "P", "Pg", "Wl", "Wg")}
-        for k in ("Wa", "ba", "P", "Pg"):
+        for k in ("Wa", "ba", "P", "Pg") + (("Wl", "Wg") if train_ll else ()):
             params[k].requires_grad_(True)
         st = GraphedHeadStep(params, cfg, B=shape.B, N=shape.N, C=shape.C, m=shape.m, n_slots=2,
                              allreduce_in_graph=in_graph, exchange=exchange)
@@ -40,7 +44,7 @@ def main():
     torch.cuda.synchronize()
     want = local_step.reducer.flat.clone()
     dist.all_reduce(want, op=dist.ReduceOp.AVG)
-    for exchange in (sys.argv[1:] or ["peer", "peer_nomc", "nccl"]):
+    for exchange in (args or ["peer", "peer_nomc", "nccl"]):
         graphed = make(True, exchange)
         for i in range(50):                       # repeated replays: no hang, no drift
             graphed.run(i % 2)
@@ -59,6 +63,13 @@ def main():
         print(f"rank {rank}/{world} [{graphed.exchange}]: in-graph exchange vs averaged local gradients: {err:.3e} "
               f"(vs own gradients {own:.3e}); {1e3 * ev[0].elapsed_time(ev[1]) / 500:.1f} us/step", flush=True)
         assert err < 1e-6, err
+        if train_ll:
+            lo, hi = graphed.reducer.segment(("Wl", "Wg"))
+            assert hi - lo == case["Wl"].numel() + case["Wg"].numel()
+            err_ll = float((got[lo:hi] - want[lo:hi]).abs().max() / want[lo:hi].abs().max())
+            own_ll = float((got[lo:hi] - local_step.reducer.flat[lo:hi]).abs().max() / want[lo:hi].abs().max())
+            print(f"rank {rank}/{world} [{graphed.exchange}]: last layers {err_ll:.3e} (vs own {own_ll:.3e})", flush=True)
+            assert err_ll < 1e-6 and own_ll > 1e-3, (err_ll, own_ll)
         assert own > 1e-3, "ranks hold different batches: the averaged gradient must differ from the local one"
         if os.environ.get("PPH_TIMELINE") and rank != 0:
             for i in range(6):                # every rank replays: the exchange is a cross-rank barrier
