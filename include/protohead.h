@@ -436,6 +436,57 @@ int pph_peer_allreduce(const unsigned long long* buf_ptrs /* host */, unsigned l
                        long long flag_offset_bytes, int rank, int world, long long lo, long long n,
                        int n_ctas, int slot, pph_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------------------------------
+ * bf16 backbone tokens.  A backbone that runs in bf16 hands the head (B, 1+N, Din) bf16 tokens; these twins of the
+ * entry points that read tokens take them as they are (uint16_t storage, row-major, the same [B,1+N,Din] layout) and
+ * write the token gradient in bf16.  Every bf16 value is exact in fp32: the kernels widen each token at its load and
+ * nothing after the load changes, so every output equals, bit for bit, the fp32 twin's on the widened tokens, and
+ * dtokens equals the fp32 twin's dtokens rounded once to nearest-even (fp32 accumulation, one rounding at the store).
+ * Arguments, workspaces, plans, launch counts and *_supported() answers are the fp32 twin's; in addition every bf16 entry
+ * needs Din % 8 == 0 (rows are read in 16-byte groups) and returns PPH_EINVAL otherwise, before touching a device.
+ * ------------------------------------------------------------------------------------------------------------------ */
+int pph_addon_fwd_bf16tok(const uint16_t* tokens, const int32_t* idx32, const float* Wa, const float* ba,
+                          int B, int N, int Din, int D, int K,
+                          float* Zs, float* Zc, float* z2s, float* z2c,
+                          float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                          uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo, pph_stream_t stream);
+/* dtokens [B,1+N,Din] bf16 (pph_addon_bwd_ws_bytes sizes the workspace) */
+int pph_addon_bwd_bf16tok(const uint16_t* tokens, const int32_t* idx32, const float* Wa,
+                          const float* Zs, const float* Zc, const float* dZs, const float* dZc,
+                          int B, int N, int Din, int D, int K, void* workspace, int parts,
+                          float* dWa, float* dba, uint16_t* dtokens, pph_stream_t stream);
+int pph_addon_fwd2_bf16tok(const uint16_t* tokens, const int32_t* idx32, const float* Wa, const float* ba,
+                           int B, int N, int Din, int D, int K,
+                           float* Zs, float* Zc, float* z2s, float* z2c,
+                           float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                           uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                           void* workspace, pph_stream_t stream);
+int pph_select_addon_fwd_bf16tok(const float* scores /* [B,H,N] fp32 */, int H, const uint16_t* tokens, const float* Wa,
+                                 const float* ba, int B, int N, int Din, int D, int K, int32_t* idx32 /* out */,
+                                 float* Zs, float* Zc, float* z2s, float* z2c,
+                                 float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                                 uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                                 void* workspace, pph_stream_t stream);
+int pph_addon_bwd3_bf16tok(int parts, const uint16_t* tokens, const int32_t* idx32, const float* Wa,
+                           const float* dpre_s, const float* dpre_c, const float* dpre_add_s,
+                           int B, int N, int Din, int D, int K, void* workspace,
+                           float* dWa, float* dba, uint16_t* dtokens, pph_stream_t stream);
+int pph_head_prep_bf16tok(const float* scores, const uint16_t* tokens, const float* Wa, const float* ba,
+                          int B, int H, int N, int Din, int D, int K, float center,
+                          int32_t* idx32, int64_t* idx64,
+                          float* Zs, float* Zc, float* z2s, float* z2c, float* z2s_ctr, float* z2c_ctr,
+                          float* z2s_hi, float* z2c_hi, uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                          const float* Pl, int P, uint16_t* Pl_hi, uint16_t* Pl_lo, float* p2l, float* p2l_ctr, float* p2l_hi,
+                          const float* Pgl, int Pg, uint16_t* Pg_hi, uint16_t* Pg_lo, float* p2g, float* p2g_ctr, float* p2g_hi,
+                          pph_stream_t stream);
+int pph_addon_bwd2_bf16tok(int parts, const uint16_t* tokens, const int32_t* idx32, const float* Wa,
+                           const float* dpre_s, const float* dpre_c,
+                           int B, int N, int Din, int D, int K, void* workspace,
+                           float* dWa, float* dba, uint16_t* dtokens, pph_stream_t stream);
+/* pinned-host bf16 tokens -> tokens_dev bf16: half the bytes of pph_gather_rows_host over the bus. */
+int pph_gather_rows_host_bf16tok(const uint16_t* tokens_host, const int32_t* idx32, int B, int N, int Din, int K,
+                                 uint16_t* tokens_dev, int n_ctas, pph_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -72,6 +72,11 @@ SIGNATURES = {
     "pph_peer_flag_bytes": [C.POINTER(C.c_longlong)],
     "pph_peer_allreduce": [_p, C.c_ulonglong, C.c_longlong, _i, _i, C.c_longlong, C.c_longlong, _i, _i, _p],
 }
+# bf16-token twins of the entry points that read tokens (include/protohead.h): same arguments, bf16 token buffers
+BF16TOK = "_bf16tok"
+BF16TOK_TWINS = ("pph_addon_fwd", "pph_addon_bwd", "pph_addon_fwd2", "pph_select_addon_fwd", "pph_addon_bwd3",
+                 "pph_head_prep", "pph_addon_bwd2", "pph_gather_rows_host")
+SIGNATURES.update({n + BF16TOK: SIGNATURES[n] for n in BF16TOK_TWINS})
 _RESTYPES = {"pph_last_error_string": C.c_char_p}
 
 # kernels launched per entry-point call (memset nodes are not counted); used for the bench's `gpu_launches` claim
@@ -144,18 +149,19 @@ def call(name: str, *args):
     conv = [(C.cast(a, C.c_void_p) if isinstance(a, C.Array) else a) for a in conv]      # host pointer tables
     rc = getattr(lib, name)(*conv, _stream())
     global _launches
-    if name == "pph_similarity_fwd":
+    base = name[:-len(BF16TOK)] if name.endswith(BF16TOK) else name      # a twin launches what its fp32 entry launches
+    if base == "pph_similarity_fwd":
         _launches += 2 if conv[0] == MODE_FP32_FMA else 1      # local + global kernels vs one fused tcgen05 kernel
-    elif name == "pph_similarity_bwd":
+    elif base == "pph_similarity_bwd":
         _launches += (1 if conv[13] & 1 else 0) + (1 if conv[13] & 2 else 0)
-    elif name == "pph_similarity_bwd2":
+    elif base == "pph_similarity_bwd2":
         _launches += bin(conv[0] & 7).count("1")
-    elif name == "pph_addon_bwd3":
+    elif base == "pph_addon_bwd3":
         _launches += bin(conv[0] & 3).count("1")
-    elif name == "pph_addon_bwd":
+    elif base == "pph_addon_bwd":
         _launches += (2 if conv[13] & 1 else 0) + (1 if conv[13] & 2 else 0)
     else:
-        _launches += KERNELS_PER_CALL.get(name, 0)
+        _launches += KERNELS_PER_CALL.get(base, 0)
     if rc != 0:
         msg = lib.pph_last_error_string()
         raise RuntimeError(f"{name} failed (rc={rc}): {msg.decode() if msg else ''}")

@@ -17,8 +17,9 @@ namespace pph {
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kAddBM = 32, kAddBN = 192, kAddBK = 16, kAddThreads = 256;
 
+template <class T>
 __global__ void __launch_bounds__(kAddThreads)
-addon_fwd_kernel(const float* __restrict__ tokens, const int32_t* __restrict__ idx, const float* __restrict__ Wa,
+addon_fwd_kernel(const T* __restrict__ tokens, const int32_t* __restrict__ idx, const float* __restrict__ Wa,
                  const float* __restrict__ ba, int B, int N, int Din, int D, int K,
                  float* __restrict__ Zs, float* __restrict__ Zc, float* __restrict__ z2s, float* __restrict__ z2c,
                  float center, float* __restrict__ z2s_ctr, float* __restrict__ z2c_ctr,
@@ -60,7 +61,7 @@ addon_fwd_kernel(const float* __restrict__ tokens, const int32_t* __restrict__ i
                 for (int i = 0; i < 2; ++i) {
                     const int row = r + 16 * i;
                     const long so = src_off[row];
-                    As[k][row] = (so >= 0 && k0 + k < Din) ? __ldg(tokens + so + k0 + k) : 0.f;
+                    As[k][row] = (so >= 0 && k0 + k < Din) ? ldg_tok(tokens + so + k0 + k) : 0.f;
                 }
                 // W tile: 16 k x 192 n   (Wa is [D, Din], k contiguous)
 #pragma unroll
@@ -200,16 +201,17 @@ struct DpreOp {
 };
 
 // gathered source token rows as a (row = din, k = r) operand
+template <class T>
 struct XselOp {
     static constexpr bool kContigK = false;
-    const float* tokens;
+    const T* tokens;
     const int32_t* idx;
     int B, N, Din, K, R;
     __device__ __forceinline__ float operator()(int din, int r) const {
         if (r >= R || din >= Din) return 0.f;
         const int b = r / (K + 1), j = r - b * (K + 1);
         const int tok = j < K ? 1 + __ldg(idx + (size_t)b * K + j) : 0;
-        return __ldg(tokens + ((size_t)b * (1 + N) + tok) * Din + din);
+        return ldg_tok(tokens + ((size_t)b * (1 + N) + tok) * Din + din);
     }
 };
 
@@ -222,14 +224,15 @@ struct WgradEpi {   // split-K accumulation of dWa and dba
     }
 };
 
+template <class T>
 struct DxEpi {      // scatter of the token gradient rows
-    float* dtokens;
+    T* dtokens;
     const int32_t* idx;
     int N, Din, K;
     __device__ __forceinline__ void operator()(int r, int n, float acc, float) const {
         const int b = r / (K + 1), j = r - b * (K + 1);
         const int tok = j < K ? 1 + __ldg(idx + (size_t)b * K + j) : 0;
-        dtokens[((size_t)b * (1 + N) + tok) * Din + n] = acc;
+        st_tok(dtokens + ((size_t)b * (1 + N) + tok) * Din + n, acc);
     }
 };
 
@@ -254,6 +257,107 @@ wgrad_reduce_kernel(const float* __restrict__ part, int splits, int D, int Din, 
 static bool addon_tc_ok(int Din, int D) { return Din % 8 == 0 && D % 8 == 0 && Din >= 8 && D >= 16; }
 static int wgrad_splits(int R) { int s = ceil_div(R, 2 * kTgBK); return s < 1 ? 1 : (s > 64 ? 64 : s); }
 
+template <class T>
+static int addon_fwd_impl(const char* name, const T* tokens, const int32_t* idx32, const float* Wa, const float* ba,
+                          int B, int N, int Din, int D, int K,
+                          float* Zs, float* Zc, float* z2s, float* z2c,
+                          float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                          uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                          pph_stream_t stream) {
+    PPH_REQUIRE(tokens && idx32 && Wa && ba && Zs && Zc && z2s && z2c, PPH_EINVAL, "%s: null pointer", name);
+    PPH_REQUIRE(B >= 0 && N >= 1 && Din >= 1 && D >= 1 && K >= 1 && K <= N, PPH_EINVAL,
+                "%s: bad dims B=%d N=%d Din=%d D=%d K=%d", name, B, N, Din, D, K);
+    PPH_REQUIRE(sizeof(T) == 4 || Din % 8 == 0, PPH_EINVAL, "%s: bf16 tokens need Din %% 8 == 0 (Din=%d)", name, Din);
+    if (B == 0) return 0;
+    const int R = B * (K + 1);
+    if (addon_tc_ok(Din, D)) {
+        RowSrc src{idx32, B, N, Din, K, R};
+        FwdAOp<T> a{tokens, src};
+        FwdBOp b{Wa, D, Din};
+        FwdEpi e{ba, Zs, Zc, z2s, z2c, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, center, K, D};
+        return launch_tcgemm(R, D, Din, tcgemm_pick_bn(D), 1, a, b, e, as_stream(stream), "pph_addon_fwd(tcgen05)");
+    }
+    launch_k(addon_fwd_kernel<T>, dim3(ceil_div(R, kAddBM)), dim3(kAddThreads), (size_t)(0), as_stream(stream), tokens, idx32, Wa, ba, B, N, Din, D, K, Zs, Zc, z2s, z2c, center, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo);
+    return launch_status(name);
+}
+
+template <class T>
+static int addon_bwd_impl(const char* name, const T* tokens, const int32_t* idx32, const float* Wa,
+                          const float* Zs, const float* Zc, const float* dZs, const float* dZc,
+                          int B, int N, int Din, int D, int K, void* workspace, int parts,
+                          float* dWa, float* dba, T* dtokens, pph_stream_t stream) {
+    PPH_REQUIRE((parts & 3) != 0, PPH_EINVAL, "%s: parts must include PPH_ADDON_WGRAD and/or PPH_ADDON_DGRAD", name);
+    if (!(parts & PPH_ADDON_DGRAD)) dtokens = nullptr;
+    const bool want_w = (parts & PPH_ADDON_WGRAD) != 0;
+    PPH_REQUIRE(tokens && idx32 && Wa && Zs && Zc && dZs && dZc && (!want_w || (dWa && dba)), PPH_EINVAL,
+                "%s: null pointer", name);
+    PPH_REQUIRE(B >= 0 && N >= 1 && Din >= 1 && D >= 1 && K >= 1 && K <= N, PPH_EINVAL,
+                "%s: bad dims B=%d N=%d Din=%d D=%d K=%d", name, B, N, Din, D, K);
+    PPH_REQUIRE(sizeof(T) == 4 || Din % 8 == 0, PPH_EINVAL, "%s: bf16 tokens need Din %% 8 == 0 (Din=%d)", name, Din);
+    cudaStream_t st = as_stream(stream);
+    const bool tc = addon_tc_ok(Din, D) && B > 0;
+    cudaError_t e = cudaSuccess;
+    if (!tc && want_w) {
+        e = cudaMemsetAsync(dWa, 0, sizeof(float) * (size_t)D * Din, st);
+        if (e == cudaSuccess) e = cudaMemsetAsync(dba, 0, sizeof(float) * (size_t)D, st);
+    }
+    if (e == cudaSuccess && dtokens)
+        e = cudaMemsetAsync(dtokens, 0, sizeof(T) * (size_t)B * (1 + N) * Din, st);
+    if (e != cudaSuccess) {
+        set_error("%s: memset: %s", name, cudaGetErrorString(e));
+        return (int)e;
+    }
+    if (B == 0) return 0;
+    const int R = B * (K + 1);
+    if (tc) {
+        PPH_REQUIRE(workspace || !want_w, PPH_EINVAL, "%s: null workspace (size it with pph_addon_bwd_ws_bytes)", name);
+        RowSrc src{idx32, B, N, Din, K, R};
+        if (want_w) {   // dWa / dba: [D x (Din+1)] = dpre^T [D x R] * [Xsel | 1]^T, split over r, partials + ordered reduction
+            const int ldn = ceil_div(Din + 1, 4) * 4;
+            int splits = wgrad_splits(R);
+            const int k_per_split = ceil_div(ceil_div(R, splits), kTgBK) * kTgBK;
+            splits = ceil_div(R, k_per_split);
+            float* part = static_cast<float*>(workspace);
+            DpreColOp a{Zs, Zc, dZs, dZc, K, D, R};
+            XselColOp<T> b{tokens, src};
+            WgradPartEpi epi{part, D, ldn};
+            int rc = launch_tcgemm(D, ldn, R, tcgemm_pick_bn(ldn), splits, a, b, epi, st, "pph_addon_bwd(wgrad tcgen05)");
+            if (rc) return rc;
+            launch_k(wgrad_reduce_kernel, dim3(ceil_div(D * (Din + 1), 256)), dim3(256), (size_t)(0), st, part, splits, D, Din, ldn, dWa, dba);
+            rc = launch_status("pph_addon_bwd(wgrad reduce)");
+            if (rc) return rc;
+        }
+        if (dtokens) {   // dX [R x Din] = dpre [R x D] * Wa [D x Din]
+            DpreRowOp a{Zs, Zc, dZs, dZc, K, D, R};
+            WaTOp b{Wa, D, Din};
+            DxTcEpi<T> epi{dtokens, src};
+            int rc = launch_tcgemm(R, Din, D, tcgemm_pick_bn(Din), 1, a, b, epi, st, "pph_addon_bwd(dgrad tcgen05)");
+            if (rc) return rc;
+        }
+        return 0;
+    }
+    RowMap map{B, K, D};
+    if (want_w) {   // dWa[d, din] = sum_r dpre[r,d] * X[r,din];  dba[d] = sum_r dpre[r,d]   (split over r)
+        DpreOp<true> a{Zs, Zc, dZs, dZc, map, R};
+        XselOp<T> b{tokens, idx32, B, N, Din, K, R};
+        WgradEpi epi{dWa, dba, Din};
+        const int tiles = ceil_div(D, kGemmBM) * ceil_div(Din, kGemmBN);
+        int splits = ceil_div(2 * 148, tiles);
+        launch_sgemm<true>(D, Din, R, splits, a, b, epi, st);
+        int rc = launch_status("pph_addon_bwd(wgrad)");
+        if (rc) return rc;
+    }
+    if (dtokens) {   // dX[r, din] = sum_d dpre[r,d] * Wa[d,din]  -> scattered into the zero-filled token gradient
+        DpreOp<false> a{Zs, Zc, dZs, dZc, map, R};
+        StridedOp<false> b{Wa, Din, 1, Din};       // (row = din, k = d) -> Wa[d*Din + din]
+        DxEpi<T> epi{dtokens, idx32, N, Din, K};
+        launch_sgemm<false>(R, Din, D, 1, a, b, epi, st);
+        int rc = launch_status("pph_addon_bwd(dgrad)");
+        if (rc) return rc;
+    }
+    return 0;
+}
+
 }  // namespace pph
 
 extern "C" int pph_addon_fwd(const float* tokens, const int32_t* idx32, const float* Wa, const float* ba,
@@ -262,21 +366,18 @@ extern "C" int pph_addon_fwd(const float* tokens, const int32_t* idx32, const fl
                              float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
                              uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
                              pph_stream_t stream) {
-    PPH_REQUIRE(tokens && idx32 && Wa && ba && Zs && Zc && z2s && z2c, PPH_EINVAL, "pph_addon_fwd: null pointer");
-    PPH_REQUIRE(B >= 0 && N >= 1 && Din >= 1 && D >= 1 && K >= 1 && K <= N, PPH_EINVAL,
-                "pph_addon_fwd: bad dims B=%d N=%d Din=%d D=%d K=%d", B, N, Din, D, K);
-    if (B == 0) return 0;
-    const int R = B * (K + 1);
-    if (pph::addon_tc_ok(Din, D)) {
-        using namespace pph;
-        RowSrc src{idx32, B, N, Din, K, R};
-        FwdAOp a{tokens, src};
-        FwdBOp b{Wa, D, Din};
-        FwdEpi e{ba, Zs, Zc, z2s, z2c, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, center, K, D};
-        return launch_tcgemm(R, D, Din, tcgemm_pick_bn(D), 1, a, b, e, as_stream(stream), "pph_addon_fwd(tcgen05)");
-    }
-    pph::launch_k(pph::addon_fwd_kernel, dim3(pph::ceil_div(R, pph::kAddBM)), dim3(pph::kAddThreads), (size_t)(0), pph::as_stream(stream), tokens, idx32, Wa, ba, B, N, Din, D, K, Zs, Zc, z2s, z2c, center, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo);
-    return pph::launch_status("pph_addon_fwd");
+    return pph::addon_fwd_impl("pph_addon_fwd", tokens, idx32, Wa, ba, B, N, Din, D, K, Zs, Zc, z2s, z2c, center, z2s_ctr,
+                               z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, stream);
+}
+
+extern "C" int pph_addon_fwd_bf16tok(const uint16_t* tokens, const int32_t* idx32, const float* Wa, const float* ba,
+                                     int B, int N, int Din, int D, int K,
+                                     float* Zs, float* Zc, float* z2s, float* z2c,
+                                     float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                                     uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                                     pph_stream_t stream) {
+    return pph::addon_fwd_impl("pph_addon_fwd_bf16tok", tokens, idx32, Wa, ba, B, N, Din, D, K, Zs, Zc, z2s, z2c, center,
+                               z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, stream);
 }
 
 extern "C" int pph_split_rows(const float* V, int R, int D, float center, uint16_t* hi, uint16_t* lo, float* v2,
@@ -309,74 +410,14 @@ extern "C" int pph_addon_bwd(const float* tokens, const int32_t* idx32, const fl
                              const float* Zs, const float* Zc, const float* dZs, const float* dZc,
                              int B, int N, int Din, int D, int K, void* workspace, int parts,
                              float* dWa, float* dba, float* dtokens, pph_stream_t stream) {
-    using namespace pph;
-    PPH_REQUIRE((parts & 3) != 0, PPH_EINVAL, "pph_addon_bwd: parts must include PPH_ADDON_WGRAD and/or PPH_ADDON_DGRAD");
-    if (!(parts & PPH_ADDON_DGRAD)) dtokens = nullptr;
-    const bool want_w = (parts & PPH_ADDON_WGRAD) != 0;
-    PPH_REQUIRE(tokens && idx32 && Wa && Zs && Zc && dZs && dZc && (!want_w || (dWa && dba)), PPH_EINVAL,
-                "pph_addon_bwd: null pointer");
-    PPH_REQUIRE(B >= 0 && N >= 1 && Din >= 1 && D >= 1 && K >= 1 && K <= N, PPH_EINVAL,
-                "pph_addon_bwd: bad dims B=%d N=%d Din=%d D=%d K=%d", B, N, Din, D, K);
-    cudaStream_t st = as_stream(stream);
-    const bool tc = addon_tc_ok(Din, D) && B > 0;
-    cudaError_t e = cudaSuccess;
-    if (!tc && want_w) {
-        e = cudaMemsetAsync(dWa, 0, sizeof(float) * (size_t)D * Din, st);
-        if (e == cudaSuccess) e = cudaMemsetAsync(dba, 0, sizeof(float) * (size_t)D, st);
-    }
-    if (e == cudaSuccess && dtokens)
-        e = cudaMemsetAsync(dtokens, 0, sizeof(float) * (size_t)B * (1 + N) * Din, st);
-    if (e != cudaSuccess) {
-        set_error("pph_addon_bwd: memset: %s", cudaGetErrorString(e));
-        return (int)e;
-    }
-    if (B == 0) return 0;
-    const int R = B * (K + 1);
-    if (tc) {
-        PPH_REQUIRE(workspace || !want_w, PPH_EINVAL, "pph_addon_bwd: null workspace (size it with pph_addon_bwd_ws_bytes)");
-        RowSrc src{idx32, B, N, Din, K, R};
-        if (want_w) {   // dWa / dba: [D x (Din+1)] = dpre^T [D x R] * [Xsel | 1]^T, split over r, partials + ordered reduction
-            const int ldn = ceil_div(Din + 1, 4) * 4;
-            int splits = wgrad_splits(R);
-            const int k_per_split = ceil_div(ceil_div(R, splits), kTgBK) * kTgBK;
-            splits = ceil_div(R, k_per_split);
-            float* part = static_cast<float*>(workspace);
-            DpreColOp a{Zs, Zc, dZs, dZc, K, D, R};
-            XselColOp b{tokens, src};
-            WgradPartEpi epi{part, D, ldn};
-            int rc = launch_tcgemm(D, ldn, R, tcgemm_pick_bn(ldn), splits, a, b, epi, st, "pph_addon_bwd(wgrad tcgen05)");
-            if (rc) return rc;
-            launch_k(wgrad_reduce_kernel, dim3(ceil_div(D * (Din + 1), 256)), dim3(256), (size_t)(0), st, part, splits, D, Din, ldn, dWa, dba);
-            rc = launch_status("pph_addon_bwd(wgrad reduce)");
-            if (rc) return rc;
-        }
-        if (dtokens) {   // dX [R x Din] = dpre [R x D] * Wa [D x Din]
-            DpreRowOp a{Zs, Zc, dZs, dZc, K, D, R};
-            WaTOp b{Wa, D, Din};
-            DxTcEpi epi{dtokens, src};
-            int rc = launch_tcgemm(R, Din, D, tcgemm_pick_bn(Din), 1, a, b, epi, st, "pph_addon_bwd(dgrad tcgen05)");
-            if (rc) return rc;
-        }
-        return 0;
-    }
-    RowMap map{B, K, D};
-    if (want_w) {   // dWa[d, din] = sum_r dpre[r,d] * X[r,din];  dba[d] = sum_r dpre[r,d]   (split over r)
-        DpreOp<true> a{Zs, Zc, dZs, dZc, map, R};
-        XselOp b{tokens, idx32, B, N, Din, K, R};
-        WgradEpi epi{dWa, dba, Din};
-        const int tiles = ceil_div(D, kGemmBM) * ceil_div(Din, kGemmBN);
-        int splits = ceil_div(2 * 148, tiles);
-        launch_sgemm<true>(D, Din, R, splits, a, b, epi, st);
-        int rc = launch_status("pph_addon_bwd(wgrad)");
-        if (rc) return rc;
-    }
-    if (dtokens) {   // dX[r, din] = sum_d dpre[r,d] * Wa[d,din]  -> scattered into the zero-filled token gradient
-        DpreOp<false> a{Zs, Zc, dZs, dZc, map, R};
-        StridedOp<false> b{Wa, Din, 1, Din};       // (row = din, k = d) -> Wa[d*Din + din]
-        DxEpi epi{dtokens, idx32, N, Din, K};
-        launch_sgemm<false>(R, Din, D, 1, a, b, epi, st);
-        int rc = launch_status("pph_addon_bwd(dgrad)");
-        if (rc) return rc;
-    }
-    return 0;
+    return pph::addon_bwd_impl("pph_addon_bwd", tokens, idx32, Wa, Zs, Zc, dZs, dZc, B, N, Din, D, K, workspace, parts, dWa,
+                               dba, dtokens, stream);
+}
+
+extern "C" int pph_addon_bwd_bf16tok(const uint16_t* tokens, const int32_t* idx32, const float* Wa,
+                                     const float* Zs, const float* Zc, const float* dZs, const float* dZc,
+                                     int B, int N, int Din, int D, int K, void* workspace, int parts,
+                                     float* dWa, float* dba, uint16_t* dtokens, pph_stream_t stream) {
+    return pph::addon_bwd_impl("pph_addon_bwd_bf16tok", tokens, idx32, Wa, Zs, Zc, dZs, dZc, B, N, Din, D, K, workspace,
+                               parts, dWa, dba, dtokens, stream);
 }

@@ -23,9 +23,11 @@ struct AddonBwdArgs {
     int TR, Dp, nchunks, threadsX, nX;     // role X plan
     int tilesO, tilesI, S, RS, nW;         // role W plan: S row splits of RS rows
     int want_dx, want_dw;
-    const float *tokens, *Wa, *dpre_s, *dpre_c;
+    const float *Wa, *dpre_s, *dpre_c;
+    const void* tokens;                    // [B, 1+N, Din] of the kernel's token type (float or bf16)
     const int32_t* idx;
-    float *dWa, *dba, *dtokens;
+    float *dWa, *dba;
+    void* dtokens;                         // same type as tokens
     float *part, *partb;                   // [S][D][Din], [S][D]
     unsigned int* cnt;                     // [tilesO * tilesI]
 };
@@ -43,6 +45,7 @@ __device__ __forceinline__ const float* dpre_ptr(const AddonBwdArgs& a, int r, i
 }
 
 // ---- role X ----------------------------------------------------------------------------------------------------
+template <class T>
 __device__ __forceinline__ void addon_bwd_x(const AddonBwdArgs& a, float* sm) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nthr = a.threadsX, nwarp = nthr >> 5;
     const int K = a.K, N = a.N, Din = a.Din, D = a.D, TR = a.TR, Dp = a.Dp;
@@ -122,11 +125,11 @@ __device__ __forceinline__ void addon_bwd_x(const AddonBwdArgs& a, float* sm) {
             int b, j;
             row_of(r0 + rl, K, b, j);
             const int tok = j < K ? 1 + __ldg(a.idx + (size_t)b * K + j) : 0;
-            float* dst = a.dtokens + ((size_t)b * (1 + N) + tok) * Din;
+            T* dst = static_cast<T*>(a.dtokens) + ((size_t)b * (1 + N) + tok) * Din;
 #pragma unroll
             for (int h = 0; h < 2; ++h)
-                *reinterpret_cast<float4*>(dst + h * (Din >> 1) + cg * 4) =
-                    make_float4(acc[i][h * 4], acc[i][h * 4 + 1], acc[i][h * 4 + 2], acc[i][h * 4 + 3]);
+                st4_tok(dst + h * (Din >> 1) + cg * 4,
+                        make_float4(acc[i][h * 4], acc[i][h * 4 + 1], acc[i][h * 4 + 2], acc[i][h * 4 + 3]));
         }
     }
     // zero fill of the token rows nobody selected: this CTA's share of the B * (1 + N) rows, one warp per row
@@ -139,8 +142,9 @@ __device__ __forceinline__ void addon_bwd_x(const AddonBwdArgs& a, float* sm) {
         bool hit = false;
         for (int k = lane; k < K; k += 32) hit |= (__ldg(a.idx + (size_t)b * K + k) == t - 1);
         if (__any_sync(0xffffffffu, hit)) continue;
-        float4* dst = reinterpret_cast<float4*>(a.dtokens + (size_t)row * Din);
-        for (int c = lane; c < i4; c += 32) dst[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+        float4* dst = reinterpret_cast<float4*>(static_cast<T*>(a.dtokens) + (size_t)row * Din);
+        const int row16 = Din * (int)sizeof(T) / 16;                   // 16-byte words per row (Din % 8 == 0)
+        for (int c = lane; c < row16; c += 32) dst[c] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
 }
 
@@ -148,6 +152,7 @@ __device__ __forceinline__ void addon_bwd_x(const AddonBwdArgs& a, float* sm) {
 // barrier of the 256 threads that run role W (the launch may have more threads per CTA: role X sizes it)
 __device__ __forceinline__ void bar_w() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
 
+template <class T>
 __device__ __forceinline__ void addon_bwd_w(const AddonBwdArgs& a, int vb, float* sm) {
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
     const int K = a.K, N = a.N, Din = a.Din, D = a.D;
@@ -179,7 +184,9 @@ __device__ __forceinline__ void addon_bwd_w(const AddonBwdArgs& a, int vb, float
                 row_of(r, K, b, j);
                 if (i0 + lq * 4 < Din) {
                     const int tok = j < K ? 1 + __ldg(a.idx + (size_t)b * K + j) : 0;
-                    cp_async16(dx, a.tokens + ((size_t)b * (1 + N) + tok) * Din + i0 + lq * 4);
+                    const T* src = static_cast<const T*>(a.tokens) + ((size_t)b * (1 + N) + tok) * Din + i0 + lq * 4;
+                    if constexpr (sizeof(T) == 4) cp_async16(dx, src);
+                    else *reinterpret_cast<float4*>(dx) = ldg4_tok(src);     // bf16: widened on the way in
                 } else {
                     *reinterpret_cast<float4*>(dx) = make_float4(0.f, 0.f, 0.f, 0.f);
                 }
@@ -256,15 +263,15 @@ __device__ __forceinline__ void addon_bwd_w(const AddonBwdArgs& a, int vb, float
     if (tid == 0) a.cnt[tile] = 0u;                   // self-resetting (graph replay)
 }
 
-template <int MAXT>
+template <int MAXT, class T>
 __global__ void __launch_bounds__(MAXT, 1)
 addon_bwd2_kernel(const AddonBwdArgs a) {
     pdl_sync();
     extern __shared__ __align__(16) float sm_ab[];
     if ((int)blockIdx.x < a.nX) {
-        addon_bwd_x(a, sm_ab);
+        addon_bwd_x<T>(a, sm_ab);
     } else {
-        if ((int)threadIdx.x < kAbWThreads) addon_bwd_w(a, blockIdx.x - a.nX, sm_ab);
+        if ((int)threadIdx.x < kAbWThreads) addon_bwd_w<T>(a, blockIdx.x - a.nX, sm_ab);
     }
 }
 
@@ -330,20 +337,23 @@ extern "C" int pph_addon_bwd2_ws_bytes(int B, int N, int Din, int D, int K, long
     return 0;
 }
 
-extern "C" int pph_addon_bwd2(int parts, const float* tokens, const int32_t* idx32, const float* Wa,
-                              const float* dpre_s, const float* dpre_c,
-                              int B, int N, int Din, int D, int K, void* workspace,
-                              float* dWa, float* dba, float* dtokens, pph_stream_t stream) {
-    using namespace pph;
-    PPH_REQUIRE((parts & 3) != 0, PPH_EINVAL, "pph_addon_bwd2: parts must name WGRAD and/or DGRAD");
-    PPH_REQUIRE(tokens && idx32 && Wa && dpre_s && dpre_c && workspace, PPH_EINVAL, "pph_addon_bwd2: null pointer");
-    PPH_REQUIRE(!(parts & PPH_ADDON_WGRAD) || (dWa && dba), PPH_EINVAL, "pph_addon_bwd2(WGRAD): null output");
-    PPH_REQUIRE(!(parts & PPH_ADDON_DGRAD) || dtokens, PPH_EINVAL, "pph_addon_bwd2(DGRAD): null dtokens");
-    PPH_REQUIRE(pph_addon_bwd2_supported(B, N, Din, D, K), PPH_EUNSUP, "pph_addon_bwd2: unsupported shape");
+namespace pph {
+
+template <class T>
+static int addon_bwd2_impl(const char* name, int parts, const T* tokens, const int32_t* idx32, const float* Wa,
+                           const float* dpre_s, const float* dpre_c,
+                           int B, int N, int Din, int D, int K, void* workspace,
+                           float* dWa, float* dba, T* dtokens, pph_stream_t stream) {
+    PPH_REQUIRE((parts & 3) != 0, PPH_EINVAL, "%s: parts must name WGRAD and/or DGRAD", name);
+    PPH_REQUIRE(tokens && idx32 && Wa && dpre_s && dpre_c && workspace, PPH_EINVAL, "%s: null pointer", name);
+    PPH_REQUIRE(!(parts & PPH_ADDON_WGRAD) || (dWa && dba), PPH_EINVAL, "%s(WGRAD): null output", name);
+    PPH_REQUIRE(!(parts & PPH_ADDON_DGRAD) || dtokens, PPH_EINVAL, "%s(DGRAD): null dtokens", name);
+    PPH_REQUIRE(sizeof(T) == 4 || Din % 8 == 0, PPH_EINVAL, "%s: bf16 tokens need Din %% 8 == 0 (Din=%d)", name, Din);
+    PPH_REQUIRE(pph_addon_bwd2_supported(B, N, Din, D, K), PPH_EUNSUP, "%s: unsupported shape", name);
     int sms = pph_sm_count();
     if (sms <= 0) sms = 148;
     AddonBwdPlan p;
-    PPH_REQUIRE(addon_bwd_plan(B, N, Din, D, K, sms, &p), PPH_EUNSUP, "pph_addon_bwd2: no plan");
+    PPH_REQUIRE(addon_bwd_plan(B, N, Din, D, K, sms, &p), PPH_EUNSUP, "%s: no plan", name);
     AddonBwdArgs a;
     a.B = B; a.N = N; a.Din = Din; a.D = D; a.K = K; a.R = B * (K + 1);
     a.TR = p.TR; a.Dp = p.Dp; a.nchunks = p.nchunks; a.threadsX = p.threadsX;
@@ -360,11 +370,29 @@ extern "C" int pph_addon_bwd2(int parts, const float* tokens, const int32_t* idx
     off = (off + 255) / 256 * 256;
     a.part = reinterpret_cast<float*>(w + off);
     a.partb = a.part + (size_t)p.S * D * Din;
-    auto k_small = addon_bwd2_kernel<256>;
-    auto k_large = addon_bwd2_kernel<640>;
+    auto k_small = addon_bwd2_kernel<256, T>;
+    auto k_large = addon_bwd2_kernel<640, T>;
     auto kern = p.threads <= 256 ? k_small : k_large;
     cudaError_t e = opt_in_smem(kern, (int)p.smem);
-    if (e != cudaSuccess) { set_error("pph_addon_bwd2: %s", cudaGetErrorString(e)); return (int)e; }
+    if (e != cudaSuccess) { set_error("%s: %s", name, cudaGetErrorString(e)); return (int)e; }
     launch_k(kern, dim3(a.nX + a.nW), dim3(p.threads), p.smem, as_stream(stream), a);
-    return launch_status("pph_addon_bwd2");
+    return launch_status(name);
+}
+
+}  // namespace pph
+
+extern "C" int pph_addon_bwd2(int parts, const float* tokens, const int32_t* idx32, const float* Wa,
+                              const float* dpre_s, const float* dpre_c,
+                              int B, int N, int Din, int D, int K, void* workspace,
+                              float* dWa, float* dba, float* dtokens, pph_stream_t stream) {
+    return pph::addon_bwd2_impl("pph_addon_bwd2", parts, tokens, idx32, Wa, dpre_s, dpre_c, B, N, Din, D, K, workspace, dWa,
+                                dba, dtokens, stream);
+}
+
+extern "C" int pph_addon_bwd2_bf16tok(int parts, const uint16_t* tokens, const int32_t* idx32, const float* Wa,
+                                      const float* dpre_s, const float* dpre_c,
+                                      int B, int N, int Din, int D, int K, void* workspace,
+                                      float* dWa, float* dba, uint16_t* dtokens, pph_stream_t stream) {
+    return pph::addon_bwd2_impl("pph_addon_bwd2_bf16tok", parts, tokens, idx32, Wa, dpre_s, dpre_c, B, N, Din, D, K,
+                                workspace, dWa, dba, dtokens, stream);
 }

@@ -22,15 +22,25 @@ __device__ __forceinline__ void ld8(const float* p, float (&v)[8]) {
     const float4 a = __ldg(reinterpret_cast<const float4*>(p)), b = __ldg(reinterpret_cast<const float4*>(p) + 1);
     v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
 }
+__device__ __forceinline__ void ld8(const uint16_t* p, float (&v)[8]) {     // eight bf16 tokens values: one 16-byte load
+    const uint4 q = __ldg(reinterpret_cast<const uint4*>(p));
+    const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        v[2 * i] = __uint_as_float(w[i] << 16);
+        v[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
+    }
+}
 __device__ __forceinline__ void zero8(float (&v)[8]) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) v[i] = 0.f;
 }
 
 // ---- forward: Z = sigmoid(Xsel Wa^T + ba) --------------------------------------------------------------------------
+template <class T>   // token element type: float or bf16 (uint16_t), here and in every token operand / epilogue below
 struct FwdAOp {     // (row = r, k = din): gathered token rows
     static constexpr bool kContigK = true;
-    const float* tokens;
+    const T* tokens;
     RowSrc src;
     __device__ __forceinline__ void load8(int r, int k0, float (&v)[8]) const {
         if (r < src.R && k0 < src.Din) ld8(tokens + src(r) + k0, v); else zero8(v);
@@ -40,10 +50,11 @@ struct FwdAOp {     // (row = r, k = din): gathered token rows
 // CTA ranks the CLS-attention scores of the (<= 4) images its 128-row tile touches -- rank by counting with the same
 // total order as select_topk_kernel (larger score first, lower index on ties, NaN first) -- and keeps the ascending index
 // lists in shared memory; the CTAs of the first column tile also write them to idx_out for the kernels downstream.
+template <class T>
 struct FwdSelAOp {
     static constexpr bool kContigK = true;
     static constexpr bool kSelect = true;
-    const float* tokens;
+    const T* tokens;
     const float* scores;       // [B, H, N]
     int32_t* idx_out;          // [B, K]
     int B, N, Din, K, R, H;
@@ -242,9 +253,10 @@ struct WaTOp {      // (row = din, k = d): Wa[d, din]
         for (int i = 0; i < 8; ++i) v[i] = (din < Din && d0 + i < D) ? __ldg(Wa + (size_t)(d0 + i) * Din + din) : 0.f;
     }
 };
+template <class T>
 struct XselColOp {  // (row = din, k = r): gathered token rows transposed; row Din is the all-ones column (-> dba)
     static constexpr bool kContigK = false;
-    const float* tokens;
+    const T* tokens;
     RowSrc src;
     __device__ __forceinline__ void load8(int din, int r0, float (&v)[8]) const {
         const int K = src.K;
@@ -255,7 +267,7 @@ struct XselColOp {  // (row = din, k = r): gathered token rows transposed; row D
             if (r0 + i < src.R) {
                 if (din < src.Din) {
                     const int tok = j < K ? 1 + __ldg(src.idx + (size_t)b * K + j) : 0;
-                    val = __ldg(tokens + ((size_t)b * (1 + src.N) + tok) * src.Din + din);
+                    val = ldg_tok(tokens + ((size_t)b * (1 + src.N) + tok) * src.Din + din);
                 } else if (din == src.Din) {
                     val = 1.0f;
                 }
@@ -265,17 +277,18 @@ struct XselColOp {  // (row = din, k = r): gathered token rows transposed; row D
         }
     }
 };
+template <class T>
 struct DxTcEpi {    // scatter rows of dX into the (zero-filled) token gradient
     static constexpr bool kDirect = false;
     static constexpr bool kGridReduce = false;
-    float* dtokens;
+    T* dtokens;
     RowSrc src;
     struct State { int dummy; };
     __device__ __forceinline__ void init(State& s) const { s.dummy = 0; }
     __device__ __forceinline__ void row_ptrs(int r, void* (&p)[3]) const { p[0] = dtokens + src(r); }
     __device__ __forceinline__ void transform(State&, int, int, uint32_t (&)[32]) const {}
     __device__ __forceinline__ void store2(void* const* p, int n, float v0, float v1) const {
-        *reinterpret_cast<float2*>(static_cast<float*>(p[0]) + n) = make_float2(v0, v1);
+        st2_tok(static_cast<T*>(p[0]) + n, v0, v1);
     }
     __device__ __forceinline__ void finish(State&, int, int, int, float*, bool) const {}
 };

@@ -130,9 +130,11 @@ struct PreColQOp : PreColOp {       // (rows d..d+3, k = r0..r0+7); D % 4 == 0
         }
     }
 };
-struct XselColQOp : XselColOp {     // (rows din..din+3, k = r0..r0+7); Din % 4 == 0; row Din = the all-ones column
+template <class T>
+struct XselColQOp : XselColOp<T> {  // (rows din..din+3, k = r0..r0+7); Din % 4 == 0; row Din = the all-ones column
     static constexpr bool kQuad = true;
     __device__ __forceinline__ void load8x4(int din, int r0, float (&v)[4][8]) const {
+        const RowSrc& src = this->src;
         const int K = src.K;
         int b = r0 / (K + 1), j = r0 - b * (K + 1);
 #pragma unroll
@@ -141,7 +143,7 @@ struct XselColQOp : XselColOp {     // (rows din..din+3, k = r0..r0+7); Din % 4 
             if (r0 + i < src.R) {
                 if (din < src.Din) {
                     const int tok = j < K ? 1 + __ldg(src.idx + (size_t)b * K + j) : 0;
-                    x = ldg4(tokens + ((size_t)b * (1 + src.N) + tok) * src.Din + din);
+                    x = ldg4_tok(this->tokens + ((size_t)b * (1 + src.N) + tok) * src.Din + din);
                 } else if (din == src.Din) {
                     x.x = 1.0f;
                 }
@@ -251,7 +253,7 @@ extern "C" int pph_addon_tc2_supported(int B, int N, int Din, int D, int K) {
     using namespace pph;
     if (B < 1 || N < 1 || K < 1 || K > N || B * (K + 1) > 1008 * kTsBM) return 0;
     const Tc2Plan p = tc2_plan(B, Din, D, K, 148);
-    const bool sel_ok = p.fwd_ok && N <= 256 && FwdSelAOp::words(N, K) <= 128 * 16;
+    const bool sel_ok = p.fwd_ok && N <= 256 && FwdSelAOp<float>::words(N, K) <= 128 * 16;
     return (p.fwd_ok ? 1 : 0) | (p.dx_ok ? 2 : 0) | (p.w_ok ? 4 : 0) | (sel_ok ? 8 : 0);
 }
 
@@ -263,21 +265,24 @@ extern "C" int pph_addon_tc2_ws_bytes(int B, int N, int Din, int D, int K, long 
     return 0;
 }
 
-extern "C" int pph_addon_fwd2(const float* tokens, const int32_t* idx32, const float* Wa, const float* ba,
-                              int B, int N, int Din, int D, int K,
-                              float* Zs, float* Zc, float* z2s, float* z2c,
-                              float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
-                              uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
-                              void* workspace, pph_stream_t stream) {
-    using namespace pph;
-    PPH_REQUIRE(tokens && idx32 && Wa && ba && Zs && Zc && z2s && z2c && workspace, PPH_EINVAL, "pph_addon_fwd2: null pointer");
-    PPH_REQUIRE(B >= 1 && N >= 1 && K >= 1 && K <= N, PPH_EINVAL, "pph_addon_fwd2: bad dims");
+namespace pph {
+
+template <class T>
+static int addon_fwd2_impl(const char* name, const T* tokens, const int32_t* idx32, const float* Wa, const float* ba,
+                           int B, int N, int Din, int D, int K,
+                           float* Zs, float* Zc, float* z2s, float* z2c,
+                           float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                           uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                           void* workspace, pph_stream_t stream) {
+    PPH_REQUIRE(tokens && idx32 && Wa && ba && Zs && Zc && z2s && z2c && workspace, PPH_EINVAL, "%s: null pointer", name);
+    PPH_REQUIRE(B >= 1 && N >= 1 && K >= 1 && K <= N, PPH_EINVAL, "%s: bad dims", name);
+    PPH_REQUIRE(sizeof(T) == 4 || Din % 8 == 0, PPH_EINVAL, "%s: bf16 tokens need Din %% 8 == 0 (Din=%d)", name, Din);
     const Tc2Plan p = tc2_plan(B, Din, D, K, tc2_sms());
-    PPH_REQUIRE(p.fwd_ok && B * (K + 1) <= 1008 * kTsBM, PPH_EUNSUP, "pph_addon_fwd2: Din=%d D=%d outside the single-shot kernel", Din, D);
+    PPH_REQUIRE(p.fwd_ok && B * (K + 1) <= 1008 * kTsBM, PPH_EUNSUP, "%s: Din=%d D=%d outside the single-shot kernel", name, Din, D);
     const int R = B * (K + 1);
     const Tc2Ws w = tc2_carve(workspace, R);
     RowSrc src{idx32, B, N, Din, K, R};
-    FwdAOp a{tokens, src};
+    FwdAOp<T> a{tokens, src};
     FwdBOp b{Wa, D, Din};
     FwdEpi2 e;
     static_cast<FwdEpi&>(e) = FwdEpi{ba, Zs, Zc, z2s, z2c, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, center, K, D};
@@ -286,22 +291,23 @@ extern "C" int pph_addon_fwd2(const float* tokens, const int32_t* idx32, const f
                          "pph_addon_fwd2(tcgen05 single shot)");
 }
 
-extern "C" int pph_select_addon_fwd(const float* scores, int H, const float* tokens, const float* Wa, const float* ba,
-                                    int B, int N, int Din, int D, int K, int32_t* idx32,
-                                    float* Zs, float* Zc, float* z2s, float* z2c,
-                                    float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
-                                    uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
-                                    void* workspace, pph_stream_t stream) {
-    using namespace pph;
+template <class T>
+static int select_addon_fwd_impl(const char* name, const float* scores, int H, const T* tokens, const float* Wa,
+                                 const float* ba, int B, int N, int Din, int D, int K, int32_t* idx32,
+                                 float* Zs, float* Zc, float* z2s, float* z2c,
+                                 float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                                 uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                                 void* workspace, pph_stream_t stream) {
     PPH_REQUIRE(scores && tokens && idx32 && Wa && ba && Zs && Zc && z2s && z2c && workspace, PPH_EINVAL,
-                "pph_select_addon_fwd: null pointer");
-    PPH_REQUIRE(B >= 1 && H >= 1 && N >= 1 && K >= 1 && K <= N, PPH_EINVAL, "pph_select_addon_fwd: bad dims");
+                "%s: null pointer", name);
+    PPH_REQUIRE(B >= 1 && H >= 1 && N >= 1 && K >= 1 && K <= N, PPH_EINVAL, "%s: bad dims", name);
+    PPH_REQUIRE(sizeof(T) == 4 || Din % 8 == 0, PPH_EINVAL, "%s: bf16 tokens need Din %% 8 == 0 (Din=%d)", name, Din);
     const Tc2Plan p = tc2_plan(B, Din, D, K, tc2_sms());
-    PPH_REQUIRE(p.fwd_ok && B * (K + 1) <= 1008 * kTsBM && N <= 256 && FwdSelAOp::words(N, K) <= 128 * 16, PPH_EUNSUP,
-                "pph_select_addon_fwd: N=%d K=%d Din=%d D=%d outside the fused selection + add-on kernel", N, K, Din, D);
+    PPH_REQUIRE(p.fwd_ok && B * (K + 1) <= 1008 * kTsBM && N <= 256 && FwdSelAOp<T>::words(N, K) <= 128 * 16, PPH_EUNSUP,
+                "%s: N=%d K=%d Din=%d D=%d outside the fused selection + add-on kernel", name, N, K, Din, D);
     const int R = B * (K + 1);
     const Tc2Ws w = tc2_carve(workspace, R);
-    FwdSelAOp a{tokens, scores, idx32, B, N, Din, K, R, H};
+    FwdSelAOp<T> a{tokens, scores, idx32, B, N, Din, K, R, H};
     FwdBOp b{Wa, D, Din};
     FwdEpi2 e;
     static_cast<FwdEpi&>(e) = FwdEpi{ba, Zs, Zc, z2s, z2c, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, center, K, D};
@@ -310,41 +316,102 @@ extern "C" int pph_select_addon_fwd(const float* scores, int H, const float* tok
                          "pph_select_addon_fwd(tcgen05 single shot)");
 }
 
-extern "C" int pph_addon_bwd3(int parts, const float* tokens, const int32_t* idx32, const float* Wa,
-                              const float* dpre_s, const float* dpre_c, const float* dpre_add_s,
-                              int B, int N, int Din, int D, int K, void* workspace,
-                              float* dWa, float* dba, float* dtokens, pph_stream_t stream) {
-    using namespace pph;
-    PPH_REQUIRE((parts & 3) != 0, PPH_EINVAL, "pph_addon_bwd3: parts must name WGRAD and/or DGRAD");
-    PPH_REQUIRE(tokens && idx32 && Wa && dpre_s && dpre_c && workspace, PPH_EINVAL, "pph_addon_bwd3: null pointer");
-    PPH_REQUIRE(B >= 1 && N >= 1 && K >= 1 && K <= N, PPH_EINVAL, "pph_addon_bwd3: bad dims");
+template <class T>
+static int addon_bwd3_impl(const char* name, int parts, const T* tokens, const int32_t* idx32, const float* Wa,
+                           const float* dpre_s, const float* dpre_c, const float* dpre_add_s,
+                           int B, int N, int Din, int D, int K, void* workspace,
+                           float* dWa, float* dba, T* dtokens, pph_stream_t stream) {
+    PPH_REQUIRE((parts & 3) != 0, PPH_EINVAL, "%s: parts must name WGRAD and/or DGRAD", name);
+    PPH_REQUIRE(tokens && idx32 && Wa && dpre_s && dpre_c && workspace, PPH_EINVAL, "%s: null pointer", name);
+    PPH_REQUIRE(B >= 1 && N >= 1 && K >= 1 && K <= N, PPH_EINVAL, "%s: bad dims", name);
+    PPH_REQUIRE(sizeof(T) == 4 || Din % 8 == 0, PPH_EINVAL, "%s: bf16 tokens need Din %% 8 == 0 (Din=%d)", name, Din);
     const Tc2Plan p = tc2_plan(B, Din, D, K, tc2_sms());
     const int R = B * (K + 1);
     const Tc2Ws w = tc2_carve(workspace, R);
     cudaStream_t st = as_stream(stream);
     RowSrc src{idx32, B, N, Din, K, R};
     if (parts & PPH_ADDON_WGRAD) {
-        PPH_REQUIRE(dWa && dba, PPH_EINVAL, "pph_addon_bwd3(WGRAD): null output");
-        PPH_REQUIRE(p.w_ok, PPH_EUNSUP, "pph_addon_bwd3(WGRAD): %d CTAs for B=%d K=%d Din=%d D=%d", p.w_ctas, B, K, Din, D);
+        PPH_REQUIRE(dWa && dba, PPH_EINVAL, "%s(WGRAD): null output", name);
+        PPH_REQUIRE(p.w_ok, PPH_EUNSUP, "%s(WGRAD): %d CTAs for B=%d K=%d Din=%d D=%d", name, p.w_ctas, B, K, Din, D);
         PreColQOp a;
         static_cast<PreColOp&>(a) = PreColOp{dpre_s, dpre_c, dpre_add_s, K, D, R};
-        XselColQOp b;
-        static_cast<XselColOp&>(b) = XselColOp{tokens, src};
+        XselColQOp<T> b;
+        static_cast<XselColOp<T>&>(b) = XselColOp<T>{tokens, src};
         WgradEpi2 e{w.wpart, dWa, dba, D, Din, p.ldn, p.w_splits};
         const int rc = launch_tcshot(D, Din + 1, R, p.bn_w, kTsMaxKB * kTsBK, w.sync_ctr, a, b, e, st,
                                      "pph_addon_bwd3(wgrad tcgen05 single shot)");
         if (rc) return rc;
     }
     if (parts & PPH_ADDON_DGRAD) {
-        PPH_REQUIRE(dtokens, PPH_EINVAL, "pph_addon_bwd3(DGRAD): null dtokens");
-        PPH_REQUIRE(p.dx_ok, PPH_EUNSUP, "pph_addon_bwd3(DGRAD): D=%d outside the single-shot kernel", D);
+        PPH_REQUIRE(dtokens, PPH_EINVAL, "%s(DGRAD): null dtokens", name);
+        PPH_REQUIRE(p.dx_ok, PPH_EUNSUP, "%s(DGRAD): D=%d outside the single-shot kernel", name, D);
         PreRowOp a{dpre_s, dpre_c, dpre_add_s, K, D, R};
         WaTQOp b;
         static_cast<WaTOp&>(b) = WaTOp{Wa, D, Din};
-        DxTcEpi e{dtokens, src};
+        DxTcEpi<T> e{dtokens, src};
         const int rc = launch_tcshot(R, Din, D, p.bn_dx, ceil_div(D, kTsBK) * kTsBK, w.sync_ctr, a, b, e, st,
                                      "pph_addon_bwd3(dgrad tcgen05 single shot)");
         if (rc) return rc;
     }
     return 0;
+}
+
+}  // namespace pph
+
+extern "C" int pph_addon_fwd2(const float* tokens, const int32_t* idx32, const float* Wa, const float* ba,
+                              int B, int N, int Din, int D, int K,
+                              float* Zs, float* Zc, float* z2s, float* z2c,
+                              float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                              uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                              void* workspace, pph_stream_t stream) {
+    return pph::addon_fwd2_impl("pph_addon_fwd2", tokens, idx32, Wa, ba, B, N, Din, D, K, Zs, Zc, z2s, z2c, center, z2s_ctr,
+                                z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, workspace, stream);
+}
+
+extern "C" int pph_addon_fwd2_bf16tok(const uint16_t* tokens, const int32_t* idx32, const float* Wa, const float* ba,
+                                      int B, int N, int Din, int D, int K,
+                                      float* Zs, float* Zc, float* z2s, float* z2c,
+                                      float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                                      uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                                      void* workspace, pph_stream_t stream) {
+    return pph::addon_fwd2_impl("pph_addon_fwd2_bf16tok", tokens, idx32, Wa, ba, B, N, Din, D, K, Zs, Zc, z2s, z2c, center,
+                                z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, workspace, stream);
+}
+
+extern "C" int pph_select_addon_fwd(const float* scores, int H, const float* tokens, const float* Wa, const float* ba,
+                                    int B, int N, int Din, int D, int K, int32_t* idx32,
+                                    float* Zs, float* Zc, float* z2s, float* z2c,
+                                    float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                                    uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                                    void* workspace, pph_stream_t stream) {
+    return pph::select_addon_fwd_impl("pph_select_addon_fwd", scores, H, tokens, Wa, ba, B, N, Din, D, K, idx32, Zs, Zc, z2s,
+                                      z2c, center, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, workspace,
+                                      stream);
+}
+
+extern "C" int pph_select_addon_fwd_bf16tok(const float* scores, int H, const uint16_t* tokens, const float* Wa,
+                                            const float* ba, int B, int N, int Din, int D, int K, int32_t* idx32,
+                                            float* Zs, float* Zc, float* z2s, float* z2c,
+                                            float center, float* z2s_ctr, float* z2c_ctr, float* z2s_hi, float* z2c_hi,
+                                            uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi, uint16_t* Zc_lo,
+                                            void* workspace, pph_stream_t stream) {
+    return pph::select_addon_fwd_impl("pph_select_addon_fwd_bf16tok", scores, H, tokens, Wa, ba, B, N, Din, D, K, idx32, Zs,
+                                      Zc, z2s, z2c, center, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo,
+                                      workspace, stream);
+}
+
+extern "C" int pph_addon_bwd3(int parts, const float* tokens, const int32_t* idx32, const float* Wa,
+                              const float* dpre_s, const float* dpre_c, const float* dpre_add_s,
+                              int B, int N, int Din, int D, int K, void* workspace,
+                              float* dWa, float* dba, float* dtokens, pph_stream_t stream) {
+    return pph::addon_bwd3_impl("pph_addon_bwd3", parts, tokens, idx32, Wa, dpre_s, dpre_c, dpre_add_s, B, N, Din, D, K,
+                                workspace, dWa, dba, dtokens, stream);
+}
+
+extern "C" int pph_addon_bwd3_bf16tok(int parts, const uint16_t* tokens, const int32_t* idx32, const float* Wa,
+                                      const float* dpre_s, const float* dpre_c, const float* dpre_add_s,
+                                      int B, int N, int Din, int D, int K, void* workspace,
+                                      float* dWa, float* dba, uint16_t* dtokens, pph_stream_t stream) {
+    return pph::addon_bwd3_impl("pph_addon_bwd3_bf16tok", parts, tokens, idx32, Wa, dpre_s, dpre_c, dpre_add_s, B, N, Din, D,
+                                K, workspace, dWa, dba, dtokens, stream);
 }

@@ -194,4 +194,31 @@ __device__ __forceinline__ float bf16_to_float(uint16_t b) {
     return __uint_as_float(((uint32_t)b) << 16);
 }
 
+// ---- backbone token rows: fp32 (float) or bf16 (uint16_t storage) ------------------------------------------------
+// Every bf16 value is exact in fp32, so a bf16 token is widened at its load and nothing downstream changes: the
+// results equal those of the fp32 kernels fed the widened tokens.  Token gradients are accumulated in fp32 and
+// rounded to nearest-even once, at the store.
+__device__ __forceinline__ float tok_f(float x) { return x; }
+__device__ __forceinline__ float tok_f(uint16_t x) { return bf16_to_float(x); }
+template <class T>
+__device__ __forceinline__ float ldg_tok(const T* p) { return tok_f(__ldg(p)); }
+// four consecutive tokens values (16-byte aligned fp32 / 8-byte aligned bf16)
+__device__ __forceinline__ float4 ldg4_tok(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
+__device__ __forceinline__ float4 ldg4_tok(const uint16_t* p) {
+    const uint2 q = __ldg(reinterpret_cast<const uint2*>(p));
+    return make_float4(__uint_as_float(q.x << 16), __uint_as_float(q.x & 0xffff0000u), __uint_as_float(q.y << 16),
+                       __uint_as_float(q.y & 0xffff0000u));
+}
+__device__ __forceinline__ void st_tok(float* p, float v) { *p = v; }
+__device__ __forceinline__ void st_tok(uint16_t* p, float v) { *p = bf16_bits(v); }
+__device__ __forceinline__ void st2_tok(float* p, float a, float b) { *reinterpret_cast<float2*>(p) = make_float2(a, b); }
+__device__ __forceinline__ void st2_tok(uint16_t* p, float a, float b) {
+    *reinterpret_cast<uint32_t*>(p) = (uint32_t)bf16_bits(a) | ((uint32_t)bf16_bits(b) << 16);
+}
+__device__ __forceinline__ void st4_tok(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
+__device__ __forceinline__ void st4_tok(uint16_t* p, float4 v) {
+    *reinterpret_cast<uint2*>(p) = make_uint2((uint32_t)bf16_bits(v.x) | ((uint32_t)bf16_bits(v.y) << 16),
+                                              (uint32_t)bf16_bits(v.z) | ((uint32_t)bf16_bits(v.w) << 16));
+}
+
 }  // namespace pph

@@ -23,9 +23,9 @@ __device__ __forceinline__ float4 ld_host4(const float4* p) {
     return v;
 }
 
+// rows are moved as q 16-byte words (fp32: Din / 4, bf16: Din / 8): the kernel never looks at the element type
 __global__ void __launch_bounds__(kHgThreads) host_rows_kernel(const float* __restrict__ src, const int* __restrict__ idx32,
-                                                               int B, int N, int Din, int K, float* __restrict__ dst) {
-    const int q = Din >> 2;                                  // float4 per row
+                                                               int B, int N, int q, int K, float* __restrict__ dst) {
     const long long total = (long long)B * (K + 1) * q;
     const long long stride = (long long)gridDim.x * kHgThreads;
     for (long long i0 = (long long)blockIdx.x * kHgThreads + threadIdx.x; i0 < total; i0 += kHgBatch * stride) {
@@ -54,21 +54,32 @@ __global__ void __launch_bounds__(kHgThreads) host_rows_kernel(const float* __re
 
 using namespace pph;
 
-extern "C" int pph_gather_rows_host(const float* tokens_host, const int32_t* idx32, int B, int N, int Din, int K,
-                                    float* tokens_dev, int n_ctas, pph_stream_t stream) {
-    PPH_REQUIRE(tokens_host && idx32 && tokens_dev, PPH_EINVAL, "pph_gather_rows_host: null pointer");
-    PPH_REQUIRE(B >= 0 && N >= 1 && K >= 1 && K <= N && Din >= 4 && (Din & 3) == 0 && n_ctas >= 1 && n_ctas <= 1024, PPH_EINVAL,
-                "pph_gather_rows_host: need 1 <= K <= N, Din a multiple of 4, 1 <= n_ctas <= 1024");
+static int gather_rows_host(const char* name, const void* tokens_host, const int32_t* idx32, int B, int N, int Din, int K,
+                            int elem_bytes, void* tokens_dev, int n_ctas, pph_stream_t stream) {
+    const int per16 = 16 / elem_bytes;                       // elements per 16-byte word
+    PPH_REQUIRE(tokens_host && idx32 && tokens_dev, PPH_EINVAL, "%s: null pointer", name);
+    PPH_REQUIRE(B >= 0 && N >= 1 && K >= 1 && K <= N && Din >= per16 && Din % per16 == 0 && n_ctas >= 1 && n_ctas <= 1024,
+                PPH_EINVAL, "%s: need 1 <= K <= N, Din a multiple of %d, 1 <= n_ctas <= 1024", name, per16);
     if (B == 0) return 0;
     const void* dev_view = nullptr;     // the device-side address of the mapped host allocation (equal under UVA)
-    cudaError_t e = cudaHostGetDevicePointer(const_cast<void**>(&dev_view), const_cast<float*>(tokens_host), 0);
+    cudaError_t e = cudaHostGetDevicePointer(const_cast<void**>(&dev_view), const_cast<void*>(tokens_host), 0);
     if (e != cudaSuccess) {
         cudaGetLastError();
-        set_error("pph_gather_rows_host: tokens_host is not pinned / mapped host memory (%s)", cudaGetErrorString(e));
+        set_error("%s: tokens_host is not pinned / mapped host memory (%s)", name, cudaGetErrorString(e));
         return PPH_EINVAL;
     }
     cudaFuncSetAttribute(host_rows_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
-    host_rows_kernel<<<n_ctas, kHgThreads, 0, as_stream(stream)>>>(static_cast<const float*>(dev_view), idx32, B, N, Din, K,
-                                                                   tokens_dev);
-    return launch_status("pph_gather_rows_host");
+    host_rows_kernel<<<n_ctas, kHgThreads, 0, as_stream(stream)>>>(static_cast<const float*>(dev_view), idx32, B, N,
+                                                                   Din / per16, K, static_cast<float*>(tokens_dev));
+    return launch_status(name);
+}
+
+extern "C" int pph_gather_rows_host(const float* tokens_host, const int32_t* idx32, int B, int N, int Din, int K,
+                                    float* tokens_dev, int n_ctas, pph_stream_t stream) {
+    return gather_rows_host("pph_gather_rows_host", tokens_host, idx32, B, N, Din, K, 4, tokens_dev, n_ctas, stream);
+}
+
+extern "C" int pph_gather_rows_host_bf16tok(const uint16_t* tokens_host, const int32_t* idx32, int B, int N, int Din, int K,
+                                            uint16_t* tokens_dev, int n_ctas, pph_stream_t stream) {
+    return gather_rows_host("pph_gather_rows_host_bf16tok", tokens_host, idx32, B, N, Din, K, 2, tokens_dev, n_ctas, stream);
 }

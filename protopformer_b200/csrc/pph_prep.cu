@@ -28,7 +28,8 @@ struct PrepArgs {
     int max_img;                       // images one tile can touch
     int threads;
     float center;
-    const float *scores, *tokens, *Wa, *ba;
+    const float *scores, *Wa, *ba;
+    const void* tokens;                // [B, 1+N, Din] of the kernel's token type (float or bf16)
     int32_t* idx32;
     int64_t* idx64;
     float *Zs, *Zc, *z2s, *z2c, *z2s_ctr, *z2c_ctr, *z2s_hi, *z2c_hi;
@@ -64,7 +65,7 @@ __device__ __forceinline__ void split_row(const float* __restrict__ v, int D, fl
     }
 }
 
-template <int MAXT, int LD>
+template <int MAXT, int LD, class T>
 __global__ void __launch_bounds__(MAXT, 1)
 head_prep_kernel(const PrepArgs a) {
     pdl_sync();
@@ -156,8 +157,10 @@ head_prep_kernel(const PrepArgs a) {
     }
     __syncthreads();
 
-    // ---- 2. gather the source rows (zero rows past the end / zero padding of the k axis) ---------------------------
+    // ---- 2. gather the source rows (zero rows past the end / zero padding of the k axis); bf16 rows are widened to
+    //         fp32 on the way in (a register round trip instead of cp.async) ------------------------------------------
     {
+        const T* tokens = static_cast<const T*>(a.tokens);
         const int c4 = a.Dinp >> 2;
         for (int i = tid; i < TR * c4; i += nthr) {
             const int rl = i / c4, q = i - rl * c4;
@@ -166,7 +169,9 @@ head_prep_kernel(const PrepArgs a) {
                 const int r = r0 + rl;
                 const int b = r / (K + 1), j = r - b * (K + 1);
                 const int tok = j < K ? 1 + sel[(size_t)(b - bF) * K + j] : 0;
-                cp_async16(dst, a.tokens + ((size_t)b * (1 + N) + tok) * Din + q * 4);
+                const T* srcp = tokens + ((size_t)b * (1 + N) + tok) * Din + q * 4;
+                if constexpr (sizeof(T) == 4) cp_async16(dst, srcp);
+                else *reinterpret_cast<float4*>(dst) = ldg4_tok(srcp);
             } else {
                 *reinterpret_cast<float4*>(dst) = make_float4(0.f, 0.f, 0.f, 0.f);
             }
@@ -364,6 +369,48 @@ extern "C" int pph_head_prep_supported(int B, int N, int Din, int D, int K) {
     return prep_plan(B, N, Din, D, K, 148, &p) ? 1 : 0;
 }
 
+namespace pph {
+
+template <class T>
+static int head_prep_impl(const char* name, const float* scores, const T* tokens, const float* Wa, const float* ba,
+                          int B, int H, int N, int Din, int D, int K, float center,
+                          int32_t* idx32, int64_t* idx64,
+                          float* Zs, float* Zc, float* z2s, float* z2c, float* z2s_ctr, float* z2c_ctr,
+                          float* z2s_hi, float* z2c_hi, uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi,
+                          uint16_t* Zc_lo,
+                          const float* Pl, int P, uint16_t* Pl_hi, uint16_t* Pl_lo, float* p2l, float* p2l_ctr,
+                          float* p2l_hi,
+                          const float* Pgl, int Pg, uint16_t* Pg_hi, uint16_t* Pg_lo, float* p2g, float* p2g_ctr,
+                          float* p2g_hi, pph_stream_t stream) {
+    PPH_REQUIRE(scores && tokens && Wa && ba && idx32 && Zs && Zc && z2s && z2c, PPH_EINVAL, "%s: null pointer", name);
+    PPH_REQUIRE(H >= 1 && (P == 0 || Pl) && (Pg == 0 || Pgl) && P >= 0 && Pg >= 0, PPH_EINVAL, "%s: bad args", name);
+    PPH_REQUIRE(sizeof(T) == 4 || Din % 8 == 0, PPH_EINVAL, "%s: bf16 tokens need Din %% 8 == 0 (Din=%d)", name, Din);
+    PPH_REQUIRE(pph_head_prep_supported(B, N, Din, D, K), PPH_EUNSUP,
+                "%s: shape B=%d N=%d Din=%d D=%d K=%d (Din %% 4, D %% 8, N <= 1024)", name, B, N, Din, D, K);
+    int sms = pph_sm_count();
+    if (sms <= 0) sms = 148;
+    PrepPlan p;
+    PPH_REQUIRE(prep_plan(B, N, Din, D, K, sms, &p), PPH_EUNSUP, "%s: no plan", name);
+    PrepArgs a;
+    a.B = B; a.H = H; a.N = N; a.Din = Din; a.D = D; a.K = K; a.R = B * (K + 1);
+    a.TR = p.TR; a.KC = p.KC; a.nchunks = p.nchunks; a.Dinp = p.Dinp; a.max_img = p.max_img; a.threads = p.threads;
+    a.center = center;
+    a.scores = scores; a.tokens = tokens; a.Wa = Wa; a.ba = ba; a.idx32 = idx32; a.idx64 = idx64;
+    a.Zs = Zs; a.Zc = Zc; a.z2s = z2s; a.z2c = z2c; a.z2s_ctr = z2s_ctr; a.z2c_ctr = z2c_ctr; a.z2s_hi = z2s_hi;
+    a.z2c_hi = z2c_hi; a.Zs_hi = Zs_hi; a.Zs_lo = Zs_lo; a.Zc_hi = Zc_hi; a.Zc_lo = Zc_lo;
+    a.V[0] = Pl; a.VR[0] = Pl ? P : 0; a.Vhi[0] = Pl_hi; a.Vlo[0] = Pl_lo; a.V2[0] = p2l; a.V2ctr[0] = p2l_ctr; a.V2hi[0] = p2l_hi;
+    a.V[1] = Pgl; a.VR[1] = Pgl ? Pg : 0; a.Vhi[1] = Pg_hi; a.Vlo[1] = Pg_lo; a.V2[1] = p2g; a.V2ctr[1] = p2g_ctr; a.V2hi[1] = p2g_hi;
+    auto k_small = head_prep_kernel<256, 8, T>;
+    auto k_large = head_prep_kernel<640, 6, T>;
+    auto kern = p.threads <= 256 ? k_small : k_large;
+    cudaError_t e = opt_in_smem(kern, (int)p.smem);
+    if (e != cudaSuccess) { set_error("%s: %s", name, cudaGetErrorString(e)); return (int)e; }
+    launch_k(kern, dim3(p.grid), dim3(p.threads), p.smem, as_stream(stream), a);
+    return launch_status(name);
+}
+
+}  // namespace pph
+
 extern "C" int pph_head_prep(const float* scores, const float* tokens, const float* Wa, const float* ba,
                              int B, int H, int N, int Din, int D, int K, float center,
                              int32_t* idx32, int64_t* idx64,
@@ -374,29 +421,22 @@ extern "C" int pph_head_prep(const float* scores, const float* tokens, const flo
                              float* p2l_hi,
                              const float* Pgl, int Pg, uint16_t* Pg_hi, uint16_t* Pg_lo, float* p2g, float* p2g_ctr,
                              float* p2g_hi, pph_stream_t stream) {
-    using namespace pph;
-    PPH_REQUIRE(scores && tokens && Wa && ba && idx32 && Zs && Zc && z2s && z2c, PPH_EINVAL, "pph_head_prep: null pointer");
-    PPH_REQUIRE(H >= 1 && (P == 0 || Pl) && (Pg == 0 || Pgl) && P >= 0 && Pg >= 0, PPH_EINVAL, "pph_head_prep: bad args");
-    PPH_REQUIRE(pph_head_prep_supported(B, N, Din, D, K), PPH_EUNSUP,
-                "pph_head_prep: shape B=%d N=%d Din=%d D=%d K=%d (Din %% 4, D %% 8, N <= 1024)", B, N, Din, D, K);
-    int sms = pph_sm_count();
-    if (sms <= 0) sms = 148;
-    PrepPlan p;
-    PPH_REQUIRE(prep_plan(B, N, Din, D, K, sms, &p), PPH_EUNSUP, "pph_head_prep: no plan");
-    PrepArgs a;
-    a.B = B; a.H = H; a.N = N; a.Din = Din; a.D = D; a.K = K; a.R = B * (K + 1);
-    a.TR = p.TR; a.KC = p.KC; a.nchunks = p.nchunks; a.Dinp = p.Dinp; a.max_img = p.max_img; a.threads = p.threads;
-    a.center = center;
-    a.scores = scores; a.tokens = tokens; a.Wa = Wa; a.ba = ba; a.idx32 = idx32; a.idx64 = idx64;
-    a.Zs = Zs; a.Zc = Zc; a.z2s = z2s; a.z2c = z2c; a.z2s_ctr = z2s_ctr; a.z2c_ctr = z2c_ctr; a.z2s_hi = z2s_hi;
-    a.z2c_hi = z2c_hi; a.Zs_hi = Zs_hi; a.Zs_lo = Zs_lo; a.Zc_hi = Zc_hi; a.Zc_lo = Zc_lo;
-    a.V[0] = Pl; a.VR[0] = Pl ? P : 0; a.Vhi[0] = Pl_hi; a.Vlo[0] = Pl_lo; a.V2[0] = p2l; a.V2ctr[0] = p2l_ctr; a.V2hi[0] = p2l_hi;
-    a.V[1] = Pgl; a.VR[1] = Pgl ? Pg : 0; a.Vhi[1] = Pg_hi; a.Vlo[1] = Pg_lo; a.V2[1] = p2g; a.V2ctr[1] = p2g_ctr; a.V2hi[1] = p2g_hi;
-    auto k_small = head_prep_kernel<256, 8>;
-    auto k_large = head_prep_kernel<640, 6>;
-    auto kern = p.threads <= 256 ? k_small : k_large;
-    cudaError_t e = opt_in_smem(kern, (int)p.smem);
-    if (e != cudaSuccess) { set_error("pph_head_prep: %s", cudaGetErrorString(e)); return (int)e; }
-    launch_k(kern, dim3(p.grid), dim3(p.threads), p.smem, as_stream(stream), a);
-    return launch_status("pph_head_prep");
+    return pph::head_prep_impl("pph_head_prep", scores, tokens, Wa, ba, B, H, N, Din, D, K, center, idx32, idx64, Zs, Zc, z2s,
+                               z2c, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, Pl, P, Pl_hi, Pl_lo, p2l,
+                               p2l_ctr, p2l_hi, Pgl, Pg, Pg_hi, Pg_lo, p2g, p2g_ctr, p2g_hi, stream);
+}
+
+extern "C" int pph_head_prep_bf16tok(const float* scores, const uint16_t* tokens, const float* Wa, const float* ba,
+                                     int B, int H, int N, int Din, int D, int K, float center,
+                                     int32_t* idx32, int64_t* idx64,
+                                     float* Zs, float* Zc, float* z2s, float* z2c, float* z2s_ctr, float* z2c_ctr,
+                                     float* z2s_hi, float* z2c_hi, uint16_t* Zs_hi, uint16_t* Zs_lo, uint16_t* Zc_hi,
+                                     uint16_t* Zc_lo,
+                                     const float* Pl, int P, uint16_t* Pl_hi, uint16_t* Pl_lo, float* p2l, float* p2l_ctr,
+                                     float* p2l_hi,
+                                     const float* Pgl, int Pg, uint16_t* Pg_hi, uint16_t* Pg_lo, float* p2g, float* p2g_ctr,
+                                     float* p2g_hi, pph_stream_t stream) {
+    return pph::head_prep_impl("pph_head_prep_bf16tok", scores, tokens, Wa, ba, B, H, N, Din, D, K, center, idx32, idx64, Zs,
+                               Zc, z2s, z2c, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo, Pl, P, Pl_hi,
+                               Pl_lo, p2l, p2l_ctr, p2l_hi, Pgl, Pg, Pg_hi, Pg_lo, p2g, p2g_ctr, p2g_hi, stream);
 }

@@ -32,18 +32,21 @@ class GraphedHeadStep:
                  heads: int = 0, ppc_cov_coe: float = 0.1, ppc_mean_coe: float = 0.5, train: bool = True,
                  process_group=None, device=None, fused: bool = True, allreduce_in_graph: bool = False,
                  schedule: int | None = None, use_ppc: bool = True, impl: str = "auto", variants=None,
-                 exchange: str = "nccl"):
+                 exchange: str = "nccl", token_dtype=torch.float32):
         """params: dict with Wa (D,Din), ba (D), P (P,D), Pg (Pg,D) [leaf tensors, requires_grad in training] and
         the last layers Wl (C,P), Wg (C,Pg), frozen as in the reference unless their requires_grad is set: a training step
         then also writes their gradients (appended to the flat buffer behind ba, Wl before Wg).  ppc_*_coe follow
-        scripts/train_cub.sh:43-44."""
+        scripts/train_cub.sh:43-44.  token_dtype: torch.float32 or torch.bfloat16 (a bf16 backbone's tokens, read as they
+        are: half the bytes per token row in the slots, in `dtokens` and over the bus in load_host)."""
+        ops.token_entry("", token_dtype)
+        self.token_dtype = token_dtype
         self.p, self.cfg, self.B, self.N, self.C, self.m = params, cfg, B, N, C, m
         self.train = train
         self.cov_coe, self.mean_coe = ppc_cov_coe, ppc_mean_coe
         dev = device or params["P"].device
         Din = params["Wa"].shape[1]
         sshape = (B, heads, N) if heads > 0 else (B, N)
-        self.tokens = [torch.zeros(B, 1 + N, Din, device=dev, requires_grad=train) for _ in range(n_slots)]
+        self.tokens = [torch.zeros(B, 1 + N, Din, device=dev, dtype=token_dtype, requires_grad=train) for _ in range(n_slots)]
         self.scores = [torch.zeros(sshape, device=dev) for _ in range(n_slots)]
         self.labels = [torch.zeros(B, dtype=torch.int64, device=dev) for _ in range(n_slots)]
         self.loss = [None] * n_slots
@@ -79,12 +82,13 @@ class GraphedHeadStep:
             # impl: "v2" = the round-2 launch sequence (11 launches), "v1" = the round-1 sequence (fallback / A-B arm), "auto" = v2 if the
             # shape is inside what those kernels were built for
             if impl == "auto":
-                impl = "v2" if ops.fused_step_supported(B, N, Din, D, cfg.K, P, Pg, C, m) else "v1"
+                impl = "v2" if ops.fused_step_supported(B, N, Din, D, cfg.K, P, Pg, C, m, token_dtype) else "v1"
             self.impl = impl
             cls = ops.FusedHeadStep if impl == "v2" else ops.FusedHeadStepV1
             kw = dict(variants=variants) if impl == "v2" else {}
             self.fused = cls(cfg, B, N, Din, D, P, Pg, C, m, dev, heads=heads, ppc_cov_coe=ppc_cov_coe,
-                             ppc_mean_coe=ppc_mean_coe, train=train, use_ppc=use_ppc, schedule=schedule, **kw)
+                             ppc_mean_coe=ppc_mean_coe, train=train, use_ppc=use_ppc, schedule=schedule,
+                             token_dtype=token_dtype, **kw)
             if train:
                 self.grads = dict(zip((n for n, _ in self.reducer.named), self.reducer.views))
 
@@ -176,7 +180,8 @@ class GraphedHeadStep:
 
     # --------------------------------------------------------------------------------------------------------
     def load(self, slot: int, tokens, scores, labels):
-        """Asynchronous copy of one batch into the slot (host tensors should be pinned)."""
+        """Asynchronous copy of one batch into the slot (host tensors should be pinned); the tokens are converted to the
+        slot's dtype (`token_dtype`) by the copy."""
         with torch.no_grad():
             self.tokens[slot].copy_(tokens, non_blocking=True)
             self.scores[slot].copy_(scores, non_blocking=True)
@@ -248,9 +253,12 @@ class GraphedHeadStep:
         """Selection-first transfer of one batch from PINNED host tensors (current stream): scores and labels by copy,
         the top-K ranking on the device, then only the CLS row and the K selected rows of every image are read out of
         the host buffer by a gather kernel (pph_gather_rows_host).  The slot's other token rows keep stale values that
-        neither the forward nor the backward reads.  Returns the bytes that crossed the bus."""
+        neither the forward nor the backward reads.  `tokens` has the step's token dtype (bf16 rows move half the bytes).
+        Returns the bytes that crossed the bus."""
         from . import _lib
-        assert tokens.is_pinned() and tokens.is_contiguous() and tokens.dtype == torch.float32
+        assert tokens.is_pinned() and tokens.is_contiguous()
+        if tokens.dtype != self.token_dtype:
+            raise TypeError(f"load_host: this step holds {self.token_dtype} tokens, got {tokens.dtype} (no conversion on this path)")
         if not hasattr(self, "_load_idx"):
             self._load_idx = [torch.empty(self.B, self.cfg.K, dtype=torch.int32, device=self.tokens[0].device)
                               for _ in self.tokens]
@@ -261,9 +269,16 @@ class GraphedHeadStep:
             self.scores[slot].copy_(scores, non_blocking=True)
             self.labels[slot].copy_(labels, non_blocking=True)
             _lib.call("pph_select_topk", self.scores[slot], B, H, N, K, self._load_idx[slot], None)
-            _lib.call("pph_gather_rows_host", tokens.data_ptr(), self._load_idx[slot], B, N, Din, K,
-                      self.tokens[slot].detach(), n_ctas)
-        return scores.numel() * 4 + labels.numel() * 8 + B * (K + 1) * Din * 4
+            _lib.call(ops.token_entry("pph_gather_rows_host", tokens.dtype), tokens.data_ptr(), self._load_idx[slot], B, N,
+                      Din, K, self.tokens[slot].detach(), n_ctas)
+        return self.host_transfer_bytes(tokens, scores, labels, K)
+
+    @staticmethod
+    def host_transfer_bytes(tokens, scores, labels, K: int) -> int:
+        """Bytes load_host moves over the bus for one batch: scores (fp32) and labels (int64) whole, and the CLS row plus the
+        K selected rows of every image in the tokens' own dtype (bf16 rows are half the bytes of fp32 rows)."""
+        B, Din = tokens.shape[0], tokens.shape[-1]
+        return scores.numel() * 4 + labels.numel() * 8 + B * (K + 1) * Din * tokens.element_size()
 
     def capture_load_host(self, slot: int, tokens, scores, labels, n_ctas: int = 48):
         """load_host() of one fixed (slot, pinned staging buffer) pair recorded as a CUDA graph: a caller that cycles

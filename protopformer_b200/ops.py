@@ -40,6 +40,37 @@ def _empty(shape, dtype, like):
     return torch.empty(shape, dtype=dtype, device=like.device)
 
 
+TOKEN_DTYPES = (torch.float32, torch.bfloat16)
+
+
+def token_entry(name: str, dtype) -> str:
+    """The entry point that reads backbone tokens of `dtype`: `name` itself for float32, its bf16 twin (`name` + "_bf16tok",
+    include/protohead.h) for bfloat16.  Any other dtype raises TypeError here, before anything is launched."""
+    if dtype == torch.float32:
+        return name
+    if dtype == torch.bfloat16:
+        return name + _lib.BF16TOK
+    raise TypeError(f"backbone tokens must be torch.float32 or torch.bfloat16, got {dtype} "
+                    "(fp16 tokens are taken only inside an autocast region, which casts them to float32)")
+
+
+def _autocast_casts() -> bool:
+    """Inside a CUDA autocast region the head's autograd functions cast their floating inputs to float32 (custom_fwd)."""
+    return torch.is_autocast_enabled("cuda")
+
+
+def check_head_dtypes(tokens, *params):
+    """Refuse, before any launch, what the kernels cannot read: tokens other than float32 / bfloat16 and head parameters
+    other than float32.  Inside an autocast region nothing is refused: the float32 cast policy applies there as before."""
+    if _autocast_casts():
+        return
+    token_entry("", tokens.dtype)
+    for p in params:
+        if p is not None and p.dtype != torch.float32:
+            raise TypeError(f"prototype-head parameters must be torch.float32, got {p.dtype} of shape {tuple(p.shape)} "
+                            "(bf16 backbone tokens are supported; bf16 head parameters are not)")
+
+
 def tc_supported(D: int, K: int) -> bool:
     """Shapes the tcgen05 similarity kernel was built for (include/protohead.h, pph_similarity_fwd)."""
     return D % 64 == 0 and 64 <= D <= 512 and 1 <= K <= 256
@@ -155,6 +186,7 @@ class _Addon(torch.autograd.Function):
         B, n1, Din = tokens.shape
         N, K, D = n1 - 1, idx32.shape[1], Wa.shape[0]
         f32, bf = torch.float32, torch.bfloat16
+        check_head_dtypes(tokens, Wa, ba)
         Zs, Zc = _empty((B, K, D), f32, tokens), _empty((B, D), f32, tokens)
         z2s, z2c = _empty((B, K), f32, tokens), _empty((B,), f32, tokens)
         if want_split:
@@ -164,7 +196,7 @@ class _Addon(torch.autograd.Function):
             Zc_hi, Zc_lo = _empty((B, D), bf, tokens), _empty((B, D), bf, tokens)
         else:
             z2s_ctr = z2c_ctr = z2s_hi = z2c_hi = Zs_hi = Zs_lo = Zc_hi = Zc_lo = None
-        _lib.call("pph_addon_fwd", tokens, idx32, Wa, ba, B, N, Din, D, K, Zs, Zc, z2s, z2c, float(center),
+        _lib.call(token_entry("pph_addon_fwd", tokens.dtype), tokens, idx32, Wa, ba, B, N, Din, D, K, Zs, Zc, z2s, z2c, float(center),
                   z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo)
         ctx.save_for_backward(tokens, idx32, Wa, Zs, Zc)
         ctx.dims = (B, N, Din, D, K)
@@ -188,13 +220,13 @@ class _Addon(torch.autograd.Function):
             # measured 3e-4 (scripts/measure_tolerances.py); they take the pre-activation gradient
             dpre_s, dpre_c = dZs * Zs * (1.0 - Zs), dZc * Zc * (1.0 - Zc)
             ws = _cached_zero_ws("pph_addon_tc2_ws_bytes", (B, N, Din, D, K), tokens.device)
-            dtok = torch.zeros_like(tokens) if want_dtok else None
-            _lib.call("pph_addon_bwd3", 1 | (2 if want_dtok else 0), tokens, idx32, Wa, dpre_s, dpre_c, None, B, N, Din, D, K,
+            dtok = torch.zeros_like(tokens) if want_dtok else None       # a bf16 leaf gets a bf16 gradient
+            _lib.call(token_entry("pph_addon_bwd3", tokens.dtype), 1 | (2 if want_dtok else 0), tokens, idx32, Wa, dpre_s, dpre_c, None, B, N, Din, D, K,
                       ws, dWa, dba, dtok)
             return dtok, None, dWa, dba, None, None
         dtok = torch.empty_like(tokens) if want_dtok else None
         ws = addon_bwd_workspace(B, N, Din, D, K, tokens.device)
-        _lib.call("pph_addon_bwd", tokens, idx32, Wa, Zs, Zc, dZs, dZc, B, N, Din, D, K, ws,
+        _lib.call(token_entry("pph_addon_bwd", tokens.dtype), tokens, idx32, Wa, Zs, Zc, dZs, dZc, B, N, Din, D, K, ws,
                   1 | (2 if dtok is not None else 0), dWa, dba, dtok)
         return dtok, None, dWa, dba, None, None
 
@@ -232,7 +264,8 @@ class TokenFeatures:
 
 
 def addon(tokens, idx32, Wa, ba, want_split: bool, center: float = 0.5) -> TokenFeatures:
-    """tokens (B,1+N,Din), idx32 (B,K), Wa (D,Din) or (D,Din,1,1), ba (D)."""
+    """tokens (B,1+N,Din) float32 or bfloat16, idx32 (B,K), Wa (D,Din) or (D,Din,1,1), ba (D)."""
+    check_head_dtypes(tokens, Wa, ba)
     Wa2 = Wa.reshape(Wa.shape[0], -1)
     out = _Addon.apply(tokens, idx32, Wa2, ba, want_split, center)
     Zs, Zc, z2s, z2c, z2s_ctr, z2c_ctr, z2s_hi, z2c_hi, Zs_hi, Zs_lo, Zc_hi, Zc_lo = out
@@ -389,9 +422,11 @@ class HeadOutput:
 def head_forward(cfg: HeadConfig, tokens, scores, Wa, ba, P, Pg, Wl, Wg) -> HeadOutput:
     """The whole prototype head after the backbone: selection -> add-on -> similarity/pool -> logits.
 
-    tokens (B,1+N,Din), scores (B,N)|(B,H,N), Wa (D,Din[,1,1]), ba (D), P (P,D[,1,1]), Pg (Pg,D[,1,1]),
-    Wl (C,P), Wg (C,Pg).  Replaces protopformer.py:156-172 + 311-316.
+    tokens (B,1+N,Din) float32 or bfloat16 (a bf16 backbone's output, read as it is), scores (B,N)|(B,H,N),
+    Wa (D,Din[,1,1]), ba (D), P (P,D[,1,1]), Pg (Pg,D[,1,1]), Wl (C,P), Wg (C,Pg) float32.
+    Replaces protopformer.py:156-172 + 311-316.
     """
+    check_head_dtypes(tokens, Wa, ba, P, Pg, Wl, Wg)
     if tokens.shape[0] == 0:
         return _empty_head_output(cfg, tokens, Wa, P, Pg, Wl)
     idx32 = select_topk(scores, cfg.K)
@@ -548,6 +583,16 @@ def _last_layer_grad_targets(train: bool, Wl, Wg, grads):
     return tuple(out)
 
 
+def _step_token_entries(step, tokens, *params):
+    """Host-side checks of a fused step's inputs (before any launch) -> name -> the entry point for the step's token type."""
+    if tokens.dtype != step.token_dtype:
+        token_entry("", tokens.dtype)
+        raise TypeError(f"this step was built for {step.token_dtype} tokens, got {tokens.dtype} "
+                        "(pass token_dtype= to the constructor)")
+    check_head_dtypes(tokens, *params)
+    return lambda name: token_entry(name, step.token_dtype)
+
+
 class FusedHeadStepV1:
     """Round-1 launch sequence (16 launches over three streams), kept as the fallback for shapes the round-2 step (FusedHeadStep)
     was not built for and as an A/B arm.  forward (+ PPC + cross-entropy + backward) of the head for a fixed shape.
@@ -561,9 +606,11 @@ class FusedHeadStepV1:
     grad: pph_last_layer_wgrad right after the loss tail)."""
 
     def __init__(self, cfg: HeadConfig, B, N, Din, D, P, Pg, C, m, device, heads: int = 0, ppc_cov_coe: float = 0.1,
-                 ppc_mean_coe: float = 0.5, train: bool = True, use_ppc: bool = True, schedule: int | None = None):
+                 ppc_mean_coe: float = 0.5, train: bool = True, use_ppc: bool = True, schedule: int | None = None,
+                 token_dtype=torch.float32):
         import os
-        self.cfg, self.train, self.use_ppc = cfg, train, use_ppc
+        token_entry("", token_dtype)
+        self.cfg, self.train, self.use_ppc, self.token_dtype = cfg, train, use_ppc, token_dtype
         # stream schedule of the training step: 1 (default) = three streams (token bins on their own branch, the
         # cross-entropy tail does not wait for the PPC loss: the weighted sum is a separate 1-thread kernel on the
         # side branch, PPC gradient buffer cleared at the start of the step); 0 = the first round-1 schedule, two
@@ -600,7 +647,7 @@ class FusedHeadStepV1:
             self.dlogits, self.g_l, self.g_g = e(B, C), e(B, P), e(B, Pg)
             self.dZs, self.dZc = e(B, K, D), e(B, D)
             self.dZs_ppc, self.dP_ppc = e(B, K, D), z(P, D)
-            self.dtokens = e(B, 1 + N, Din)
+            self.dtokens = e(B, 1 + N, Din, dt=token_dtype)
             self.ws = bwd_workspace(B, K, D, P, Pg, device)
             self.ws_addon = addon_bwd_workspace(B, N, Din, D, K, device)
         # independent kernels run on a forked stream (under CUDA-graph capture this becomes a parallel branch)
@@ -612,6 +659,7 @@ class FusedHeadStepV1:
         B, N, Din, D, Pn, Pgn, C, m, H = self.dims
         cfg, K = self.cfg, self.cfg.K
         c = _lib.call
+        tok = _step_token_entries(self, tokens, Wa, ba, P, Pg, Wl, Wg)
         main, side, ev = torch.cuda.current_stream(), self.side, self.ev
         sched1 = self.schedule == 1 and self.use_ppc and self.train
         # branch: prototype operand preparation || selection + add-on
@@ -624,7 +672,7 @@ class FusedHeadStepV1:
             c("pph_split_rows", Pg, Pgn, D, float(cfg.center), self.Pg_hi, self.Pg_lo, self.pg2, self.pg2_ctr, self.pg2_hi)
             ev[1].record(side)
         c("pph_select_topk", scores, B, max(H, 1), N, K, self.idx32, None)
-        c("pph_addon_fwd", tokens, self.idx32, Wa, ba, B, N, Din, D, K, self.Zs, self.Zc, self.z2s, self.z2c,
+        c(tok("pph_addon_fwd"), tokens, self.idx32, Wa, ba, B, N, Din, D, K, self.Zs, self.Zc, self.z2s, self.z2c,
           float(cfg.center), self.z2s_ctr, self.z2c_ctr, self.z2s_hi, self.z2c_hi, self.Zs_hi, self.Zs_lo,
           self.Zc_hi, self.Zc_lo)
         main.wait_event(ev[1])
@@ -703,10 +751,10 @@ class FusedHeadStepV1:
         ev[5].record(main)
         side.wait_event(ev[5])
         with torch.cuda.stream(side):
-            c("pph_addon_bwd", tokens, self.idx32, Wa, self.Zs, self.Zc, self.dZs, self.dZc, B, N, Din, D, K,
+            c(tok("pph_addon_bwd"), tokens, self.idx32, Wa, self.Zs, self.Zc, self.dZs, self.dZc, B, N, Din, D, K,
               self.ws_addon, 2, None, None, self.dtokens)
             ev[6].record(side)
-        c("pph_addon_bwd", tokens, self.idx32, Wa, self.Zs, self.Zc, self.dZs, self.dZc, B, N, Din, D, K,
+        c(tok("pph_addon_bwd"), tokens, self.idx32, Wa, self.Zs, self.Zc, self.dZs, self.dZc, B, N, Din, D, K,
           self.ws_addon, 1, grads["Wa"], grads["ba"], None)
         main.wait_event(ev[6])
         return self.losses
@@ -724,10 +772,10 @@ def _ws(fn: str, *dims, zero: bool, device) -> torch.Tensor:
     return alloc(max(int(n.value), 256), dtype=torch.uint8, device=device)
 
 
-def fused_step_supported(B, N, Din, D, K, P, Pg, C, m) -> bool:
+def fused_step_supported(B, N, Din, D, K, P, Pg, C, m, token_dtype=torch.float32) -> bool:
     """Host-side check (no device needed): can FusedHeadStep (the round-2 launch sequence) run this shape?"""
     lib = _lib.load()
-    if C > 256 or B < 1 or B > 64 * 74:
+    if C > 256 or B < 1 or B > 64 * 74 or (token_dtype == torch.bfloat16 and Din % 8 != 0):
         return False
     ppc_smem = 4 * (m * D + K * (D + 4) + 2 * m * K + 8 * m + 32)
     return bool(lib.pph_head_prep_supported(B, N, Din, D, K) and lib.pph_addon_bwd2_supported(B, N, Din, D, K)
@@ -759,10 +807,12 @@ class FusedHeadStep:
     grad; with both frozen, the default, the step is exactly the 11 launches above).  Reference: tools/engine_proto.py:49-76."""
 
     def __init__(self, cfg: HeadConfig, B, N, Din, D, P, Pg, C, m, device, heads: int = 0, ppc_cov_coe: float = 0.1,
-                 ppc_mean_coe: float = 0.5, train: bool = True, use_ppc: bool = True, schedule=None, variants=None):
-        if not fused_step_supported(B, N, Din, D, cfg.K, P, Pg, C, m):
+                 ppc_mean_coe: float = 0.5, train: bool = True, use_ppc: bool = True, schedule=None, variants=None,
+                 token_dtype=torch.float32):
+        token_entry("", token_dtype)
+        if not fused_step_supported(B, N, Din, D, cfg.K, P, Pg, C, m, token_dtype):
             raise ValueError("shape outside FusedHeadStep's kernels: use FusedHeadStepV1")
-        self.cfg, self.train, self.use_ppc = cfg, train, use_ppc
+        self.cfg, self.train, self.use_ppc, self.token_dtype = cfg, train, use_ppc, token_dtype
         # kernel choice per stage: "tc" = single-shot tcgen05 kernels (pph_addon_fwd2 / pph_addon_bwd3) where the shape
         # allows, "simt" = the exact-FP32 CUDA-core kernels (pph_head_prep / pph_addon_bwd2)
         tc_bits = _lib.load().pph_addon_tc2_supported(B, N, Din, D, cfg.K)
@@ -831,7 +881,7 @@ class FusedHeadStep:
             if use_ppc:
                 self.dZs_ppc, self.dP_img = e(B, K, D), e(B, m, D)
             self.dZs, self.dZc = e(B, K, D), e(B, D)
-            self.dtokens = e(B, 1 + N, Din)
+            self.dtokens = e(B, 1 + N, Din, dt=token_dtype)
             self.ws_addon = _ws("pph_addon_bwd2_ws_bytes", B, N, Din, D, K, zero=True, device=device)
             if self.variants["addon_bwd"] == "tc":
                 self.dtokens.zero_()
@@ -852,6 +902,7 @@ class FusedHeadStep:
         B, N, Din, D, Pn, Pgn, C, m, H = self.dims
         cfg, K = self.cfg, self.cfg.K
         c = _lib.call
+        tok = _step_token_entries(self, tokens, Wa, ba, P, Pg, Wl, Wg)
         main, side, side2, ev = torch.cuda.current_stream(), self.side, self.side2, self.ev
         hook = reduce_hook or (lambda which: None)
 
@@ -875,18 +926,18 @@ class FusedHeadStep:
             if self.variants["prep"] == "tc1":
                 if idx32 is None:
                     c("pph_select_topk", scores, B, max(H, 1), N, K, sel_idx, None)
-                c("pph_addon_fwd", tokens, sel_idx, Wa, ba, B, N, Din, D, K, self.Zs, self.Zc, self.z2s, self.z2c,
+                c(tok("pph_addon_fwd"), tokens, sel_idx, Wa, ba, B, N, Din, D, K, self.Zs, self.Zc, self.z2s, self.z2c,
                   float(cfg.center), self.z2s_ctr, self.z2c_ctr, self.z2s_hi, self.z2c_hi, self.Zs_hi, self.Zs_lo,
                   self.Zc_hi, self.Zc_lo)
             elif idx32 is None and self.variants["select"] == "fused":
                 # the ranking runs in the add-on kernel's prologue: one launch for protopformer.py:157-172
-                c("pph_select_addon_fwd", scores, max(H, 1), tokens, Wa, ba, B, N, Din, D, K, sel_idx, self.Zs, self.Zc,
+                c(tok("pph_select_addon_fwd"), scores, max(H, 1), tokens, Wa, ba, B, N, Din, D, K, sel_idx, self.Zs, self.Zc,
                   self.z2s, self.z2c, float(cfg.center), self.z2s_ctr, self.z2c_ctr, self.z2s_hi, self.z2c_hi, self.Zs_hi,
                   self.Zs_lo, self.Zc_hi, self.Zc_lo, self.ws_tc)
             else:
                 if idx32 is None:
                     c("pph_select_topk", scores, B, max(H, 1), N, K, sel_idx, None)
-                c("pph_addon_fwd2", tokens, sel_idx, Wa, ba, B, N, Din, D, K, self.Zs, self.Zc, self.z2s, self.z2c,
+                c(tok("pph_addon_fwd2"), tokens, sel_idx, Wa, ba, B, N, Din, D, K, self.Zs, self.Zc, self.z2s, self.z2c,
                   float(cfg.center), self.z2s_ctr, self.z2c_ctr, self.z2s_hi, self.z2c_hi, self.Zs_hi, self.Zs_lo,
                   self.Zc_hi, self.Zc_lo, self.ws_tc)
             main.wait_event(ev[4])
@@ -898,7 +949,7 @@ class FusedHeadStep:
                     self.dtokens.zero_()
                     ev[4].record(side)
                 last_layer_pattern()
-            c("pph_head_prep", scores, tokens, Wa, ba, B, max(H, 1), N, Din, D, K, float(cfg.center), sel_idx, None,
+            c(tok("pph_head_prep"), scores, tokens, Wa, ba, B, max(H, 1), N, Din, D, K, float(cfg.center), sel_idx, None,
               self.Zs, self.Zc, self.z2s, self.z2c, self.z2s_ctr, self.z2c_ctr, self.z2s_hi, self.z2c_hi,
               self.Zs_hi, self.Zs_lo, self.Zc_hi, self.Zc_lo,
               P, Pn, self.P_hi, self.P_lo, self.p2, self.p2_ctr, self.p2_hi,
@@ -1016,11 +1067,11 @@ class FusedHeadStep:
             # token gradient (82 CTAs) then weight gradient (112 CTAs behind a grid barrier): both want one CTA per SM, as
             # graph branches they only time-slice the machine (measured), so they run back to back
             def dgrad():
-                c("pph_addon_bwd3", 2, tokens, sel_idx, Wa, self.dZs, self.dZc, dpre_add, B, N, Din, D, K, self.ws_tc,
+                c(tok("pph_addon_bwd3"), 2, tokens, sel_idx, Wa, self.dZs, self.dZc, dpre_add, B, N, Din, D, K, self.ws_tc,
                   None, None, self.dtokens)
 
             def wgrad():
-                c("pph_addon_bwd3", 1, tokens, sel_idx, Wa, self.dZs, self.dZc, dpre_add, B, N, Din, D, K, self.ws_tc,
+                c(tok("pph_addon_bwd3"), 1, tokens, sel_idx, Wa, self.dZs, self.dZc, dpre_add, B, N, Din, D, K, self.ws_tc,
                   grads["Wa"], grads["ba"], None)
 
             if reduce_hook is not None:     # weight gradient first: its exchange then runs under the token gradient
@@ -1036,7 +1087,7 @@ class FusedHeadStep:
                 dgrad()
                 wgrad()
         else:
-            c("pph_addon_bwd2", 3, tokens, sel_idx, Wa, self.dZs, self.dZc, B, N, Din, D, K,
+            c(tok("pph_addon_bwd2"), 3, tokens, sel_idx, Wa, self.dZs, self.dZc, B, N, Din, D, K,
               self.ws_addon, grads["Wa"], grads["ba"], self.dtokens)
             hook("addon")
         main.wait_event(ev[1])
