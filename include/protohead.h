@@ -14,7 +14,8 @@
  *   - return 0 on success, a negative PPH_E* argument error, or a positive cudaError_t from the launch.
  *     pph_last_error_string() describes the last non-zero return on the calling thread.
  *   - there is NO CPU fallback: without a CUDA device every compute entry point returns a cudaError_t.
- *   - float tensors are fp32 row-major contiguous; "bf16" is the 16-bit brain float (uint16_t storage).
+ *   - float tensors are fp32 row-major contiguous; "bf16" is the 16-bit brain float (uint16_t storage); "f16" is
+ *     IEEE binary16 (uint16_t storage).
  *
  * Symbols (B images, N patch tokens, K reserved tokens, Din backbone width, D prototype dim, P local
  * prototypes, Pg global prototypes, C classes, m = P / C prototypes per class):
@@ -253,6 +254,27 @@ int pph_adamw_step(int n_seg, float* const* params, const float* const* grads, f
  * pph_rollout_scores(patch_layers, ..., T = Tc-1, v0, drop_first = 0) = `cls_attn_ma[:, 0]` (cait_models_attn.py:328-330). */
 int pph_rollout_cls_rows(const float* const* cls_layers /* host array of device pointers */, int n_cls, int B, int H,
                          int Tc, int k_discard, int head_fusion, float identity_w, float* v0, pph_stream_t stream);
+
+/* Half-precision attention maps (a bf16 backbone, or one run under fp16 autocast): twins of pph_rollout_scores and
+ * pph_rollout_cls_rows whose layer tables point at bf16 ("_bf16attn") or f16 ("_f16attn") maps of the same layout.
+ * Every bf16 and f16 value is exact in fp32: the kernels widen each map value at its load and nothing after the load
+ * changes (head fusion, discard, normalisation and chain in fp32), so every output equals, bit for bit, the fp32
+ * entry's on the widened maps.  Arguments, argument checks and error codes, pph_rollout_ws_bytes, the "rollout" kernel
+ * versions and the launch count are the fp32 entry's; scores and v0 stay fp32.  No fp32 copy of the maps is made. */
+int pph_rollout_scores_bf16attn(const uint16_t* const* attn_layers /* host array of device pointers */, int L, int B,
+                                int H, int T, int k_discard, int head_fusion, float identity_w, const float* v0,
+                                int drop_first, void* workspace, float* scores, int K, int32_t* idx32, int64_t* idx64,
+                                pph_stream_t stream);
+int pph_rollout_scores_f16attn(const uint16_t* const* attn_layers /* host array of device pointers */, int L, int B,
+                               int H, int T, int k_discard, int head_fusion, float identity_w, const float* v0,
+                               int drop_first, void* workspace, float* scores, int K, int32_t* idx32, int64_t* idx64,
+                               pph_stream_t stream);
+int pph_rollout_cls_rows_bf16attn(const uint16_t* const* cls_layers /* host array of device pointers */, int n_cls,
+                                  int B, int H, int Tc, int k_discard, int head_fusion, float identity_w, float* v0,
+                                  pph_stream_t stream);
+int pph_rollout_cls_rows_f16attn(const uint16_t* const* cls_layers /* host array of device pointers */, int n_cls,
+                                 int B, int H, int Tc, int k_discard, int head_fusion, float identity_w, float* v0,
+                                 pph_stream_t stream);
 
 /* (next #4, consumers of the materialised map) eval_interpretability.py:195-225 / main_visualize.py:343-388:
  * activation maps of the m prototypes of each image's label on the ORIGINAL side x side token grid, zeros on pruned

@@ -77,6 +77,10 @@ BF16TOK = "_bf16tok"
 BF16TOK_TWINS = ("pph_addon_fwd", "pph_addon_bwd", "pph_addon_fwd2", "pph_select_addon_fwd", "pph_addon_bwd3",
                  "pph_head_prep", "pph_addon_bwd2", "pph_gather_rows_host")
 SIGNATURES.update({n + BF16TOK: SIGNATURES[n] for n in BF16TOK_TWINS})
+# half-precision attention-map twins of the rollout entry points: same arguments, bf16 / f16 map tables
+ATTN_TWINS = {torch.bfloat16: "_bf16attn", torch.float16: "_f16attn"}
+SIGNATURES.update({n + sfx: SIGNATURES[n] for n in ("pph_rollout_scores", "pph_rollout_cls_rows")
+                   for sfx in ATTN_TWINS.values()})
 _RESTYPES = {"pph_last_error_string": C.c_char_p}
 
 # kernels launched per entry-point call (memset nodes are not counted); used for the bench's `gpu_launches` claim
@@ -149,7 +153,10 @@ def call(name: str, *args):
     conv = [(C.cast(a, C.c_void_p) if isinstance(a, C.Array) else a) for a in conv]      # host pointer tables
     rc = getattr(lib, name)(*conv, _stream())
     global _launches
-    base = name[:-len(BF16TOK)] if name.endswith(BF16TOK) else name      # a twin launches what its fp32 entry launches
+    base = name                                                         # a twin launches what its fp32 entry launches
+    for sfx in (BF16TOK, *ATTN_TWINS.values()):
+        if name.endswith(sfx):
+            base = name[:-len(sfx)]
     if base == "pph_similarity_fwd":
         _launches += 2 if conv[0] == MODE_FP32_FMA else 1      # local + global kernels vs one fused tcgen05 kernel
     elif base == "pph_similarity_bwd":

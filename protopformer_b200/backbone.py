@@ -11,7 +11,8 @@ transformer blocks themselves stay the backbone's own modules -- they are out of
     patch_deit_features(ppnet.features)        # binds the method below over the reference's one; same signature
     patch_cait_features(ppnet.features)        # ... the CaiT form (tools/cait_models_attn.py:310-343)
 
-Not differentiable through the score, exactly like the reference (``attn_rollout.detach()``, :225).
+Not differentiable through the score, exactly like the reference (``attn_rollout.detach()``, :225).  The blocks' maps are
+passed as they come: a bf16 or fp16 backbone's maps are read in that precision, without an fp32 copy.
 """
 from __future__ import annotations
 

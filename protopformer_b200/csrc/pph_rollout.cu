@@ -16,7 +16,9 @@
 //    one CTA per image: v = e_0 (or a caller-supplied start row, the CaiT variant cait_models_attn.py:255-259);
 //    for l = L-1 .. 0: v <- v @ a_l as a gather over the columns' entry lists (one warp per column, fixed summation
 //    order -> bit-reproducible); scores[b, :] = v[1:] (or all of v).
+#include <cuda_fp16.h>
 #include <math.h>
+#include <stdio.h>
 #include <stdlib.h>
 
 #include "pph_common.cuh"
@@ -28,9 +30,16 @@ constexpr int kRoMaxLayers = 32;
 constexpr int kRoMaxT = 224;              // T*T*4 B must fit in shared memory beside the scratch
 constexpr int kRoChainThreads = 512;
 
+// Attention maps of element type E: float, __nv_bfloat16 or __half.  Every bf16 and fp16 value is exact in fp32, so
+// a half-precision map is widened at its load and nothing after the load changes: the results equal, bit for bit,
+// those of the fp32 maps holding the widened values.
+template <class E>
 struct RoLayers {
-    const float* p[kRoMaxLayers];
+    const E* p[kRoMaxLayers];
 };
+__device__ __forceinline__ float ro_f32(float x) { return x; }
+__device__ __forceinline__ float ro_f32(__nv_bfloat16 x) { return __bfloat162float(x); }
+__device__ __forceinline__ float ro_f32(__half x) { return __half2float(x); }
 
 struct RoWorkspace {
     int32_t* col_ptr;      // [L*B][T+1]
@@ -67,6 +76,82 @@ __device__ __forceinline__ uint32_t ro_key(float x) {
     return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
 }
 
+// Step 1 of the prepare kernels for half-precision maps (E = __nv_bfloat16 / __half): stream the H head maps of one
+// (layer, image) tile and fuse them into M exactly as the fp32 loop does (fp32 arithmetic, heads in order 0..H-1, the
+// mean as sum / H).  A thread holds 16 elements (8 fp32 registers' worth of 4-byte words) per head: the fp32 loop's
+// 32*H bytes in flight without its register count, which the 64-register budget of a 1024-thread CTA cannot grow.
+// Words: a per-(image, head) slab starts at element (b*H + h)*T*T, odd for odd T*T, so a slab is only 2-byte aligned
+// and the heads fused in one register can have different alignments.  Each slab is read as the 4-byte words of its
+// own alignment (word j holds elements 2j - odd and 2j + 1 - odd); on an odd slab the element pair of a thread is the
+// upper half of its word and the lower half of the next lane's, fetched by one shuffle.  Warp w covers element pairs
+// [256 w, 256 w + 256) of a 16384-element chunk, lane-major per step i, so lane 31's next word is lane 0's word of step
+// i + 1, and of step 8 for i = 7 (one more word, loaded by lane 0).  A word is loaded when it holds an element of the
+// slab; being 4-byte aligned, it never crosses an allocation granule.
+__device__ __forceinline__ float ro_lo(uint32_t w, __nv_bfloat16) { return __uint_as_float(w << 16); }
+__device__ __forceinline__ float ro_hi(uint32_t w, __nv_bfloat16) { return __uint_as_float(w & 0xffff0000u); }
+__device__ __forceinline__ float ro_lo(uint32_t w, __half) { return __low2float(*reinterpret_cast<const __half2*>(&w)); }
+__device__ __forceinline__ float ro_hi(uint32_t w, __half) { return __high2float(*reinterpret_cast<const __half2*>(&w)); }
+
+template <int HT, class E>
+__device__ __forceinline__ void ro_stream_fuse_half(const E* A, int n, int Hh, int head_fusion, float* M) {
+    static_assert(sizeof(E) == 2, "half-precision maps");
+    constexpr int kChunk = 16 * kRoThreads;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int e0 = 0; e0 < n; e0 += kChunk) {
+        const int j0 = (e0 >> 1) + warp * 256 + lane;          // word of step i: j0 + 32 i
+        float s[16];
+#pragma unroll (HT > 0 ? HT : 1)                                   // runtime H: no unrolling (64-register budget)
+        for (int h = 0; h < Hh; ++h) {
+            const E* S = A + (size_t)h * n;
+            const int odd = (int)((reinterpret_cast<uintptr_t>(S) >> 1) & 1);      // uniform over the CTA
+            const uint32_t* W = reinterpret_cast<const uint32_t*>(S - odd);
+            uint32_t w[8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                const int j = j0 + 32 * i;
+                w[i] = 2 * j - odd < n ? __ldcs(W + j) : 0u;
+            }
+            if (odd) {
+                const int j8 = j0 + 256;                                 // lane 0: the word after the warp's range
+                const uint32_t w8 = lane == 0 && 2 * j8 - 1 < n ? __ldcs(W + j8) : 0u;
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    const uint32_t nb = __shfl_sync(0xffffffffu, lane == 0 ? (i < 7 ? w[i + 1] : w8) : w[i], (lane + 1) & 31);
+                    w[i] = __byte_perm(w[i], nb, 0x5432);               // (upper half of w[i], lower half of nb)
+                }
+            }
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+                const float x0 = ro_lo(w[i], E()), x1 = ro_hi(w[i], E());
+                if (h == 0) {
+                    s[2 * i] = x0;
+                    s[2 * i + 1] = x1;
+                } else if (head_fusion == 0) {
+                    s[2 * i] += x0;
+                    s[2 * i + 1] += x1;
+                } else if (head_fusion == 1) {
+                    s[2 * i] = fmaxf(s[2 * i], x0);
+                    s[2 * i + 1] = fmaxf(s[2 * i + 1], x1);
+                } else {
+                    s[2 * i] = fminf(s[2 * i], x0);
+                    s[2 * i + 1] = fminf(s[2 * i + 1], x1);
+                }
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int e = 2 * (j0 + 32 * i);
+            const float a = head_fusion == 0 ? s[2 * i] / (float)Hh : s[2 * i];
+            const float c = head_fusion == 0 ? s[2 * i + 1] / (float)Hh : s[2 * i + 1];
+            if (e + 1 < n) {
+                *reinterpret_cast<float2*>(M + e) = make_float2(a, c);      // e even: 8-byte aligned
+            } else if (e < n) {
+                M[e] = a;
+            }
+        }
+    }
+}
+
 // exclusive scan of one value per thread over the whole CTA (kRoThreads threads); `wsum` = 32 ints of scratch
 __device__ __forceinline__ int block_excl_scan(int v, int* wsum, int& total) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -96,9 +181,11 @@ __device__ __forceinline__ int block_excl_scan(int v, int* wsum, int& total) {
     return r;
 }
 
-template <int HT>      // HT > 0: compile-time head count (the head loop unrolls, 8*HT loads in flight); 0: runtime H
+// HT > 0: compile-time head count (the head loop unrolls, 8*HT loads in flight); 0: runtime H.  E: element type of the
+// maps (fp32 is streamed below, half precision by ro_stream_fuse_half).
+template <int HT, class E>
 __global__ void __launch_bounds__(kRoThreads, 1)
-rollout_prepare_kernel(const RoLayers layers, int L, int B, int H, int T, int k_discard, int head_fusion,
+rollout_prepare_kernel(const RoLayers<E> layers, int L, int B, int H, int T, int k_discard, int head_fusion,
                        float identity_w, int cap, int32_t* __restrict__ col_ptr, float* __restrict__ ent_val,
                        uint16_t* __restrict__ ent_row) {
     pdl_sync();
@@ -120,30 +207,34 @@ rollout_prepare_kernel(const RoLayers layers, int L, int B, int H, int T, int k_
     for (int tile = blockIdx.x; tile < L * B; tile += gridDim.x) {
         const int l = tile / B, b = tile - l * B;
         // ---- 1. stream the H head maps once, fuse (deit_models_attn.py:102-107); 8 x H loads in flight per thread ----
-        const float* A = layers.p[l] + (size_t)b * Hh * n;
-        for (int e0 = 0; e0 < n; e0 += 8 * kRoThreads) {
-            float s[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int e = e0 + i * kRoThreads + tid;
-                s[i] = e < n ? __ldcs(A + e) : 0.0f;
-            }
-#pragma unroll
-            for (int h = 1; h < Hh; ++h) {
-                float t[8];
+        const E* A = layers.p[l] + (size_t)b * Hh * n;
+        if constexpr (sizeof(E) == 2) {
+            ro_stream_fuse_half<HT>(A, n, Hh, head_fusion, M);
+        } else {
+            for (int e0 = 0; e0 < n; e0 += 8 * kRoThreads) {
+                float s[8];
 #pragma unroll
                 for (int i = 0; i < 8; ++i) {
                     const int e = e0 + i * kRoThreads + tid;
-                    t[i] = e < n ? __ldcs(A + (size_t)h * n + e) : 0.0f;
+                    s[i] = e < n ? __ldcs(A + e) : 0.0f;
                 }
 #pragma unroll
-                for (int i = 0; i < 8; ++i)
-                    s[i] = head_fusion == 0 ? s[i] + t[i] : head_fusion == 1 ? fmaxf(s[i], t[i]) : fminf(s[i], t[i]);
-            }
+                for (int h = 1; h < Hh; ++h) {
+                    float t[8];
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int e = e0 + i * kRoThreads + tid;
-                if (e < n) M[e] = head_fusion == 0 ? s[i] / (float)Hh : s[i];      // torch.mean = sum / count
+                    for (int i = 0; i < 8; ++i) {
+                        const int e = e0 + i * kRoThreads + tid;
+                        t[i] = e < n ? __ldcs(A + (size_t)h * n + e) : 0.0f;
+                    }
+#pragma unroll
+                    for (int i = 0; i < 8; ++i)
+                        s[i] = head_fusion == 0 ? s[i] + t[i] : head_fusion == 1 ? fmaxf(s[i], t[i]) : fminf(s[i], t[i]);
+                }
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    const int e = e0 + i * kRoThreads + tid;
+                    if (e < n) M[e] = head_fusion == 0 ? s[i] / (float)Hh : s[i];      // torch.mean = sum / count
+                }
             }
         }
         __syncthreads();
@@ -356,9 +447,9 @@ rollout_chain_kernel(int L, int B, int T, int cap, const int32_t* __restrict__ c
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kRo2Bins = 2048;
 
-template <int HT>
+template <int HT, class E>
 __global__ void __launch_bounds__(kRoThreads, 1)
-rollout_prepare2_kernel(const RoLayers layers, int L, int B, int H, int T, int k_discard, int head_fusion,
+rollout_prepare2_kernel(const RoLayers<E> layers, int L, int B, int H, int T, int k_discard, int head_fusion,
                         float identity_w, int cap, int32_t* __restrict__ col_ptr, float* __restrict__ ent_val,
                         uint16_t* __restrict__ ent_row, int norm_mode) {
     pdl_sync();
@@ -378,31 +469,35 @@ rollout_prepare2_kernel(const RoLayers layers, int L, int B, int H, int T, int k
 
     for (int tile = blockIdx.x; tile < L * B; tile += gridDim.x) {
         const int l = tile / B, b = tile - l * B;
-        // ---- 1. stream + fuse the head maps (as v1) ----
-        const float* A = layers.p[l] + (size_t)b * Hh * n;
-        for (int e0 = 0; e0 < n; e0 += 8 * kRoThreads) {
-            float s[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int e = e0 + i * kRoThreads + tid;
-                s[i] = e < n ? __ldcs(A + e) : 0.0f;
-            }
-#pragma unroll
-            for (int h = 1; h < Hh; ++h) {
-                float t[8];
+        // ---- 1. stream + fuse the head maps (as v1, same element type rule) ----
+        const E* A = layers.p[l] + (size_t)b * Hh * n;
+        if constexpr (sizeof(E) == 2) {
+            ro_stream_fuse_half<HT>(A, n, Hh, head_fusion, M);
+        } else {
+            for (int e0 = 0; e0 < n; e0 += 8 * kRoThreads) {
+                float s[8];
 #pragma unroll
                 for (int i = 0; i < 8; ++i) {
                     const int e = e0 + i * kRoThreads + tid;
-                    t[i] = e < n ? __ldcs(A + (size_t)h * n + e) : 0.0f;
+                    s[i] = e < n ? __ldcs(A + e) : 0.0f;
                 }
 #pragma unroll
-                for (int i = 0; i < 8; ++i)
-                    s[i] = head_fusion == 0 ? s[i] + t[i] : head_fusion == 1 ? fmaxf(s[i], t[i]) : fminf(s[i], t[i]);
-            }
+                for (int h = 1; h < Hh; ++h) {
+                    float t[8];
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int e = e0 + i * kRoThreads + tid;
-                if (e < n) M[e] = head_fusion == 0 ? s[i] / (float)Hh : s[i];
+                    for (int i = 0; i < 8; ++i) {
+                        const int e = e0 + i * kRoThreads + tid;
+                        t[i] = e < n ? __ldcs(A + (size_t)h * n + e) : 0.0f;
+                    }
+#pragma unroll
+                    for (int i = 0; i < 8; ++i)
+                        s[i] = head_fusion == 0 ? s[i] + t[i] : head_fusion == 1 ? fmaxf(s[i], t[i]) : fminf(s[i], t[i]);
+                }
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    const int e = e0 + i * kRoThreads + tid;
+                    if (e < n) M[e] = head_fusion == 0 ? s[i] / (float)Hh : s[i];
+                }
             }
         }
         __syncthreads();
@@ -592,20 +687,21 @@ rollout_chain2_kernel(int L, int B, int T, int cap, const int32_t* __restrict__ 
 // equal values the lowest index is discarded first).
 constexpr int kRoClsThreads = 256;
 
+template <class E>
 __global__ void __launch_bounds__(kRoClsThreads)
-rollout_cls_rows_kernel(const RoLayers layers, int n_cls, int B, int H, int Tc, int k_discard, int head_fusion,
+rollout_cls_rows_kernel(const RoLayers<E> layers, int n_cls, int B, int H, int Tc, int k_discard, int head_fusion,
                         float identity_w, float* __restrict__ v0) {
     pdl_sync();
     __shared__ float x[kRoClsThreads], acc[kRoClsThreads], wred[kRoClsThreads / 32];
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     acc[tid] = 0.0f;
     for (int c = 0; c < n_cls; ++c) {
-        const float* A = layers.p[c] + (size_t)b * H * Tc;
+        const E* A = layers.p[c] + (size_t)b * H * Tc;
         float s = 0.0f;
         if (tid < Tc) {
-            s = A[tid];
+            s = ro_f32(A[tid]);
             for (int h = 1; h < H; ++h) {
-                const float t = A[(size_t)h * Tc + tid];
+                const float t = ro_f32(A[(size_t)h * Tc + tid]);
                 s = head_fusion == 0 ? s + t : head_fusion == 1 ? fmaxf(s, t) : fminf(s, t);
             }
             if (head_fusion == 0) s = s / (float)H;
@@ -638,26 +734,31 @@ extern "C" int pph_rollout_ws_bytes(int L, int B, int T, int k_discard, long lon
     return 0;
 }
 
-extern "C" int pph_rollout_scores(const float* const* attn_layers, int L, int B, int H, int T, int k_discard,
-                                  int head_fusion, float identity_w, const float* v0, int drop_first, void* workspace,
-                                  float* scores, int K, int32_t* idx32, int64_t* idx64, pph_stream_t stream) {
-    using namespace pph;
-    PPH_REQUIRE(attn_layers && workspace && scores, PPH_EINVAL, "pph_rollout_scores: null pointer");
-    PPH_REQUIRE(L >= 1 && L <= kRoMaxLayers, PPH_EUNSUP, "pph_rollout_scores: 1 <= L <= %d (L=%d)", kRoMaxLayers, L);
+namespace pph {
+
+// pph_rollout_scores and its half-precision-map twins: `fn` names the entry point in error messages
+template <class E>
+static int rollout_scores_impl(const char* fn, const E* const* attn_layers, int L, int B, int H, int T, int k_discard,
+                               int head_fusion, float identity_w, const float* v0, int drop_first, void* workspace,
+                               float* scores, int K, int32_t* idx32, int64_t* idx64, pph_stream_t stream) {
+    PPH_REQUIRE(attn_layers && workspace && scores, PPH_EINVAL, "%s: null pointer", fn);
+    PPH_REQUIRE(L >= 1 && L <= kRoMaxLayers, PPH_EUNSUP, "%s: 1 <= L <= %d (L=%d)", fn, kRoMaxLayers, L);
     PPH_REQUIRE(B >= 0 && H >= 1 && T >= 2 && k_discard >= 0 && (drop_first == 0 || drop_first == 1), PPH_EINVAL,
-                "pph_rollout_scores: bad dims B=%d H=%d T=%d k=%d", B, H, T, k_discard);
-    PPH_REQUIRE(T <= kRoMaxT, PPH_EUNSUP, "pph_rollout_scores: T=%d > %d (the fused map must fit in shared memory)", T,
-                kRoMaxT);
-    PPH_REQUIRE(head_fusion >= 0 && head_fusion <= 2, PPH_EINVAL, "pph_rollout_scores: head_fusion %d", head_fusion);
+                "%s: bad dims B=%d H=%d T=%d k=%d", fn, B, H, T, k_discard);
+    PPH_REQUIRE(T <= kRoMaxT, PPH_EUNSUP, "%s: T=%d > %d (the fused map must fit in shared memory)", fn, T, kRoMaxT);
+    PPH_REQUIRE(head_fusion >= 0 && head_fusion <= 2, PPH_EINVAL, "%s: head_fusion %d", fn, head_fusion);
     PPH_REQUIRE(K == 0 || (K >= 1 && K <= T - drop_first && idx32), PPH_EINVAL,
-                "pph_rollout_scores: fused selection needs 1 <= K <= %d and idx32 (K=%d)", T - drop_first, K);
+                "%s: fused selection needs 1 <= K <= %d and idx32 (K=%d)", fn, T - drop_first, K);
     if (B == 0) return 0;
     if (k_discard > T * T) k_discard = T * T;
-    RoLayers layers;
+    RoLayers<E> layers;
     for (int l = 0; l < kRoMaxLayers; ++l) layers.p[l] = l < L ? attn_layers[l] : nullptr;
-    for (int l = 0; l < L; ++l) PPH_REQUIRE(layers.p[l], PPH_EINVAL, "pph_rollout_scores: layer %d is null", l);
+    for (int l = 0; l < L; ++l) PPH_REQUIRE(layers.p[l], PPH_EINVAL, "%s: layer %d is null", fn, l);
     const RoWorkspace w = rollout_carve(workspace, L, B, T, k_discard);
     const int n = T * T;
+    char what_prep[96], what_chain[96];
+    snprintf(what_prep, sizeof what_prep, "%s(prepare)", fn);
+    snprintf(what_chain, sizeof what_chain, "%s(chain)", fn);
     // PPH_ROLLOUT=1 selects the first version of both kernels (kept for A/B measurements)
     const bool use_v1 = option(kOptRollout) == 1;
     // default: one reciprocal per row instead of two IEEE divisions per entry (261.7 vs 292.4 us at the DeiT-Ti shape,
@@ -674,54 +775,101 @@ extern "C" int pph_rollout_scores(const float* const* attn_layers, int L, int B,
     const dim3 grid(tiles < sms ? tiles : sms);
     auto go = [&](auto kern) -> int {
         cudaError_t e = opt_in_smem(kern, 220 * 1024);
-        if (e != cudaSuccess) { set_error("pph_rollout_scores: cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return (int)e; }
+        if (e != cudaSuccess) { set_error("%s: cudaFuncSetAttribute: %s", fn, cudaGetErrorString(e)); return (int)e; }
         launch_k(kern, grid, dim3(kRoThreads), smem, st, layers, L, B, H, T, k_discard, head_fusion, identity_w, w.cap,
                  w.col_ptr, w.ent_val, w.ent_row);
-        return launch_status("pph_rollout_scores(prepare)");
+        return launch_status(what_prep);
     };
     auto go2 = [&](auto kern) -> int {
         cudaError_t e = opt_in_smem(kern, 220 * 1024);
-        if (e != cudaSuccess) { set_error("pph_rollout_scores: cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return (int)e; }
+        if (e != cudaSuccess) { set_error("%s: cudaFuncSetAttribute: %s", fn, cudaGetErrorString(e)); return (int)e; }
         launch_k(kern, grid, dim3(kRoThreads), smem, st, layers, L, B, H, T, k_discard, head_fusion, identity_w, w.cap,
                  w.col_ptr, w.ent_val, w.ent_row, norm_mode);
-        return launch_status("pph_rollout_scores(prepare)");
+        return launch_status(what_prep);
     };
     // head counts of the reference's backbones: DeiT-Ti 3, CaiT-XXS 4, DeiT-S 6 (deit_models_attn.py:288,303)
     int rc;
     if (v1)
-        rc = H == 3 ? go(rollout_prepare_kernel<3>) : H == 4 ? go(rollout_prepare_kernel<4>)
-             : H == 6 ? go(rollout_prepare_kernel<6>) : go(rollout_prepare_kernel<0>);
+        rc = H == 3 ? go(rollout_prepare_kernel<3, E>) : H == 4 ? go(rollout_prepare_kernel<4, E>)
+             : H == 6 ? go(rollout_prepare_kernel<6, E>) : go(rollout_prepare_kernel<0, E>);
     else
-        rc = H == 3 ? go2(rollout_prepare2_kernel<3>) : H == 4 ? go2(rollout_prepare2_kernel<4>)
-             : H == 6 ? go2(rollout_prepare2_kernel<6>) : go2(rollout_prepare2_kernel<0>);
+        rc = H == 3 ? go2(rollout_prepare2_kernel<3, E>) : H == 4 ? go2(rollout_prepare2_kernel<4, E>)
+             : H == 6 ? go2(rollout_prepare2_kernel<6, E>) : go2(rollout_prepare2_kernel<0, E>);
     if (rc) return rc;
     // staged chain needs the layer's entry list in shared memory (cap * 6 B): small discard ratios fall back to v1
     const size_t csmem = (size_t)w.cap * 4 + (size_t)(T + 1) * 4 + (size_t)w.cap * 2 + 16;
     if (!use_v1 && csmem <= 160 * 1024) {
         cudaError_t e = opt_in_smem(rollout_chain2_kernel, 160 * 1024);
-        if (e != cudaSuccess) { set_error("pph_rollout_scores: cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return (int)e; }
+        if (e != cudaSuccess) { set_error("%s: cudaFuncSetAttribute: %s", fn, cudaGetErrorString(e)); return (int)e; }
         launch_k(rollout_chain2_kernel, dim3(B), dim3(kRoChainThreads), csmem, st, L, B, T, w.cap, w.col_ptr, w.ent_val,
                  w.ent_row, v0, drop_first, scores, K, idx32, idx64);
     } else {
         launch_k(rollout_chain_kernel, dim3(B), dim3(kRoChainThreads), (size_t)0, st, L, B, T, w.cap, w.col_ptr,
                  w.ent_val, w.ent_row, v0, drop_first, scores, K, idx32, idx64);
     }
-    return launch_status("pph_rollout_scores(chain)");
+    return launch_status(what_chain);
+}
+
+template <class E>
+static int rollout_cls_rows_impl(const char* fn, const E* const* cls_layers, int n_cls, int B, int H, int Tc,
+                                 int k_discard, int head_fusion, float identity_w, float* v0, pph_stream_t stream) {
+    PPH_REQUIRE(cls_layers && v0, PPH_EINVAL, "%s: null pointer", fn);
+    PPH_REQUIRE(n_cls >= 1 && n_cls <= kRoMaxLayers, PPH_EUNSUP, "%s: 1 <= n_cls <= %d", fn, kRoMaxLayers);
+    PPH_REQUIRE(B >= 0 && H >= 1 && Tc >= 2 && k_discard >= 0, PPH_EINVAL, "%s: bad dims", fn);
+    PPH_REQUIRE(Tc <= kRoClsThreads, PPH_EUNSUP, "%s: Tc=%d > %d", fn, Tc, kRoClsThreads);
+    PPH_REQUIRE(head_fusion >= 0 && head_fusion <= 2, PPH_EINVAL, "%s: head_fusion %d", fn, head_fusion);
+    if (B == 0) return 0;
+    RoLayers<E> layers;
+    for (int l = 0; l < kRoMaxLayers; ++l) layers.p[l] = l < n_cls ? cls_layers[l] : nullptr;
+    for (int l = 0; l < n_cls; ++l) PPH_REQUIRE(layers.p[l], PPH_EINVAL, "%s: layer %d is null", fn, l);
+    launch_k(rollout_cls_rows_kernel<E>, dim3(B), dim3(kRoClsThreads), (size_t)0, as_stream(stream), layers, n_cls, B,
+             H, Tc, k_discard, head_fusion, identity_w, v0);
+    return launch_status(fn);
+}
+}  // namespace pph
+
+extern "C" int pph_rollout_scores(const float* const* attn_layers, int L, int B, int H, int T, int k_discard,
+                                  int head_fusion, float identity_w, const float* v0, int drop_first, void* workspace,
+                                  float* scores, int K, int32_t* idx32, int64_t* idx64, pph_stream_t stream) {
+    return pph::rollout_scores_impl("pph_rollout_scores", attn_layers, L, B, H, T, k_discard, head_fusion, identity_w,
+                                    v0, drop_first, workspace, scores, K, idx32, idx64, stream);
+}
+
+extern "C" int pph_rollout_scores_bf16attn(const uint16_t* const* attn_layers, int L, int B, int H, int T,
+                                           int k_discard, int head_fusion, float identity_w, const float* v0,
+                                           int drop_first, void* workspace, float* scores, int K, int32_t* idx32,
+                                           int64_t* idx64, pph_stream_t stream) {
+    return pph::rollout_scores_impl("pph_rollout_scores_bf16attn",
+                                    reinterpret_cast<const __nv_bfloat16* const*>(attn_layers), L, B, H, T, k_discard,
+                                    head_fusion, identity_w, v0, drop_first, workspace, scores, K, idx32, idx64, stream);
+}
+
+extern "C" int pph_rollout_scores_f16attn(const uint16_t* const* attn_layers, int L, int B, int H, int T,
+                                          int k_discard, int head_fusion, float identity_w, const float* v0,
+                                          int drop_first, void* workspace, float* scores, int K, int32_t* idx32,
+                                          int64_t* idx64, pph_stream_t stream) {
+    return pph::rollout_scores_impl("pph_rollout_scores_f16attn", reinterpret_cast<const __half* const*>(attn_layers),
+                                    L, B, H, T, k_discard, head_fusion, identity_w, v0, drop_first, workspace, scores,
+                                    K, idx32, idx64, stream);
 }
 
 extern "C" int pph_rollout_cls_rows(const float* const* cls_layers, int n_cls, int B, int H, int Tc, int k_discard,
                                     int head_fusion, float identity_w, float* v0, pph_stream_t stream) {
-    using namespace pph;
-    PPH_REQUIRE(cls_layers && v0, PPH_EINVAL, "pph_rollout_cls_rows: null pointer");
-    PPH_REQUIRE(n_cls >= 1 && n_cls <= kRoMaxLayers, PPH_EUNSUP, "pph_rollout_cls_rows: 1 <= n_cls <= %d", kRoMaxLayers);
-    PPH_REQUIRE(B >= 0 && H >= 1 && Tc >= 2 && k_discard >= 0, PPH_EINVAL, "pph_rollout_cls_rows: bad dims");
-    PPH_REQUIRE(Tc <= kRoClsThreads, PPH_EUNSUP, "pph_rollout_cls_rows: Tc=%d > %d", Tc, kRoClsThreads);
-    PPH_REQUIRE(head_fusion >= 0 && head_fusion <= 2, PPH_EINVAL, "pph_rollout_cls_rows: head_fusion %d", head_fusion);
-    if (B == 0) return 0;
-    RoLayers layers;
-    for (int l = 0; l < kRoMaxLayers; ++l) layers.p[l] = l < n_cls ? cls_layers[l] : nullptr;
-    for (int l = 0; l < n_cls; ++l) PPH_REQUIRE(layers.p[l], PPH_EINVAL, "pph_rollout_cls_rows: layer %d is null", l);
-    launch_k(rollout_cls_rows_kernel, dim3(B), dim3(kRoClsThreads), (size_t)0, as_stream(stream), layers, n_cls, B, H, Tc,
-             k_discard, head_fusion, identity_w, v0);
-    return launch_status("pph_rollout_cls_rows");
+    return pph::rollout_cls_rows_impl("pph_rollout_cls_rows", cls_layers, n_cls, B, H, Tc, k_discard, head_fusion,
+                                      identity_w, v0, stream);
+}
+
+extern "C" int pph_rollout_cls_rows_bf16attn(const uint16_t* const* cls_layers, int n_cls, int B, int H, int Tc,
+                                             int k_discard, int head_fusion, float identity_w, float* v0,
+                                             pph_stream_t stream) {
+    return pph::rollout_cls_rows_impl("pph_rollout_cls_rows_bf16attn",
+                                      reinterpret_cast<const __nv_bfloat16* const*>(cls_layers), n_cls, B, H, Tc,
+                                      k_discard, head_fusion, identity_w, v0, stream);
+}
+
+extern "C" int pph_rollout_cls_rows_f16attn(const uint16_t* const* cls_layers, int n_cls, int B, int H, int Tc,
+                                            int k_discard, int head_fusion, float identity_w, float* v0,
+                                            pph_stream_t stream) {
+    return pph::rollout_cls_rows_impl("pph_rollout_cls_rows_f16attn", reinterpret_cast<const __half* const*>(cls_layers),
+                                      n_cls, B, H, Tc, k_discard, head_fusion, identity_w, v0, stream);
 }

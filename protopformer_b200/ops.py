@@ -111,24 +111,30 @@ def rollout_workspace(L: int, B: int, T: int, k_discard: int, device) -> torch.T
     return torch.empty(max(int(n.value), 256), dtype=torch.uint8, device=device)
 
 
+def _attn_tables(maps, entry: str):
+    """The entry point and layer list for one set of attention maps: bf16 or fp16 maps, all of one of those dtypes, go
+    to the half-precision twin of `entry` as they are (no fp32 copy); any other list is widened to an fp32 copy."""
+    maps = [m.detach() for m in maps]
+    dt = maps[0].dtype
+    if dt in _lib.ATTN_TWINS and all(m.dtype == dt for m in maps):
+        return entry + _lib.ATTN_TWINS[dt], [m.contiguous() for m in maps]
+    return entry, [m.float().contiguous() for m in maps]
+
+
 def rollout_scores(all_attn, discard_ratio: float = 0.9, head_fusion: str = "mean", identity_w: float = 0.2,
                    v0: torch.Tensor | None = None, drop_first: bool = True, workspace: torch.Tensor | None = None,
                    topk: int = 0, want_int64: bool = False):
     """``attn_rollout(all_attn)[:, 0, 1:]`` of the reference (deit_models_attn.py:99-124, :226) without the (T,T)
-    products.  all_attn: list of L fp32 CUDA tensors (B,H,T,T) (the attention maps of the first L blocks);
-    returns the detached score (B, T-1) [(B,T) when drop_first is False].  ``v0`` (B,T): start row instead of e_0
+    products.  all_attn: list of L CUDA tensors (B,H,T,T) (the attention maps of the first L blocks): fp32, or all
+    bf16 / all fp16, read as they are with the result of their fp32 widening bit for bit (other lists are widened to
+    fp32 first); returns the detached score (B, T-1) [(B,T) when drop_first is False].  ``v0`` (B,T): start row instead of e_0
     (CaiT, cait_models_attn.py:255-259).  The result is not differentiable -- the reference detaches it (:225).
     ``topk`` = K > 0: the same launch also selects the K highest-scoring tokens of every image (ascending int32 index
     list, deit_models_attn.py:229-230 / protopformer.py:157-158) and ``(scores, idx32[, idx64])`` is returned."""
     import ctypes
     L = len(all_attn)
     assert L >= 1
-    layers = []
-    for a in all_attn:
-        a = a.detach()
-        if a.dtype != torch.float32:
-            a = a.float()
-        layers.append(a.contiguous())
+    entry, layers = _attn_tables(all_attn, "pph_rollout_scores")
     B, H, T, T2 = layers[0].shape
     assert T == T2 and all(a.shape == layers[0].shape for a in layers), "square (B,H,T,T) maps of one shape expected"
     k = int(T * T * discard_ratio)                    # deit_models_attn.py:110
@@ -144,7 +150,7 @@ def rollout_scores(all_attn, discard_ratio: float = 0.9, head_fusion: str = "mea
         v0 = v0.detach().float().contiguous()
     idx32 = _empty((B, topk), torch.int32, layers[0]) if topk > 0 else None
     idx64 = _empty((B, topk), torch.int64, layers[0]) if (topk > 0 and want_int64) else None
-    _lib.call("pph_rollout_scores", table, L, B, H, T, k, FUSIONS[head_fusion], float(identity_w), v0,
+    _lib.call(entry, table, L, B, H, T, k, FUSIONS[head_fusion], float(identity_w), v0,
               int(drop_first), workspace, scores, int(topk), idx32, idx64)
     if topk > 0:
         return (scores, idx32, idx64) if want_int64 else (scores, idx32)
@@ -155,16 +161,17 @@ def rollout_scores_cait(all_attn, pre_layer_num: int, discard_ratio: float = 0.9
                         identity_w: float = 0.2):
     """``attn_rollout_cait(all_attn, discard_ratio, head_fusion, layer_nums=[pre_layer_num, i])[1][:, 0]`` of the
     reference (tools/cait_models_attn.py:223-261, :328-330): all_attn = pre_layer_num patch-layer maps (B,H,T,T)
-    followed by i >= 1 class-attention maps (B,H,1,T+1).  Returns the detached token score (B,T)."""
+    followed by i >= 1 class-attention maps (B,H,1,T+1).  Returns the detached token score (B,T).  The dtype rule of
+    ``rollout_scores`` applies to the patch maps and to the class-attention maps separately."""
     import ctypes
     patch, cls = list(all_attn[:pre_layer_num]), list(all_attn[pre_layer_num:])
     assert patch and cls, "CaiT rollout needs patch layers and at least one class-attention layer"
-    cls = [c.detach().float().contiguous() for c in cls]
+    entry, cls = _attn_tables(cls, "pph_rollout_cls_rows")
     B, H, R, Tc = cls[0].shape
     assert R == 1 and all(c.shape == cls[0].shape for c in cls)
     v0 = _empty((B, Tc - 1), torch.float32, cls[0])
     table = (ctypes.c_void_p * len(cls))(*[_ptr_of(c) for c in cls])
-    _lib.call("pph_rollout_cls_rows", table, len(cls), B, H, Tc, int(Tc * discard_ratio), FUSIONS[head_fusion],
+    _lib.call(entry, table, len(cls), B, H, Tc, int(Tc * discard_ratio), FUSIONS[head_fusion],
               float(identity_w), v0)
     return rollout_scores(patch, discard_ratio, head_fusion, identity_w, v0=v0, drop_first=False)
 
