@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define PPH_VERSION 202
+#define PPH_VERSION 203
 
 /* argument errors */
 #define PPH_EINVAL   (-1)   /* bad dimension / null pointer */
@@ -51,11 +51,6 @@ int         pph_version(void);
 const char* pph_last_error_string(void);
 /* number of SMs of the current device (persistent-grid sizing), or <0 */
 int         pph_sm_count(void);
-/* Variant / measurement switches (process-wide; the library itself never reads the environment):
- *   "pdl" 0|1 programmatic dependent launch on every kernel; "sim_lanes" n, "sim_shared" 0|1, "sim_epi" 0|1: tcgen05
- *   similarity CTA plan / epilogue variants; "rollout" 1|2|3 and "classmap" 1|2: kernel versions of those rows.
- * Returns 0, or PPH_EINVAL for an unknown name. */
-int         pph_set_option(const char* name, int value);
 
 /* (a1) protopformer.py:157-158  topk(cls_token_attn, K)[1].sort()[0]
  * scores [B,H,N] (H>=1; H>1: the mean over H is taken first), idx32 [B,K] ascending, idx64 [B,K] or NULL.

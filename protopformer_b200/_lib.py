@@ -25,7 +25,6 @@ SIGNATURES = {
     "pph_version": [],
     "pph_last_error_string": [],
     "pph_sm_count": [],
-    "pph_set_option": [C.c_char_p, _i],
     "pph_select_topk": [_p, _i, _i, _i, _i, _p, _p, _p],
     "pph_addon_fwd": [_p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _p, _p, _f, _p, _p, _p, _p, _p, _p, _p, _p, _p],
     "pph_split_rows": [_p, _i, _i, _f, _p, _p, _p, _p, _p, _p],
@@ -92,10 +91,6 @@ KERNELS_PER_CALL = {
     "pph_ppc_dense_fwd": 1, "pph_ppc_dense_bwd": 1, "pph_select_addon_fwd": 1,
 }
 
-_ENV_OPTIONS = {"PPH_PDL": "pdl", "PPH_SIM_LANES": "sim_lanes", "PPH_SIM_SHARED": "sim_shared", "PPH_SIM_EPI": "sim_epi",
-                "PPH_ROLLOUT": "rollout", "PPH_CLASSMAP": "classmap", "PPH_DEBUG": "debug",
-                "PPH_LOGITS_BWD": "logits_bwd", "PPH_GATHER": "gather"}
-
 _lib = None
 _launches = 0
 
@@ -118,12 +113,6 @@ def load() -> C.CDLL:
             fn = getattr(lib, name)      # AttributeError here = header / library mismatch
             fn.argtypes = args
             fn.restype = _RESTYPES.get(name, C.c_int)
-        # variant switches are resolved HERE, once, from the environment (the C side never calls getenv)
-        for env, opt in _ENV_OPTIONS.items():
-            v = os.environ.get(env)
-            if v is not None and v.strip() != "":
-                if lib.pph_set_option(opt.encode(), int(v)) != 0:
-                    raise RuntimeError(f"{env}: {lib.pph_last_error_string().decode()}")
         _lib = lib
     return _lib
 

@@ -34,7 +34,6 @@ struct AdamSegs {
 __global__ void __launch_bounds__(kAdamThreads)
 adamw_kernel(const AdamSegs segs, const float* __restrict__ hyper, double beta1d, double beta2d, float eps,
              float grad_scale, int* __restrict__ step_state) {
-    pdl_sync();
     __shared__ float s_step_size, s_bc2_sqrt, s_decay;
     __shared__ int s_t;
     int sg = 0;

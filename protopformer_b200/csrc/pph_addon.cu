@@ -26,7 +26,6 @@ addon_fwd_kernel(const T* __restrict__ tokens, const int32_t* __restrict__ idx, 
                  float* __restrict__ z2s_hi, float* __restrict__ z2c_hi,
                  uint16_t* __restrict__ Zs_hi, uint16_t* __restrict__ Zs_lo,
                  uint16_t* __restrict__ Zc_hi, uint16_t* __restrict__ Zc_lo) {
-    pdl_sync();
     __shared__ __align__(16) float As[kAddBK][kAddBM + 4];
     __shared__ __align__(16) float Ws[kAddBK][kAddBN + 4];
     __shared__ long src_off[kAddBM];    // element offset of the source token row, -1 = row out of range
@@ -143,7 +142,6 @@ __global__ void __launch_bounds__(256)
 split_rows_kernel(const float* __restrict__ V, int R, int D, float center, uint16_t* __restrict__ hi,
                   uint16_t* __restrict__ lo, float* __restrict__ v2, float* __restrict__ v2_ctr,
                   float* __restrict__ v2_hi) {
-    pdl_sync();
     const int row = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (row >= R) return;
     const float* v = V + (size_t)row * D;
@@ -245,7 +243,6 @@ struct DxEpi {      // scatter of the token gradient rows
 __global__ void __launch_bounds__(256)
 wgrad_reduce_kernel(const float* __restrict__ part, int splits, int D, int Din, int ldn, float* __restrict__ dWa,
                     float* __restrict__ dba) {
-    pdl_sync();
     const int i = blockIdx.x * 256 + threadIdx.x;
     if (i >= D * (Din + 1)) return;
     const int d = i / (Din + 1), n = i - d * (Din + 1);

@@ -266,7 +266,6 @@ __device__ __forceinline__ void addon_bwd_w(const AddonBwdArgs& a, int vb, float
 template <int MAXT, class T>
 __global__ void __launch_bounds__(MAXT, 1)
 addon_bwd2_kernel(const AddonBwdArgs a) {
-    pdl_sync();
     extern __shared__ __align__(16) float sm_ab[];
     if ((int)blockIdx.x < a.nX) {
         addon_bwd_x<T>(a, sm_ab);

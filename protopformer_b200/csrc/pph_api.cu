@@ -1,7 +1,6 @@
 // Library-level entry points: version, last-error string, device query.
 #include <stdarg.h>
 #include <stdlib.h>
-#include <string.h>
 
 #include "pph_common.cuh"
 
@@ -16,26 +15,7 @@ void set_error(const char* fmt, ...) {
     va_end(ap);
 }
 
-// defaults: PDL off, similarity plan knobs off, similarity epilogue 1 (chain-split), rollout version 2, class maps 1
-static int g_opt[kOptCount] = {0, 0, 0, 1, 2, 1, 0};
-static const char* const g_opt_name[kOptCount] = {"pdl", "sim_lanes", "sim_shared", "sim_epi", "rollout", "classmap", "debug", "logits_bwd", "gather"};
-
-int option(Option o) { return g_opt[o]; }
-bool pdl_enabled() { return g_opt[kOptPdl] != 0; }
-
 }  // namespace pph
-
-extern "C" int pph_set_option(const char* name, int value) {
-    using namespace pph;
-    PPH_REQUIRE(name, PPH_EINVAL, "pph_set_option: null name");
-    for (int i = 0; i < kOptCount; ++i)
-        if (strcmp(name, g_opt_name[i]) == 0) {
-            g_opt[i] = value;
-            return 0;
-        }
-    set_error("pph_set_option: unknown option '%s'", name);
-    return PPH_EINVAL;
-}
 
 extern "C" int pph_version(void) { return PPH_VERSION; }
 

@@ -19,7 +19,6 @@ __global__ void __launch_bounds__(kCmThreads)
 class_maps_kernel(const float* __restrict__ Zs, const float* __restrict__ z2s, const float* __restrict__ Pl,
                   const float* __restrict__ p2l, const int32_t* __restrict__ idx, const int64_t* __restrict__ labels,
                   int K, int D, int P, int m, int N, int act_fn, float eps, float* __restrict__ maps) {
-    pdl_sync();
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     float* out = maps + (size_t)b * m * N;
     for (int i = tid; i < m * N; i += kCmThreads) out[i] = 0.0f;
@@ -45,60 +44,6 @@ class_maps_kernel(const float* __restrict__ Zs, const float* __restrict__ z2s, c
     }
 }
 
-// v2 (PPH_CLASSMAP=2; NOT yet validated on a GPU -- written after round 1's budget was spent).  v1 measures 76 us at
-// B = 64 (profiles/r1b_next_rows.jsonl): every warp walks ~100 dependent 192-long dot products straight from L2.
-// Here the image's K token rows and its m label-class prototype rows are staged once in shared memory with coalesced
-// loads (row stride D + 4 floats: conflict-free 128-bit reads), then thread = (token, prototype) does its dot
-// product out of shared memory with 4-wide loads, the same layout ppc_fwd_kernel uses.  Same association as v1 for the
-// distance (z2 + (p2 - 2 z.p)); the dot product is summed in a different order (sequential over D instead of a
-// lane-strided shuffle tree), so results differ from v1 by fp32 rounding only.
-__global__ void __launch_bounds__(kCmThreads)
-class_maps2_kernel(const float* __restrict__ Zs, const float* __restrict__ z2s, const float* __restrict__ Pl,
-                   const float* __restrict__ p2l, const int32_t* __restrict__ idx, const int64_t* __restrict__ labels,
-                   int K, int D, int P, int m, int N, int act_fn, float eps, float* __restrict__ maps) {
-    pdl_sync();
-    extern __shared__ __align__(16) float cm_smem[];
-    const int ld = D + 4;
-    float* zs = cm_smem;                    // [K][ld]
-    float* ps = cm_smem + (size_t)K * ld;   // [m][ld]
-    const int b = blockIdx.x, tid = threadIdx.x;
-    float* out = maps + (size_t)b * m * N;
-    for (int i = tid; i < m * N; i += kCmThreads) out[i] = 0.0f;
-    long y = labels[b];
-    const int C = P / m;
-    if (y < 0) y = 0;
-    if (y >= C) y = C - 1;
-    const int D4 = D >> 2;                  // D % 4 == 0 is required by the launcher
-    const float4* zg = reinterpret_cast<const float4*>(Zs + (size_t)b * K * D);
-    for (int i = tid; i < K * D4; i += kCmThreads) {
-        const int r = i / D4, c = i - r * D4;
-        *reinterpret_cast<float4*>(zs + (size_t)r * ld + 4 * c) = zg[i];
-    }
-    const float4* pg = reinterpret_cast<const float4*>(Pl + (size_t)y * m * D);
-    for (int i = tid; i < m * D4; i += kCmThreads) {
-        const int r = i / D4, c = i - r * D4;
-        *reinterpret_cast<float4*>(ps + (size_t)r * ld + 4 * c) = pg[i];
-    }
-    __syncthreads();                        // staged operands visible; the zero fill above precedes the scatter below
-    for (int pair = tid; pair < m * K; pair += kCmThreads) {
-        const int q = pair / K, k = pair - q * K;
-        const float4* z = reinterpret_cast<const float4*>(zs + (size_t)k * ld);
-        const float4* pr = reinterpret_cast<const float4*>(ps + (size_t)q * ld);
-        float s = 0.f;
-        for (int d = 0; d < D4; ++d) {
-            const float4 a = z[d], w = pr[d];
-            s = fmaf(a.x, w.x, s);
-            s = fmaf(a.y, w.y, s);
-            s = fmaf(a.z, w.z, s);
-            s = fmaf(a.w, w.w, s);
-        }
-        const int p = (int)y * m + q;
-        const float dist = relu_keep_nan(z2s[(size_t)b * K + k] + (p2l[p] - 2.0f * s));
-        const int n = idx[(size_t)b * K + k];
-        if (n >= 0 && n < N) out[(size_t)q * N + n] = act_of_dist(dist, act_fn, eps);
-    }
-}
-
 }  // namespace pph
 
 extern "C" int pph_class_maps(const float* Zs, const float* z2s, const float* Pl, const float* p2l,
@@ -110,15 +55,6 @@ extern "C" int pph_class_maps(const float* Zs, const float* z2s, const float* Pl
                 "pph_class_maps: bad dims B=%d K=%d D=%d P=%d m=%d N=%d", B, K, D, P, m, N);
     PPH_REQUIRE(act_fn == PPH_ACT_LOG || act_fn == PPH_ACT_LINEAR, PPH_EINVAL, "pph_class_maps: act_fn %d", act_fn);
     if (B == 0) return 0;
-    const bool use_v2 = option(kOptClassmap) != 1;       // staged kernel by default (28.9 vs 75.4 us at B = 64); 1 = first kernel
-    const size_t smem2 = (size_t)(K + m) * (D + 4) * sizeof(float);
-    if (use_v2 && D % 4 == 0 && smem2 <= 200 * 1024) {
-        cudaError_t e = opt_in_smem(class_maps2_kernel, 200 * 1024);
-        if (e != cudaSuccess) { set_error("pph_class_maps: cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return (int)e; }
-        launch_k(class_maps2_kernel, dim3(B), dim3(kCmThreads), smem2, as_stream(stream), Zs, z2s, Pl, p2l, idx32, labels,
-                 K, D, P, m, N, act_fn, eps, maps);
-        return launch_status("pph_class_maps(staged)");
-    }
     launch_k(class_maps_kernel, dim3(B), dim3(kCmThreads), (size_t)0, as_stream(stream), Zs, z2s, Pl, p2l, idx32, labels,
              K, D, P, m, N, act_fn, eps, maps);
     return launch_status("pph_class_maps");

@@ -38,18 +38,6 @@ inline int launch_status(const char* what) {
 
 inline cudaStream_t as_stream(pph_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }
 
-// Programmatic dependent launch (env PPH_PDL=1, read once): every kernel of this library is launched with the
-// programmatic-stream-serialization attribute, so the next kernel's CTAs are scheduled and run their prologue while
-// the previous kernel drains; each kernel executes pdl_sync() before its first global-memory access, which blocks
-// until every prerequisite grid has completed and flushed (so data hazards are exactly those of plain stream order).
-// Under stream capture the attribute becomes a programmatic edge of the CUDA graph.
-bool pdl_enabled();
-
-// Measurement / variant switches, set once by the host binding through pph_set_option() (protopformer_b200/_lib.py reads
-// the PPH_* environment variables at load time); the launchers never read the environment.
-enum Option { kOptPdl = 0, kOptSimLanes, kOptSimShared, kOptSimEpi, kOptRollout, kOptClassmap, kOptDebug, kOptLogitsBwd, kOptGather, kOptCount };
-int option(Option o);
-
 template <typename... KArgs, typename... Args>
 inline void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
     cudaLaunchConfig_t cfg = {};
@@ -57,11 +45,6 @@ inline void launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem,
     cfg.blockDim = block;
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 1 : 0;
     (void)cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);   // status is read by launch_status()
 }
 
@@ -108,15 +91,6 @@ __device__ __forceinline__ int rank_by_count(const float4* s4, int n, int n_pad,
         rank += (q.x > v) + (q.y > v) + (q.z > v) + (q.w > v);
     }
     return rank;
-}
-
-// First statement of every kernel (see launch_k): let the dependent grid start its prologue, then wait for the
-// prerequisite grids.  Both are no-ops for a launch without the programmatic attribute.
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_sync() {
-    pdl_launch_dependents();
-    pdl_wait();
 }
 
 // ---- cp.async (LDGSTS): 16-byte global -> shared copies that bypass the register file ---------------------------

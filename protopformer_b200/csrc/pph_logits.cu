@@ -21,7 +21,6 @@ __global__ void __launch_bounds__(kLogThreads)
 logits_fwd_kernel(const float* __restrict__ act_l, const float* __restrict__ act_g, const float* __restrict__ Wl,
                   const float* __restrict__ Wg, int B, int P, int Pg, int C, float gc,
                   float* __restrict__ logits, float* __restrict__ logits_g, float* __restrict__ logits_l) {
-    pdl_sync();
     __shared__ float red[kLogThreads / 32][kLogTB * kLogTC];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int b0 = blockIdx.y * kLogTB, c0 = blockIdx.x * kLogTC;
@@ -152,7 +151,6 @@ logits_bwd_fma_kernel(const float* __restrict__ dlogits, const float* __restrict
                       const float* __restrict__ Wl, const float* __restrict__ Wg, const float* __restrict__ dmin_l,
                       const float* __restrict__ dmin_g, int B, int P, int Pg, int C, int nbl, float gc, int act_fn, float eps,
                       float* __restrict__ g_l, float* __restrict__ g_g) {
-    pdl_sync();
     extern __shared__ float up[];                      // [kLbfTB][C]
     const bool global = (int)blockIdx.x >= nbl;
     const int p = ((int)blockIdx.x - (global ? nbl : 0)) * kLbfThreads + threadIdx.x;
@@ -259,7 +257,8 @@ extern "C" int pph_logits_bwd(const float* dlogits, const float* dlogits_g, cons
                 "pph_logits_bwd: null pointer");
     PPH_REQUIRE(B >= 0 && P >= 1 && Pg >= 0 && C >= 1, PPH_EINVAL, "pph_logits_bwd: bad dims");
     if (B == 0) return 0;
-    if (option(kOptLogitsBwd) != 1 && (size_t)kLbfTB * C * sizeof(float) <= 48 * 1024) {      // default: exact FP32 FMA
+    // exact FP32 FMA while the kernel's dlogits tile fits in 48 KB of shared memory; tcgen05 product for larger C
+    if ((size_t)kLbfTB * C * sizeof(float) <= 48 * 1024) {
         const int nbl = ceil_div(P, kLbfThreads), nbg = Pg > 0 ? ceil_div(Pg, kLbfThreads) : 0;
         launch_k(logits_bwd_fma_kernel, dim3(nbl + nbg, ceil_div(B, kLbfTB)), dim3(kLbfThreads), sizeof(float) * kLbfTB * C,
                  as_stream(stream), dlogits, dlogits_g, dlogits_l, Wl, Wg, dmin_l, dmin_g, B, P, Pg, C, nbl, global_coe, act_fn,

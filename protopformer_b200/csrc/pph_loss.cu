@@ -15,7 +15,6 @@ __global__ void __launch_bounds__(256)
 loss_tail_kernel(const float* __restrict__ logits, const int64_t* __restrict__ labels, const float* __restrict__ ppc,
                  float cov_coe, float mean_coe, float upstream, int B, int C, float* partial, unsigned int* counter,
                  float* __restrict__ out, float* __restrict__ dlogits) {
-    pdl_sync();
     const int b = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     __shared__ unsigned int s_ticket;
     if (b < B) {
@@ -62,7 +61,6 @@ loss_tail_kernel(const float* __restrict__ logits, const int64_t* __restrict__ l
 // tail (and with it the whole last-layer backward) start before the PPC loss has finished on its own stream.
 __global__ void loss_combine_kernel(const float* __restrict__ ce_losses, const float* __restrict__ ppc, float cov_coe,
                                     float mean_coe, float* __restrict__ out) {
-    pdl_sync();
     if (threadIdx.x == 0 && blockIdx.x == 0) {
         const float ce = ce_losses[1], cov = ppc ? ppc[0] : 0.f, mean = ppc ? ppc[1] : 0.f;
         out[0] = ce + cov_coe * cov + mean_coe * mean;

@@ -679,7 +679,6 @@ __device__ __forceinline__ void ppc_role(const MidArgs& a, int b, int part, int 
 template <int CJ>
 __global__ void __launch_bounds__(kMidThreads)
 head_mid_kernel(const MidArgs a) {
-    pdl_sync();
     extern __shared__ __align__(16) float sm_mid[];
     const int bid = blockIdx.x;
     if (bid < a.n_ll) {
@@ -712,7 +711,6 @@ head_mid_kernel(const MidArgs a) {
 constexpr int kPpcSplit = 2, kPpcThreads = 512;
 __global__ void __launch_bounds__(kPpcThreads)
 head_ppc_kernel(const MidArgs a) {
-    pdl_sync();
     extern __shared__ __align__(16) float sm_mid[];
     ppc_role(a, blockIdx.x / kPpcSplit, blockIdx.x % kPpcSplit, kPpcSplit, sm_mid);
 }
@@ -832,7 +830,6 @@ __device__ __forceinline__ LLPattern pattern_record(const float* W, int C, int n
 __global__ void __launch_bounds__(kPatThreads)
 last_layer_pattern_kernel(const float* __restrict__ Wl, int P, int vec_l, const float* __restrict__ Wg, int Pg, int vec_g,
                           int C, LLPatternWs* ws) {
-    pdl_sync();
     const unsigned int bits = pattern_scan(Wl, C, P, vec_l) | (pattern_scan(Wg, C, Pg, vec_g) << 1);
     const int bad_l = __syncthreads_or(bits & 1u), bad_g = __syncthreads_or(bits & 2u);
     if (threadIdx.x != 0) return;

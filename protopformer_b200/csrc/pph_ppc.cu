@@ -84,7 +84,6 @@ ppc_fwd_kernel(const float* __restrict__ Zs, const float* __restrict__ z2s, cons
                float cov_thresh, float mean_thresh,
                float* __restrict__ dslice, float* __restrict__ stats, float* partial, unsigned int* counter,
                float* __restrict__ losses) {
-    pdl_sync();
     extern __shared__ __align__(16) float sm[];
     const PpcSmem s = ppc_carve(sm, m, D, K, kc);
     __shared__ float red[kPpcThreads / 32];
@@ -205,7 +204,6 @@ ppc_bwd_kernel(const float* __restrict__ Zs, const float* __restrict__ Pl, const
                int B, int K, int D, int P, int m, int N, int side,
                int act_fn, float eps, float mean_thresh, int accumulate, float* __restrict__ dZs,
                float* __restrict__ dP) {
-    pdl_sync();
     extern __shared__ __align__(16) float sm[];
     float* Prow = sm;                         // [m][D]
     float* Zt = Prow + m * D;                 // [kPpcBwdTok][D]

@@ -68,7 +68,6 @@ __device__ __forceinline__ void split_row(const float* __restrict__ v, int D, fl
 template <int MAXT, int LD, class T>
 __global__ void __launch_bounds__(MAXT, 1)
 head_prep_kernel(const PrepArgs a) {
-    pdl_sync();
     extern __shared__ __align__(16) float sm_prep[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nthr = a.threads, nwarp = nthr >> 5;
     const int K = a.K, N = a.N, Din = a.Din, D = a.D, TR = a.TR, KC = a.KC;

@@ -6,16 +6,17 @@
 // Only row 0 of the product is consumed, so the matmul chain collapses to L vector-matrix products walked from the
 // last layer to the first, and after the discard only ~10 % of every matrix is non-zero.  Two kernels:
 //
-//  rollout_prepare_kernel  (HBM bound: reads every attention tensor exactly once, H*T*T*4 B per (layer, image))
+//  rollout_prepare2_kernel  (HBM bound: reads every attention tensor exactly once, H*T*T*4 B per (layer, image))
 //    persistent CTAs, one (layer, image) tile at a time: stream the H head maps, fuse them into a T x T fp32 tile in
-//    shared memory (155 KB at T = 197), find the EXACT k-th smallest entry with a 4-pass 8-bit radix select on the
-//    order-preserving integer image of the floats (warp-aggregated shared-memory histograms), zero the k smallest
-//    (ties at the threshold: lowest flat index first), add the identity, normalise the rows, and write the surviving
-//    entries as a column-compressed sparse matrix (<= T*T - k + T entries: ~25 KB instead of 155 KB).
-//  rollout_chain_kernel    (latency bound, tiny: the sparse matrices are L2 resident)
+//    shared memory (155 KB at T = 197), find the EXACT k-th smallest entry with a radix select on the
+//    order-preserving integer image of the floats (shared-memory histograms), zero the k smallest (ties at the
+//    threshold: lowest flat index first), add the identity, normalise the rows, and write the surviving entries as a
+//    column-compressed sparse matrix (<= T*T - k + T entries: ~25 KB instead of 155 KB).
+//  rollout_chain2_kernel    (latency bound, tiny: the sparse matrices are L2 resident)
 //    one CTA per image: v = e_0 (or a caller-supplied start row, the CaiT variant cait_models_attn.py:255-259);
-//    for l = L-1 .. 0: v <- v @ a_l as a gather over the columns' entry lists (one warp per column, fixed summation
-//    order -> bit-reproducible); scores[b, :] = v[1:] (or all of v).
+//    for l = L-1 .. 0: v <- v @ a_l as a gather over the columns' entry lists (fixed summation order ->
+//    bit-reproducible); scores[b, :] = v[1:] (or all of v).  When a layer's entry list does not fit in shared memory
+//    (small discard ratios at T = 197), rollout_chain_kernel walks it from global memory instead.
 #include <cuda_fp16.h>
 #include <math.h>
 #include <stdio.h>
@@ -181,185 +182,6 @@ __device__ __forceinline__ int block_excl_scan(int v, int* wsum, int& total) {
     return r;
 }
 
-// HT > 0: compile-time head count (the head loop unrolls, 8*HT loads in flight); 0: runtime H.  E: element type of the
-// maps (fp32 is streamed below, half precision by ro_stream_fuse_half).
-template <int HT, class E>
-__global__ void __launch_bounds__(kRoThreads, 1)
-rollout_prepare_kernel(const RoLayers<E> layers, int L, int B, int H, int T, int k_discard, int head_fusion,
-                       float identity_w, int cap, int32_t* __restrict__ col_ptr, float* __restrict__ ent_val,
-                       uint16_t* __restrict__ ent_row) {
-    pdl_sync();
-    extern __shared__ __align__(16) uint8_t ro_smem[];
-    const int n = T * T;
-    float* M = reinterpret_cast<float*>(ro_smem);                            // [T*T]
-    uint32_t* hist = reinterpret_cast<uint32_t*>(M + ((n + 3) & ~3));        // [256]
-    int* cnt = reinterpret_cast<int*>(hist + 256);                           // [1024] per-(column, segment) counts
-    int* wsum = cnt + kRoThreads;                                            // [33]
-    __shared__ uint32_t s_prefix, s_cnt;
-    __shared__ int s_krem;
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int n_pad = (n + 31) & ~31;
-    const int Hh = HT > 0 ? HT : H;
-    const int seg = min(5, kRoThreads / T);                 // row segments per column for the sparse build
-    const int rps = (T + seg - 1) / seg;
-
-    for (int tile = blockIdx.x; tile < L * B; tile += gridDim.x) {
-        const int l = tile / B, b = tile - l * B;
-        // ---- 1. stream the H head maps once, fuse (deit_models_attn.py:102-107); 8 x H loads in flight per thread ----
-        const E* A = layers.p[l] + (size_t)b * Hh * n;
-        if constexpr (sizeof(E) == 2) {
-            ro_stream_fuse_half<HT>(A, n, Hh, head_fusion, M);
-        } else {
-            for (int e0 = 0; e0 < n; e0 += 8 * kRoThreads) {
-                float s[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    const int e = e0 + i * kRoThreads + tid;
-                    s[i] = e < n ? __ldcs(A + e) : 0.0f;
-                }
-#pragma unroll
-                for (int h = 1; h < Hh; ++h) {
-                    float t[8];
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const int e = e0 + i * kRoThreads + tid;
-                        t[i] = e < n ? __ldcs(A + (size_t)h * n + e) : 0.0f;
-                    }
-#pragma unroll
-                    for (int i = 0; i < 8; ++i)
-                        s[i] = head_fusion == 0 ? s[i] + t[i] : head_fusion == 1 ? fmaxf(s[i], t[i]) : fminf(s[i], t[i]);
-                }
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    const int e = e0 + i * kRoThreads + tid;
-                    if (e < n) M[e] = head_fusion == 0 ? s[i] / (float)Hh : s[i];      // torch.mean = sum / count
-                }
-            }
-        }
-        __syncthreads();
-
-        // ---- 2. exact k-th smallest by radix select (4 passes x 8 bits, MSB first) ----
-        uint32_t prefix = 0, eq_total = 0;
-        int krem = k_discard < n ? k_discard : n;
-        if (krem > 0) {
-            for (int pass = 0; pass < 4; ++pass) {
-                const int shift = 24 - 8 * pass;
-                const uint32_t himask = pass == 0 ? 0u : (0xFFFFFFFFu << (shift + 8));
-                if (tid < 256) hist[tid] = 0;
-                __syncthreads();
-                for (int e = tid; e < n_pad; e += kRoThreads) {      // whole warps stay converged for the ballot
-                    const uint32_t key = e < n ? ro_key(M[e]) : 0u;
-                    const bool act = e < n && (key & himask) == prefix;
-                    const uint32_t digit = (key >> shift) & 0xFFu;
-                    const unsigned m_act = __ballot_sync(0xffffffffu, act);
-                    if (act) {
-                        const unsigned peers = __match_any_sync(m_act, digit);
-                        if (lane == __ffs(peers) - 1) atomicAdd(&hist[digit], (uint32_t)__popc(peers));
-                    }
-                }
-                __syncthreads();
-                if (warp == 0) {
-                    uint32_t c[8], s = 0;
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) { c[i] = hist[lane * 8 + i]; s += c[i]; }
-                    uint32_t incl = s;
-#pragma unroll
-                    for (int o = 1; o < 32; o <<= 1) {
-                        const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-                        if (lane >= o) incl += t;
-                    }
-                    const uint32_t excl = incl - s;
-                    if (excl < (uint32_t)krem && (uint32_t)krem <= incl) {      // exactly one lane
-                        uint32_t run = excl;
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            if ((uint32_t)krem > run && (uint32_t)krem <= run + c[i]) {
-                                s_prefix = prefix | ((uint32_t)(lane * 8 + i) << shift);
-                                s_krem = krem - (int)run;
-                                s_cnt = c[i];
-                            }
-                            run += c[i];
-                        }
-                    }
-                }
-                __syncthreads();
-                prefix = s_prefix;
-                krem = s_krem;
-                eq_total = s_cnt;
-                __syncthreads();
-            }
-            // ---- 3. discard (deit_models_attn.py:110-113): everything below the threshold ... ----
-            const bool all_equal_go = (uint32_t)krem == eq_total;
-            for (int e = tid; e < n; e += kRoThreads) {
-                const uint32_t key = ro_key(M[e]);
-                if (key < prefix || (all_equal_go && key == prefix)) M[e] = 0.0f;
-            }
-            __syncthreads();
-            // ... and `krem` of the entries EQUAL to it, lowest flat index first
-            if (!all_equal_go && warp == 0) {                                   // rare: a tie straddles the threshold
-                int seen = 0;
-                for (int e0 = 0; e0 < n && seen < krem; e0 += 32) {
-                    const int e = e0 + lane;
-                    const bool eq = e < n && ro_key(M[e]) == prefix;
-                    const unsigned m = __ballot_sync(0xffffffffu, eq);
-                    if (eq && seen + __popc(m & ((1u << lane) - 1u)) < krem) M[e] = 0.0f;
-                    seen += __popc(m);
-                }
-            }
-            __syncthreads();
-        }
-
-        // ---- 4. a = (A + w I) / (1 + w), rows normalised (deit_models_attn.py:118-121); warp = row ----
-        const float inv_den = 1.0f + identity_w;
-        for (int r = warp; r < T; r += kRoThreads / 32) {
-            float* row = M + r * T;
-            float s = 0.f;
-            for (int j = lane; j < T; j += 32) {
-                const float a = (row[j] + (j == r ? identity_w : 0.0f)) / inv_den;
-                row[j] = a;
-                s += a;
-            }
-            s = warp_sum(s);
-            for (int j = lane; j < T; j += 32) row[j] = row[j] / s;
-        }
-        __syncthreads();
-
-        // ---- 5. column-compressed sparse output: thread = (row segment sg, column j), entries ordered by (j, row) ----
-        const bool worker = tid < seg * T;
-        const int sg = tid / T, j = tid - sg * T;
-        const int r0 = sg * rps, r1 = min(T, r0 + rps);
-        int mine = 0;
-        if (worker)
-            for (int r = r0; r < r1; ++r) mine += (M[r * T + j] != 0.0f);
-        cnt[tid] = 0;
-        __syncthreads();
-        if (worker) cnt[j * seg + sg] = mine;
-        __syncthreads();
-        int total;
-        const int excl = block_excl_scan(cnt[tid], wsum, total);
-        cnt[tid] = excl;
-        __syncthreads();
-        int32_t* cp = col_ptr + (size_t)tile * (T + 1);
-        if (worker) {
-            int o = cnt[j * seg + sg];
-            if (sg == 0) cp[j] = o;
-            float* ev = ent_val + (size_t)tile * cap;
-            uint16_t* er = ent_row + (size_t)tile * cap;
-            for (int r = r0; r < r1; ++r) {
-                const float a = M[r * T + j];
-                if (a != 0.0f && o < cap) {
-                    ev[o] = a;
-                    er[o] = (uint16_t)r;
-                    ++o;
-                }
-            }
-        }
-        if (tid == 0) cp[T] = total < cap ? total : cap;
-        __syncthreads();                                              // M is overwritten by the next tile
-    }
-}
-
 // Fused foreground-token selection (protopformer.py:157-158 / deit_models_attn.py:229-230) on the finished score row:
 // rank by counting over the W scores in shared memory (larger score first, lower index first on ties -- the rule of
 // pph_select_topk), emitted in ascending token order.  All kRoChainThreads threads call it; W <= kRoChainThreads.
@@ -397,7 +219,6 @@ rollout_chain_kernel(int L, int B, int T, int cap, const int32_t* __restrict__ c
                      const float* __restrict__ ent_val, const uint16_t* __restrict__ ent_row,
                      const float* __restrict__ v0, int drop_first, float* __restrict__ scores, int K,
                       int32_t* __restrict__ idx32, int64_t* __restrict__ idx64) {
-    pdl_sync();
     __shared__ int wcnt[kRoChainThreads / 32];
     __shared__ float v[2][kRoMaxT];
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -433,17 +254,17 @@ rollout_chain_kernel(int L, int B, int T, int cap, const int32_t* __restrict__ c
 
 
 // ---------------------------------------------------------------------------------------------------------------
-// v2 (default).  ncu on v1 (profiles/r1b_ncu_rollout_v1.txt): 449 us for 328 MB = 9 % of HBM, 13 k instructions per
-// warp per tile, ADU (vote / match / shared atomics) and XU (IEEE divisions) pipes busiest -- instruction bound, not
-// memory bound.  Changes:
-//   * radix select in 3 passes of 11/11/10 bits with plain shared-memory atomics on a 2048-bin histogram: the
-//     8-bit first digit of v1 put ~40 % of all entries into ONE bin (same exponent), so its warp-aggregated atomics
-//     still serialised on one address; with 11 bits the hottest bin holds a few percent and no vote / match is needed;
+// Why the prepare kernel looks the way it does.  ncu on a first version (profiles/r1b_ncu_rollout_v1.txt): 449 us for
+// 328 MB = 9 % of HBM, 13 k instructions per warp per tile, ADU (vote / match / shared atomics) and XU (IEEE divisions)
+// pipes busiest -- instruction bound, not memory bound.  Hence:
+//   * radix select in 3 passes of 11/11/10 bits with plain shared-memory atomics on a 2048-bin histogram: an 8-bit
+//     first digit put ~40 % of all entries into ONE bin (same exponent), so even warp-aggregated atomics serialised on
+//     one address; with 11 bits the hottest bin holds a few percent and no vote / match is needed;
 //   * zero entries (90 % after the discard) skip both divisions of the normalisation;
 //   * the chain kernel stages each layer's sparse matrix in shared memory with coalesced loads and walks one column
 //     per THREAD (independent sequential sums) instead of one dependent global-load chain per warp and column.
-// Results are bit-identical to v1 (same arithmetic, same summation order per column is NOT kept: v1 summed a column
-// lane-strided then by shuffle tree, v2 sums it in row order; both are fixed orders -> each version is reproducible).
+// The two chain kernels sum a column in different fixed orders (rollout_chain_kernel lane-strided then by shuffle
+// tree, rollout_chain2_kernel in row order): each is reproducible, and which one runs depends on the shape alone.
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kRo2Bins = 2048;
 
@@ -451,8 +272,7 @@ template <int HT, class E>
 __global__ void __launch_bounds__(kRoThreads, 1)
 rollout_prepare2_kernel(const RoLayers<E> layers, int L, int B, int H, int T, int k_discard, int head_fusion,
                         float identity_w, int cap, int32_t* __restrict__ col_ptr, float* __restrict__ ent_val,
-                        uint16_t* __restrict__ ent_row, int norm_mode) {
-    pdl_sync();
+                        uint16_t* __restrict__ ent_row) {
     extern __shared__ __align__(16) uint8_t ro_smem[];
     const int n = T * T;
     float* M = reinterpret_cast<float*>(ro_smem);                            // [T*T]
@@ -469,7 +289,7 @@ rollout_prepare2_kernel(const RoLayers<E> layers, int L, int B, int H, int T, in
 
     for (int tile = blockIdx.x; tile < L * B; tile += gridDim.x) {
         const int l = tile / B, b = tile - l * B;
-        // ---- 1. stream + fuse the head maps (as v1, same element type rule) ----
+        // ---- 1. stream the H head maps once, fuse (deit_models_attn.py:102-107); 8 x H loads in flight per thread ----
         const E* A = layers.p[l] + (size_t)b * Hh * n;
         if constexpr (sizeof(E) == 2) {
             ro_stream_fuse_half<HT>(A, n, Hh, head_fusion, M);
@@ -557,43 +377,30 @@ rollout_prepare2_kernel(const RoLayers<E> layers, int L, int B, int H, int T, in
         }
 
         // ---- 4. a = (A + w I) / (1 + w), rows normalised; zero off-diagonal entries stay zero without arithmetic ----
+        // (both column loops unrolled by 4: left rolled, the DeiT-Ti B = 64 rollout took 295 instead of 284 us, B200 at 1000 W)
         const float den = 1.0f + identity_w;
-        if (norm_mode == 0) {
-            for (int r = warp; r < T; r += kRoThreads / 32) {
-                float* row = M + r * T;
-                float s = 0.f;
-                for (int j = lane; j < T; j += 32) {
-                    const float x = row[j];
-                    if (x != 0.0f || j == r) {
-                        const float a = (x + (j == r ? identity_w : 0.0f)) / den;
-                        row[j] = a;
-                        s += a;
-                    }
-                }
-                s = warp_sum(s);
-                for (int j = lane; j < T; j += 32) {
-                    const float a = row[j];
-                    if (a != 0.0f) row[j] = a / s;
+        for (int r = warp; r < T; r += kRoThreads / 32) {
+            float* row = M + r * T;
+            float s = 0.f;
+#pragma unroll 4
+            for (int j = lane; j < T; j += 32) {
+                const float x = row[j];
+                if (x != 0.0f || j == r) {
+                    const float a = (x + (j == r ? identity_w : 0.0f)) / den;
+                    row[j] = a;
+                    s += a;
                 }
             }
-        } else {
-            // PPH_ROLLOUT=3 (NOT yet validated on a GPU: written after round 1's budget was spent).  ncu on the exact
-            // form: this step is 33 % of the kernel's instructions -- two IEEE divisions per entry that warp divergence
-            // makes every lane pay although 90 % of the entries are zero.  The 1/(1+w) factor cancels in the row
-            // normalisation, so a_ij = (x_ij + w d_ij) * (1 / (sum_j x_ij + w)): one reciprocal per row, one multiply
-            // per entry; differs from the reference's two roundings by <= 2 ulp (parity bar of this row: 1e-5).
-            for (int r = warp; r < T; r += kRoThreads / 32) {
-                float* row = M + r * T;
-                float s = 0.f;
-                for (int j = lane; j < T; j += 32) s += row[j];
-                s = warp_sum(s) + identity_w;
-                const float rs = 1.0f / s;
-                for (int j = lane; j < T; j += 32) row[j] = (row[j] + (j == r ? identity_w : 0.0f)) * rs;
+            s = warp_sum(s);
+#pragma unroll 4
+            for (int j = lane; j < T; j += 32) {
+                const float a = row[j];
+                if (a != 0.0f) row[j] = a / s;
             }
         }
         __syncthreads();
 
-        // ---- 5. column-compressed sparse output (as v1) ----
+        // ---- 5. column-compressed sparse output: thread = (row segment sg, column j), entries ordered by (j, row) ----
         const bool worker = tid < seg * T;
         const int sg = tid / T, j = tid - sg * T;
         const int r0 = sg * rps, r1 = min(T, r0 + rps);
@@ -634,7 +441,6 @@ rollout_chain2_kernel(int L, int B, int T, int cap, const int32_t* __restrict__ 
                       const float* __restrict__ ent_val, const uint16_t* __restrict__ ent_row,
                       const float* __restrict__ v0, int drop_first, float* __restrict__ scores, int K,
                       int32_t* __restrict__ idx32, int64_t* __restrict__ idx64) {
-    pdl_sync();
     __shared__ int wcnt[kRoChainThreads / 32];
     extern __shared__ __align__(16) uint8_t ch_smem[];
     float* sval = reinterpret_cast<float*>(ch_smem);                          // [cap]
@@ -691,7 +497,6 @@ template <class E>
 __global__ void __launch_bounds__(kRoClsThreads)
 rollout_cls_rows_kernel(const RoLayers<E> layers, int n_cls, int B, int H, int Tc, int k_discard, int head_fusion,
                         float identity_w, float* __restrict__ v0) {
-    pdl_sync();
     __shared__ float x[kRoClsThreads], acc[kRoClsThreads], wred[kRoClsThreads / 32];
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     acc[tid] = 0.0f;
@@ -759,15 +564,9 @@ static int rollout_scores_impl(const char* fn, const E* const* attn_layers, int 
     char what_prep[96], what_chain[96];
     snprintf(what_prep, sizeof what_prep, "%s(prepare)", fn);
     snprintf(what_chain, sizeof what_chain, "%s(chain)", fn);
-    // PPH_ROLLOUT=1 selects the first version of both kernels (kept for A/B measurements)
-    const bool use_v1 = option(kOptRollout) == 1;
-    // default: one reciprocal per row instead of two IEEE divisions per entry (261.7 vs 292.4 us at the DeiT-Ti shape,
-    // within 2 ulp of the reference's two roundings, held to the same fixtures); PPH_ROLLOUT=2 keeps the divisions
-    const int norm_mode = option(kOptRollout) == 2 ? 0 : 1;
-    const size_t smem1 = (size_t)((n + 3) & ~3) * 4 + 256 * 4 + (kRoThreads + 40) * 4;
-    const size_t smem2 = (size_t)((n + 3) & ~3) * 4 + kRo2Bins * 4 + (kRoThreads + 40) * 4;
-    const bool v1 = use_v1 || smem2 > 220 * 1024;
-    const size_t smem = v1 ? smem1 : smem2;
+    // the fused map of the largest T fits: kRoMaxT^2 * 4 + scratch <= the 220 KB opted in below
+    static_assert((size_t)kRoMaxT * kRoMaxT * 4 + kRo2Bins * 4 + (kRoThreads + 40) * 4 <= 220 * 1024, "kRoMaxT");
+    const size_t smem = (size_t)((n + 3) & ~3) * 4 + kRo2Bins * 4 + (kRoThreads + 40) * 4;
     int sms = pph_sm_count();            // per call: the current device may differ between calls
     if (sms <= 0) sms = 148;
     const int tiles = L * B;
@@ -780,25 +579,14 @@ static int rollout_scores_impl(const char* fn, const E* const* attn_layers, int 
                  w.col_ptr, w.ent_val, w.ent_row);
         return launch_status(what_prep);
     };
-    auto go2 = [&](auto kern) -> int {
-        cudaError_t e = opt_in_smem(kern, 220 * 1024);
-        if (e != cudaSuccess) { set_error("%s: cudaFuncSetAttribute: %s", fn, cudaGetErrorString(e)); return (int)e; }
-        launch_k(kern, grid, dim3(kRoThreads), smem, st, layers, L, B, H, T, k_discard, head_fusion, identity_w, w.cap,
-                 w.col_ptr, w.ent_val, w.ent_row, norm_mode);
-        return launch_status(what_prep);
-    };
     // head counts of the reference's backbones: DeiT-Ti 3, CaiT-XXS 4, DeiT-S 6 (deit_models_attn.py:288,303)
-    int rc;
-    if (v1)
-        rc = H == 3 ? go(rollout_prepare_kernel<3, E>) : H == 4 ? go(rollout_prepare_kernel<4, E>)
-             : H == 6 ? go(rollout_prepare_kernel<6, E>) : go(rollout_prepare_kernel<0, E>);
-    else
-        rc = H == 3 ? go2(rollout_prepare2_kernel<3, E>) : H == 4 ? go2(rollout_prepare2_kernel<4, E>)
-             : H == 6 ? go2(rollout_prepare2_kernel<6, E>) : go2(rollout_prepare2_kernel<0, E>);
+    const int rc = H == 3 ? go(rollout_prepare2_kernel<3, E>) : H == 4 ? go(rollout_prepare2_kernel<4, E>)
+                   : H == 6 ? go(rollout_prepare2_kernel<6, E>) : go(rollout_prepare2_kernel<0, E>);
     if (rc) return rc;
-    // staged chain needs the layer's entry list in shared memory (cap * 6 B): small discard ratios fall back to v1
+    // the staged chain needs the layer's entry list in shared memory (cap * 6 B): small discard ratios at large T
+    // (T = 197 below a ratio of about 0.3) walk it from global memory instead
     const size_t csmem = (size_t)w.cap * 4 + (size_t)(T + 1) * 4 + (size_t)w.cap * 2 + 16;
-    if (!use_v1 && csmem <= 160 * 1024) {
+    if (csmem <= 160 * 1024) {
         cudaError_t e = opt_in_smem(rollout_chain2_kernel, 160 * 1024);
         if (e != cudaSuccess) { set_error("%s: cudaFuncSetAttribute: %s", fn, cudaGetErrorString(e)); return (int)e; }
         launch_k(rollout_chain2_kernel, dim3(B), dim3(kRoChainThreads), csmem, st, L, B, T, w.cap, w.col_ptr, w.ent_val,

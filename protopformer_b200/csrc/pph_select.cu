@@ -18,7 +18,6 @@ constexpr int kSelMaxN = 1024;
 __global__ void __launch_bounds__(kSelThreads)
 select_topk_kernel(const float* __restrict__ scores, int H, int N, int K,
                    int32_t* __restrict__ idx32, int64_t* __restrict__ idx64) {
-    pdl_sync();
     __shared__ __align__(16) float s[kSelMaxN];
     __shared__ int warp_cnt[kSelThreads / 32];
     const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;

@@ -39,7 +39,6 @@ __device__ __forceinline__ void gemm_load_tile(float (*dst)[kGemmBM + kGemmPad],
 template <bool kRowSum, class AOp, class BOp, class Epi>
 __global__ void __launch_bounds__(kGemmThreads)
 sgemm_kernel(int M, int N, int Kd, int k_per_split, AOp a_op, BOp b_op, Epi epi) {
-    pdl_sync();
     __shared__ __align__(16) float As[kGemmBK][kGemmBM + kGemmPad];
     __shared__ __align__(16) float Bs[kGemmBK][kGemmBN + kGemmPad];
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;

@@ -92,7 +92,6 @@ __device__ __forceinline__ void group_bar(int g) { asm volatile("bar.sync %0, %1
 
 __global__ void __launch_bounds__(kG2TokThreads, 1)
 grad2_tokens_kernel(const Grad2Args a) {
-    pdl_sync();
     extern __shared__ __align__(16) float sm_g2[];
     const int K = a.K, P = a.P, D = a.D;
     const int NC = (P + kG2CH - 1) / kG2CH;                 // chunks per image
@@ -216,7 +215,6 @@ grad2_tokens_kernel(const Grad2Args a) {
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kG2ProThreads)
 grad2_protos_kernel(const Grad2Args a) {
-    pdl_sync();
     extern __shared__ __align__(16) float sm_g2[];
     const int K = a.K, D = a.D, B = a.B, P = a.P, R = K + 1;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -302,7 +300,6 @@ grad2_protos_kernel(const Grad2Args a) {
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kG2ClsThreads)
 grad2_cls_kernel(const Grad2Args a) {
-    pdl_sync();
     extern __shared__ __align__(16) float sm_g2[];
     const int D = a.D, Pg = a.Pg, B = a.B, P = a.P;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarp = kG2ClsThreads / 32;

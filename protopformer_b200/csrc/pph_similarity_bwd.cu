@@ -9,7 +9,6 @@
 //   bin_tokens_kernel : per image, stable counting sort of the prototypes by argmin token (one warp, match.any) ->
 //                       deterministic bins, so every gradient row is summed in a fixed order (bit-reproducible).
 #include "pph_common.cuh"
-#include "pph_tc_ptx.cuh"
 #include "pph_bins.cuh"
 #include "pph_step2.cuh"
 
@@ -18,7 +17,6 @@ namespace pph {
 __global__ void __launch_bounds__(256)
 bin_tokens_kernel(int4* __restrict__ item_desc, const int32_t* __restrict__ argmin_l, int K, int P, int32_t* __restrict__ bin_start,
                   int32_t* __restrict__ item_start, int32_t* __restrict__ bin_list) {
-    pdl_sync();
     extern __shared__ int smi[];
     bin_tokens_body<false>(blockIdx.x, argmin_l, K, P, bin_start, item_start, bin_list, smi, item_desc);
 }
@@ -287,7 +285,6 @@ cls_grad_body(int slice, int bgroup, int nslices, const float* __restrict__ g_g,
 __global__ void __launch_bounds__(256)
 ppc_rows_add_kernel(const float* __restrict__ dP_img, const int32_t* __restrict__ cls_start,
                     const int32_t* __restrict__ cls_order, int P, int D, int m, float* __restrict__ dPl) {
-    pdl_sync();
     const int p = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (p >= P) return;
     const int cls = p / m, jj = p - cls * m;
@@ -347,7 +344,6 @@ sim_grads_kernel(const float* __restrict__ g_l, const float* __restrict__ g_g, c
                  unsigned int* cls_counters, const float* __restrict__ add_dZs, const float* __restrict__ add_dPl,
                  float* __restrict__ dZs, float* __restrict__ dZc, float* __restrict__ dPl, float* __restrict__ dPg,
                  const BwdExtras ex) {
-    pdl_sync();
     int vb = blockIdx.x;
     if (vb < n_cls) {
         cls_grad_body(vb % n_slices, vb / n_slices, n_slices, g_g, Zc, Pgl, B, D, Pg, p_per_slice, cls_part, cls_counters, dZc,
@@ -364,205 +360,6 @@ sim_grads_kernel(const float* __restrict__ g_l, const float* __restrict__ g_g, c
                               tok_gsum, tok_counters, add_dZs, dZs, ex);
 }
 
-// ---- the same gathers through the bulk-copy engine ---------------------------------------------------------------------
-// The register gathers above are bound by how many loads an SM can keep outstanding (64 registers x 32 warps: ~50 KB in
-// flight per SM, ~6 TB/s over the machine at L2 latency).  Here every lane hands ONE whole row (D floats, contiguous) to
-// cp.async.bulk: a warp's 16 rows land in its own shared-memory buffer and complete on its own mbarrier -- 12 KB in flight
-// per warp, 16 warps per SM, no registers held by data in flight.  Same entry order, same fmaf sequence -> the same bits.
-constexpr int kBulkRows = 16;
-
-__device__ __forceinline__ void bulk_row_g2s(float* dst, const float* src, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(ptx::smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(ptx::smem_u32(bar))
-                 : "memory");
-}
-// lanes u < n fetch the row at `src` (their own pointer) into rows[u]; returns when all n rows have landed
-__device__ __forceinline__ void bulk_rows(float* rows, const float* src, int n, int D, uint64_t* bar, uint32_t& phase) {
-    const int lane = threadIdx.x & 31;
-    __syncwarp();                                             // the previous batch has been consumed by every lane
-    if (lane == 0) ptx::mbar_expect_tx(bar, (uint32_t)n * (uint32_t)D * 4u);
-    __syncwarp();
-    if (lane < n) bulk_row_g2s(rows + (size_t)lane * D, src, (uint32_t)D * 4u, bar);
-    ptx::mbar_wait(bar, phase);
-    phase ^= 1u;
-}
-
-template <int DV, bool FULL>
-__device__ __forceinline__ void
-proto_grad_bulk(int vb, float* rows, uint64_t* bar, uint32_t& phase, const float* __restrict__ g_l, const float* __restrict__ g_g,
-                const int32_t* __restrict__ argmin_l, const float* __restrict__ Zs, const float* __restrict__ Zc,
-                const float* __restrict__ Pl, const float* __restrict__ Pgl, int B, int K, int D, int P, int Pg,
-                const float* __restrict__ add_dPl, float* __restrict__ dPl, float* __restrict__ dPg, const BwdExtras& ex) {
-    const int row = vb * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (row >= P + Pg) return;
-    const bool global = row >= P;
-    const int p = global ? row - P : row;
-    const int np = global ? Pg : P;
-    const float* g = global ? g_g : g_l;
-    float acc[DV];
-#pragma unroll
-    for (int i = 0; i < DV; ++i) acc[i] = 0.f;
-    float gsum = 0.f;
-    for (int b0 = 0; b0 < B; b0 += 32) {
-        const int bl = b0 + lane;
-        const float gv = bl < B ? __ldg(g + (size_t)bl * np + p) : 0.f;
-        const int av = (!global && bl < B) ? __ldg(argmin_l + (size_t)bl * P + p) : 0;
-        const int cnt = min(32, B - b0);
-        for (int t0 = 0; t0 < cnt; t0 += kBulkRows) {
-            const int n = min(kBulkRows, cnt - t0);
-            const int aa = __shfl_sync(0xffffffffu, av, (t0 + lane) & 31);
-            const int bb = min(b0 + t0 + lane, B - 1);
-            bulk_rows(rows, global ? Zc + (size_t)bb * D : Zs + ((size_t)bb * K + aa) * D, n, D, bar, phase);
-            for (int u = 0; u < n; ++u) {
-                const float gg = __shfl_sync(0xffffffffu, gv, t0 + u);
-                gsum += gg;
-#pragma unroll
-                for (int i = 0; i < DV; ++i)
-                    if (FULL || i * 32 + lane < D) acc[i] = fmaf(gg, rows[(size_t)u * D + i * 32 + lane], acc[i]);
-            }
-        }
-    }
-    const float* pr = (global ? Pgl : Pl) + (size_t)p * D;
-    float* out = (global ? dPg : dPl) + (size_t)p * D;
-    const float* add = (!global && add_dPl) ? add_dPl + (size_t)p * D : nullptr;
-    int c0 = 0, c1 = 0, jj = 0;
-    if (!global && ex.dP_img) {
-        const int cls = p / ex.m;
-        jj = p - cls * ex.m;
-        c0 = __ldg(ex.cls_start + cls);
-        c1 = __ldg(ex.cls_start + cls + 1);
-    }
-#pragma unroll
-    for (int i = 0; i < DV; ++i)
-        if (FULL || i * 32 + lane < D) {
-            float r = 2.0f * (__ldg(pr + i * 32 + lane) * gsum - acc[i]) + (add ? __ldg(add + i * 32 + lane) : 0.f);
-            for (int c = c0; c < c1; ++c)
-                r += __ldg(ex.dP_img + ((size_t)__ldg(ex.cls_order + c) * ex.m + jj) * D + i * 32 + lane);
-            out[i * 32 + lane] = r;
-        }
-}
-
-template <int DV, bool FULL>
-__device__ __forceinline__ void
-token_grad_bulk(int vb, float* rows, uint64_t* bar, uint32_t& phase, const float* __restrict__ g_l,
-                const int4* __restrict__ item_desc, const int32_t* __restrict__ bin_list, const float* __restrict__ Zs,
-                const float* __restrict__ Pl, int B, int K, int D, int P, int items_per_image, float* part, float* part_gsum,
-                unsigned int* counters, const float* __restrict__ add_dZs, float* __restrict__ dZs, const BwdExtras& ex) {
-    const int gw = vb * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    const int b = gw / items_per_image, item = gw - b * items_per_image;
-    if (b >= B) return;
-    const int4 dsc = __ldg(item_desc + (size_t)b * items_per_image + item);
-    if (dsc.x < 0) return;
-    const int k = dsc.x, e0 = dsc.y, e1 = dsc.z, nchunks = dsc.w & 0xffff, chunk = dsc.w >> 16;
-    const int32_t* list = bin_list + (size_t)b * P;
-    const float* gb = g_l + (size_t)b * P;
-    float acc[DV];
-#pragma unroll
-    for (int i = 0; i < DV; ++i) acc[i] = 0.f;
-    float gsum = 0.f;
-    {
-        const int e = e0 + lane;
-        const int pv = e < e1 ? __ldg(list + e) : 0;
-        const float gv = e < e1 ? __ldg(gb + pv) : 0.f;
-        const int cnt = max(0, e1 - e0);
-        for (int t0 = 0; t0 < cnt; t0 += kBulkRows) {
-            const int n = min(kBulkRows, cnt - t0);
-            const int pp = __shfl_sync(0xffffffffu, pv, (t0 + lane) & 31);
-            bulk_rows(rows, Pl + (size_t)pp * D, n, D, bar, phase);
-            for (int u = 0; u < n; ++u) {
-                const float gg = __shfl_sync(0xffffffffu, gv, t0 + u);
-                gsum += gg;
-#pragma unroll
-                for (int i = 0; i < DV; ++i)
-                    if (FULL || i * 32 + lane < D) acc[i] = fmaf(gg, rows[(size_t)u * D + i * 32 + lane], acc[i]);
-            }
-        }
-    }
-    const size_t row = (size_t)b * K + k;
-    const float* zr = Zs + row * D;
-    float* out = dZs + row * D;
-    const float* add = add_dZs ? add_dZs + row * D : nullptr;
-    if (nchunks == 1) {
-#pragma unroll
-        for (int i = 0; i < DV; ++i)
-            if (FULL || i * 32 + lane < D) {
-                const float z = __ldg(zr + i * 32 + lane);
-                float r = 2.0f * (z * gsum - acc[i]) + (add ? __ldg(add + i * 32 + lane) : 0.f);
-                if (ex.dpre_out) r *= z * (1.0f - z);
-                out[i * 32 + lane] = r;
-            }
-        return;
-    }
-    const size_t slot = (size_t)b * items_per_image + item;
-#pragma unroll
-    for (int i = 0; i < DV; ++i)
-        if (FULL || i * 32 + lane < D) part[slot * D + i * 32 + lane] = acc[i];
-    if (lane == 0) part_gsum[slot] = gsum;
-    __threadfence();
-    __syncwarp();
-    unsigned int ticket = 0;
-    if (lane == 0) ticket = atomicAdd(counters + row, 1u);
-    ticket = __shfl_sync(0xffffffffu, ticket, 0);
-    if (ticket != (unsigned int)(nchunks - 1)) return;
-    __threadfence();
-    const size_t slot0 = slot - chunk;
-    float tot[DV];
-#pragma unroll
-    for (int i = 0; i < DV; ++i) tot[i] = 0.f;
-    float gt = 0.f;
-    for (int c = 0; c < nchunks; ++c) {
-        gt += __ldcg(part_gsum + slot0 + c);
-#pragma unroll
-        for (int i = 0; i < DV; ++i)
-            if (FULL || i * 32 + lane < D) tot[i] += __ldcg(part + (slot0 + c) * D + i * 32 + lane);
-    }
-#pragma unroll
-    for (int i = 0; i < DV; ++i)
-        if (FULL || i * 32 + lane < D) {
-            const float z = __ldg(zr + i * 32 + lane);
-            float r = 2.0f * (z * gt - tot[i]) + (add ? __ldg(add + i * 32 + lane) : 0.f);
-            if (ex.dpre_out) r *= z * (1.0f - z);
-            out[i * 32 + lane] = r;
-        }
-    if (lane == 0) counters[row] = 0u;
-}
-
-template <int DV, bool FULL>
-__global__ void __launch_bounds__(256)
-sim_grads_bulk_kernel(const float* __restrict__ g_l, const float* __restrict__ g_g, const int32_t* __restrict__ argmin_l,
-                      const int4* __restrict__ item_desc, const int32_t* __restrict__ bin_list, const float* __restrict__ Zs,
-                      const float* __restrict__ Zc, const float* __restrict__ Pl, const float* __restrict__ Pgl, int B, int K, int D,
-                      int P, int Pg, int items_per_image, int n_cls, int n_slices, int p_per_slice, int n_proto, float* tok_part,
-                      float* tok_gsum, unsigned int* tok_counters, float* cls_part, unsigned int* cls_counters,
-                      const float* __restrict__ add_dZs, const float* __restrict__ add_dPl, float* __restrict__ dZs,
-                      float* __restrict__ dZc, float* __restrict__ dPl, float* __restrict__ dPg, const BwdExtras ex) {
-    pdl_sync();
-    extern __shared__ __align__(128) uint8_t bulk_smem[];
-    int vb = blockIdx.x;
-    if (vb < n_cls) {
-        cls_grad_body(vb % n_slices, vb / n_slices, n_slices, g_g, Zc, Pgl, B, D, Pg, p_per_slice, cls_part, cls_counters, dZc,
-                      ex.dpre_out);
-        return;
-    }
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    float* rows = reinterpret_cast<float*>(bulk_smem) + (size_t)warp * kBulkRows * D;
-    uint64_t* bar = reinterpret_cast<uint64_t*>(bulk_smem + (size_t)8 * kBulkRows * D * sizeof(float)) + warp;
-    if (lane == 0) {
-        ptx::mbar_init(bar, 1);
-        ptx::fence_mbar_init();
-    }
-    __syncwarp();
-    uint32_t phase = 0;
-    vb -= n_cls;
-    if (vb < n_proto) {
-        proto_grad_bulk<DV, FULL>(vb, rows, bar, phase, g_l, g_g, argmin_l, Zs, Zc, Pl, Pgl, B, K, D, P, Pg, add_dPl, dPl, dPg, ex);
-        return;
-    }
-    vb -= n_proto;
-    token_grad_bulk<DV, FULL>(vb, rows, bar, phase, g_l, item_desc, bin_list, Zs, Pl, B, K, D, P, items_per_image, tok_part, tok_gsum,
-                              tok_counters, add_dZs, dZs, ex);
-}
-
 template <int DV, bool FULL>
 static int launch_bwd(const float* g_l, const float* g_g, const int32_t* argmin_l, const BwdWorkspace& w,
                       const float* Zs, const float* Zc, const float* Pl, const float* Pgl,
@@ -576,15 +373,6 @@ static int launch_bwd(const float* g_l, const float* g_g, const int32_t* argmin_
     const int n_cls = (roles & 1) ? nsl * ceil_div(B, kClsTB) : 0;
     const int n_proto = (roles & 2) ? ceil_div(P + Pg, 8) : 0;
     const int n_tok = (roles & 1) ? ceil_div(B * w.items_per_image, 8) : 0;
-    const size_t bulk_bytes = (size_t)8 * kBulkRows * D * sizeof(float) + 8 * sizeof(uint64_t);
-    if (option(kOptGather) == 1 && D % 4 == 0 && bulk_bytes <= 110 * 1024) {       // rows through the bulk-copy engine
-        cudaError_t e = opt_in_smem(sim_grads_bulk_kernel<DV, FULL>, bulk_bytes);
-        if (e != cudaSuccess) { set_error("pph_similarity_bwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return (int)e; }
-        launch_k(sim_grads_bulk_kernel<DV, FULL>, dim3(n_cls + n_proto + n_tok), dim3(256), bulk_bytes, st, g_l, g_g, argmin_l,
-                 w.item_desc, w.bin_list, Zs, Zc, Pl, Pgl, B, K, D, P, Pg, w.items_per_image, n_cls, nsl, p_per_slice, n_proto,
-                 w.tok_part, w.tok_gsum, w.tok_counters, w.cls_part, w.cls_counters, add_dZs, add_dPl, dZs, dZc, dPl, dPg, ex);
-        return launch_status("pph_similarity_bwd(grads, bulk rows)");
-    }
     launch_k(sim_grads_kernel<DV, FULL>, dim3(n_cls + n_proto + n_tok), dim3(256), (size_t)(0), st, g_l, g_g, argmin_l, w.item_desc, w.bin_list, Zs, Zc, Pl, Pgl, B, K, D, P, Pg, w.items_per_image, n_cls, nsl, p_per_slice, n_proto, w.tok_part, w.tok_gsum, w.tok_counters, w.cls_part, w.cls_counters, add_dZs, add_dPl, dZs, dZc, dPl, dPg, ex);
     return launch_status("pph_similarity_bwd(grads)");
 }

@@ -19,7 +19,6 @@ similarity_local_simt_kernel(const float* __restrict__ Zs, const float* __restri
                              int K, int D, int P, int act_fn, float eps,
                              float* __restrict__ dmin, int32_t* __restrict__ argmin, float* __restrict__ act,
                              float* __restrict__ dist_map, float* __restrict__ act_map) {
-    pdl_sync();
     __shared__ __align__(16) float Zt[kSimBK][kSimTok + 4];
     __shared__ __align__(16) float Pt[kSimBK][kSimProt + 4];
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;

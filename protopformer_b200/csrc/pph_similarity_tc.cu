@@ -82,7 +82,7 @@ __device__ __forceinline__ float4 lds_f4(uint32_t saddr) {
     return v;
 }
 
-// Local tile, compile-time token count, latency-tolerant form (EPI = 1).  The straightforward running
+// Local tile, compile-time token count, latency-tolerant form.  The straightforward running
 // (min, argmin) scan is ONE dependent compare->select chain of K links per image (~10 cycles per link with 1-2
 // epilogue warps per scheduler: ncu put the 128 x 243 tile at ~4.3 k cycles, 3x the MMA time of the bf16 mode).
 // Here every image keeps four independent (min, argmin) chains over the token slots k = 0,1,2,3 (mod 4), merged at the
@@ -142,10 +142,10 @@ __device__ __forceinline__ void tc_epilogue_local_ilp(const TcParams& prm, const
 }
 
 // Drain one accumulator tile: thread = prototype row (TMEM lane), walks its columns with tcgen05.ld.
-template <int KT, int EPI = 1>
+template <int KT>
 __device__ __forceinline__ void tc_epilogue_tile(const TcParams& prm, const TcTile& t, uint32_t taddr, const float* x2,
-                                                 const float4* x2v, int quarter, int lane) {
-    if constexpr (KT >= 4 && EPI == 1) {
+                                                 int quarter, int lane) {
+    if constexpr (KT >= 4) {
         if (!t.is_global) {
             tc_epilogue_local_ilp<KT>(prm, t, taddr, ptx::smem_u32(x2), quarter, lane);
             return;
@@ -168,48 +168,22 @@ __device__ __forceinline__ void tc_epilogue_tile(const TcParams& prm, const TcTi
         };
         float best = INFINITY;
         int bk = 0;
-        if constexpr (KT > 0) {
-            constexpr int GS = kTcMaxN / KT, TC = GS * KT;
+        const int Kc = prm.K;
+        const int gcnt = min(prm.G, prm.B - b0);
+        const int ncols = gcnt * Kc;
+        int g = 0, k = 0;
+        for (int c0 = 0; c0 < ncols; c0 += 32) {
+            uint32_t v[32];
+            ptx::tmem_ld_32x32(taddr + c0, v);
+            ptx::tmem_ld_wait(v);
 #pragma unroll
-            for (int ch = 0; ch < (TC + 31) / 32; ++ch) {
-                uint32_t v[32];
-                ptx::tmem_ld_32x32(taddr + ch * 32, v);
-                float4 xq[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) xq[i] = x2v[ch * 8 + i];
-                ptx::tmem_ld_wait(v);
-#pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    const int col = ch * 32 + j;
-                    if (col < TC) {
-                        const int k = col % KT, g = col / KT;
-                        const float4 q = xq[j >> 2];
-                        const float xx = (j & 3) == 0 ? q.x : (j & 3) == 1 ? q.y : (j & 3) == 2 ? q.z : q.w;
-                        const float d = fmaf(-2.0f, __uint_as_float(v[j]), xx);
-                        if (k == 0) { best = d; bk = 0; }
-                        else if (d < best) { best = d; bk = k; }
-                        if (k == KT - 1) store(g, best, bk);
-                    }
-                }
-            }
-        } else {
-            const int Kc = prm.K;
-            const int gcnt = min(prm.G, prm.B - b0);
-            const int ncols = gcnt * Kc;
-            int g = 0, k = 0;
-            for (int c0 = 0; c0 < ncols; c0 += 32) {
-                uint32_t v[32];
-                ptx::tmem_ld_32x32(taddr + c0, v);
-                ptx::tmem_ld_wait(v);
-#pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    if (c0 + j < ncols) {
-                        const float d = fmaf(-2.0f, __uint_as_float(v[j]), x2[c0 + j]);
-                        if (d < best) { best = d; bk = k; }
-                        if (++k == Kc) {
-                            store(g, best, bk);
-                            ++g; k = 0; best = INFINITY; bk = 0;
-                        }
+            for (int j = 0; j < 32; ++j) {
+                if (c0 + j < ncols) {
+                    const float d = fmaf(-2.0f, __uint_as_float(v[j]), x2[c0 + j]);
+                    if (d < best) { best = d; bk = k; }
+                    if (++k == Kc) {
+                        store(g, best, bk);
+                        ++g; k = 0; best = INFINITY; bk = 0;
                     }
                 }
             }
@@ -267,7 +241,6 @@ similarity_tc_kernel(const __grid_constant__ CUtensorMap tmAl_hi, const __grid_c
         for (int s = 0; s < 2; ++s) { ptx::mbar_init(&tmem_full[s], 1); ptx::mbar_init(&tmem_empty[s], 4); }
         ptx::fence_mbar_init();
     }
-    pdl_sync();   // barriers and tensor-map prefetch overlap the previous kernel; TMEM and all global reads wait for it
     if (warp == 2) ptx::tmem_alloc(tmem_ptr, 512);
     ptx::tc_fence_before();
     __syncthreads();
@@ -346,7 +319,6 @@ similarity_tc_kernel(const __grid_constant__ CUtensorMap tmAl_hi, const __grid_c
         const int quarter = warp & 3;                // TMEM lane quarter this warp may read
         const int gtid = threadIdx.x - 128 - grp_id * 128;   // 0..127 inside the group
         float* x2 = x2s + grp_id * kTcMaxN;
-        const float4* x2v = reinterpret_cast<const float4*>(x2);
         int it = 0;
         for (int tile = blockIdx.x; tile < prm.n_tiles; tile += gridDim.x, ++it) {
             if ((it & 1) != grp_id) continue;
@@ -366,7 +338,7 @@ similarity_tc_kernel(const __grid_constant__ CUtensorMap tmAl_hi, const __grid_c
 
             ptx::mbar_wait(&tmem_full[grp_id], acc_phase);
             ptx::tc_fence_after();
-            tc_epilogue_tile<KT>(prm, t, taddr, x2, x2v, quarter, lane);
+            tc_epilogue_tile<KT>(prm, t, taddr, x2, quarter, lane);
             ptx::tc_fence_before();
             __syncwarp();
             if (lane == 0) ptx::mbar_arrive(&tmem_empty[grp_id]);
@@ -425,7 +397,7 @@ __host__ __device__ __forceinline__ bool tc2_phase(const TcParams& prm, int cta,
     return true;
 }
 
-template <int NTERMS, int KT, int EPI>
+template <int NTERMS, int KT>
 __global__ void __launch_bounds__(kTcThreads, 1)
 similarity_tc2_kernel(const __grid_constant__ CUtensorMap tmAl_hi, const __grid_constant__ CUtensorMap tmAl_lo,
                       const __grid_constant__ CUtensorMap tmBl_hi, const __grid_constant__ CUtensorMap tmBl_lo,
@@ -464,7 +436,6 @@ similarity_tc2_kernel(const __grid_constant__ CUtensorMap tmAl_hi, const __grid_
         ptx::mbar_init(a_empty, 1);
         ptx::fence_mbar_init();
     }
-    pdl_sync();   // barriers and tensor-map prefetch overlap the previous kernel; TMEM and all global reads wait for it
     if (warp == 2) ptx::tmem_alloc(tmem_ptr, 512);
     ptx::tc_fence_before();
     __syncthreads();
@@ -570,7 +541,6 @@ similarity_tc2_kernel(const __grid_constant__ CUtensorMap tmAl_hi, const __grid_
         const int quarter = warp & 3;
         const int gtid = threadIdx.x - 128 - grp_id * 128;
         float* x2 = x2s + grp_id * kTcMaxN;
-        const float4* x2v = reinterpret_cast<const float4*>(x2);
         int it = 0;
         Tc2Job job;
         for (int p = 0; tc2_phase(prm, cta, p, lanes_l, n_local_ctas, grid, job); ++p) {
@@ -591,7 +561,7 @@ similarity_tc2_kernel(const __grid_constant__ CUtensorMap tmAl_hi, const __grid_
                 const uint32_t taddr = tmem_base + (uint32_t)grp_id * kTcMaxN + ((uint32_t)(quarter * 32) << 16);
                 ptx::mbar_wait(&tmem_full[grp_id], acc_phase);
                 ptx::tc_fence_after();
-                tc_epilogue_tile<KT, EPI>(prm, t, taddr, x2, x2v, quarter, lane);
+                tc_epilogue_tile<KT>(prm, t, taddr, x2, quarter, lane);
                 ptx::tc_fence_before();
                 __syncwarp();
                 if (lane == 0) ptx::mbar_arrive(&tmem_empty[grp_id]);
@@ -700,13 +670,9 @@ static Tc2Plan plan_tc2(const TcParams& prm, int nterms, int sms) {
     // one CTA per global prototype tile beside the local CTAs (lanes = image-group walkers per prototype tile).
     // Measured on B200 (profiles/r1b_sim_plan_ab.txt): giving the local walkers all 148 SMs and dealing the global
     // tiles out as second jobs (9 lanes instead of 8 at the CUB shape) is 1.5-1.7x SLOWER at every batch size, so
-    // the dedicated plan stays; PPH_SIM_SHARED=1 / PPH_SIM_LANES=n select the alternatives for measurements.
-    const int knob_lanes = option(kOptSimLanes);
-    const bool knob_shared = option(kOptSimShared) != 0;
-    int avail = sms;
-    if (!knob_shared) avail = sms - (prm.MT_g <= sms / 4 ? prm.MT_g : sms / 4);
+    // the dedicated plan stays.
+    const int avail = sms - (prm.MT_g <= sms / 4 ? prm.MT_g : sms / 4);
     int lanes = avail / prm.MT_l;
-    if (knob_lanes > 0) lanes = knob_lanes;
     if (lanes < 1) lanes = 1;
     if (lanes > prm.NG_l) lanes = prm.NG_l;
     pl.lanes_l = lanes;
@@ -748,9 +714,9 @@ static void tc_shape_plan(bool x3, int B, int K, int D, int P, int Pg, int sms, 
     }
 }
 
-template <int NTERMS, int KT, int EPI = 1>
+template <int NTERMS, int KT>
 static int launch_tc2(const CUtensorMap* maps, const TcParams& prm, const Tc2Plan& pl, cudaStream_t st) {
-    auto kern = similarity_tc2_kernel<NTERMS, KT, EPI>;
+    auto kern = similarity_tc2_kernel<NTERMS, KT>;
     {   // per call, not cached in a static: the attribute is per device and setting it is cheap
         cudaError_t e = opt_in_smem(kern, kTcSmemLimit);
         if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return (int)e; }
@@ -817,10 +783,6 @@ int similarity_fwd_tc(int mode, int act_fn, float eps, int B, int K, int D, int 
         if (pl.ok) return x3 ? launch_tc2<3, KT>(maps, prm, pl, st) : launch_tc2<1, KT>(maps, prm, pl, st); \
         return x3 ? launch_tc<3, KT>(maps, prm, grid, st) : launch_tc<1, KT>(maps, prm, grid, st);   \
     } while (0)
-    // A/B switch for measurements: PPH_SIM_EPI=0 selects the sequential-scan epilogue (built for K = 81 only)
-    const bool old_epi = option(kOptSimEpi) == 0;
-    if (old_epi && K == 81 && pl.ok)
-        return x3 ? launch_tc2<3, 81, 0>(maps, prm, pl, st) : launch_tc2<1, 81, 0>(maps, prm, pl, st);
     switch (K) {
         case 49: PPH_TC_DISPATCH(49);
         case 64: PPH_TC_DISPATCH(64);

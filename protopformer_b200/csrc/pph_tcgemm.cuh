@@ -99,7 +99,6 @@ tcgemm_kernel(int M, int N, int Kd, int BN, int k_per_split, AOp a_op, BOp b_op,
         ptx::mbar_init(acc_done, 1);
         ptx::fence_mbar_init();
     }
-    pdl_sync();   // everything below reads global memory or allocates TMEM: wait for the prerequisite grids
     if (warp == 1) ptx::tmem_alloc(tmem_ptr, 256);
     if (tid >= 128 && tid < 256) {
         void* p3[3] = {nullptr, nullptr, nullptr};

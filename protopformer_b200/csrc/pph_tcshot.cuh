@@ -80,7 +80,6 @@ tcshot_kernel(int M, int N, int Kd, int BN, int k_per_split, unsigned int* sync_
         ptx::mbar_init(acc_done, 1);
         ptx::fence_mbar_init();
     }
-    pdl_sync();
     if (warp == 1) ptx::tmem_alloc(tmem_ptr, 128);
     if (tid >= 128 && tid < 256) {
         void* p3[3] = {nullptr, nullptr, nullptr};

@@ -31,7 +31,7 @@ class GraphedHeadStep:
     def __init__(self, params: dict, cfg: ops.HeadConfig, B: int, N: int, C: int, m: int, n_slots: int = 1,
                  heads: int = 0, ppc_cov_coe: float = 0.1, ppc_mean_coe: float = 0.5, train: bool = True,
                  process_group=None, device=None, fused: bool = True, allreduce_in_graph: bool = False,
-                 schedule: int | None = None, use_ppc: bool = True, impl: str = "auto", variants=None,
+                 use_ppc: bool = True, impl: str = "auto", variants=None,
                  exchange: str = "nccl", token_dtype=torch.float32):
         """params: dict with Wa (D,Din), ba (D), P (P,D), Pg (Pg,D) [leaf tensors, requires_grad in training] and
         the last layers Wl (C,P), Wg (C,Pg), frozen as in the reference unless their requires_grad is set: a training step
@@ -87,8 +87,8 @@ class GraphedHeadStep:
             cls = ops.FusedHeadStep if impl == "v2" else ops.FusedHeadStepV1
             kw = dict(variants=variants) if impl == "v2" else {}
             self.fused = cls(cfg, B, N, Din, D, P, Pg, C, m, dev, heads=heads, ppc_cov_coe=ppc_cov_coe,
-                             ppc_mean_coe=ppc_mean_coe, train=train, use_ppc=use_ppc, schedule=schedule,
-                             token_dtype=token_dtype, **kw)
+                             ppc_mean_coe=ppc_mean_coe, train=train, use_ppc=use_ppc, token_dtype=token_dtype,
+                             **kw)
             if train:
                 self.grads = dict(zip((n for n, _ in self.reducer.named), self.reducer.views))
 

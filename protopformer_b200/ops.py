@@ -613,17 +613,9 @@ class FusedHeadStepV1:
     grad: pph_last_layer_wgrad right after the loss tail)."""
 
     def __init__(self, cfg: HeadConfig, B, N, Din, D, P, Pg, C, m, device, heads: int = 0, ppc_cov_coe: float = 0.1,
-                 ppc_mean_coe: float = 0.5, train: bool = True, use_ppc: bool = True, schedule: int | None = None,
-                 token_dtype=torch.float32):
-        import os
+                 ppc_mean_coe: float = 0.5, train: bool = True, use_ppc: bool = True, token_dtype=torch.float32):
         token_entry("", token_dtype)
         self.cfg, self.train, self.use_ppc, self.token_dtype = cfg, train, use_ppc, token_dtype
-        # stream schedule of the training step: 1 (default) = three streams (token bins on their own branch, the
-        # cross-entropy tail does not wait for the PPC loss: the weighted sum is a separate 1-thread kernel on the
-        # side branch, PPC gradient buffer cleared at the start of the step); 0 = the first round-1 schedule, two
-        # streams (PPC loss, token bins and PPC backward in one side chain; the loss tail joins the PPC forward).
-        # Measured (profiles/r1b_ab_variants.txt): 187.6 -> 171.8 us per step at the CUB shape, B = 64.
-        self.schedule = int(os.environ.get("PPH_SCHEDULE", "1")) if schedule is None else int(schedule)
         self.dims = (B, N, Din, D, P, Pg, C, m, heads)
         self.cov_coe, self.mean_coe = float(ppc_cov_coe), float(ppc_mean_coe)
         K = cfg.K
@@ -668,12 +660,16 @@ class FusedHeadStepV1:
         c = _lib.call
         tok = _step_token_entries(self, tokens, Wa, ba, P, Pg, Wl, Wg)
         main, side, ev = torch.cuda.current_stream(), self.side, self.ev
-        sched1 = self.schedule == 1 and self.use_ppc and self.train
+        # Three streams while training with the PPC loss: the token bins run on their own branch, and the cross-entropy
+        # tail does not wait for the PPC loss (their weighted sum is a separate 1-thread kernel on the side branch).
+        # Measured against a two-stream order (profiles/r1b_ab_variants.txt): 187.6 -> 171.8 us per step at the CUB
+        # shape, B = 64.
+        ppc = self.use_ppc and self.train
         # branch: prototype operand preparation || selection + add-on
         ev[0].record(main)
         side.wait_event(ev[0])
         with torch.cuda.stream(side):
-            if sched1:
+            if ppc:
                 self.dP_ppc.zero_()
             c("pph_split_rows", P, Pn, D, float(cfg.center), self.P_hi, self.P_lo, self.p2, self.p2_ctr, self.p2_hi)
             c("pph_split_rows", Pg, Pgn, D, float(cfg.center), self.Pg_hi, self.Pg_lo, self.pg2, self.pg2_ctr, self.pg2_hi)
@@ -683,7 +679,6 @@ class FusedHeadStepV1:
           float(cfg.center), self.z2s_ctr, self.z2c_ctr, self.z2s_hi, self.z2c_hi, self.Zs_hi, self.Zs_lo,
           self.Zc_hi, self.Zc_lo)
         main.wait_event(ev[1])
-        ppc = self.use_ppc and self.train
         mode = cfg.mode_id
         sel = {_lib.MODE_FP32_FMA: 0, _lib.MODE_BF16X3: 1, _lib.MODE_BF16: 2}[mode]
         c("pph_similarity_fwd", mode, cfg.act_id, float(cfg.eps), B, K, D, Pn, Pgn, self.Zs, self.Zc,
@@ -693,12 +688,6 @@ class FusedHeadStepV1:
           self.P_hi, self.P_lo, self.Pg_hi, self.Pg_lo,
           self.dmin_l, self.argmin, self.act_l, self.dmin_g, self.act_g, None, None)
 
-        def ppc_bwd_side():
-            c("pph_ppc_bwd", self.Zs, P, self.idx32, labels, self.dslice, self.stats, None,
-              self.cov_coe * float(upstream), self.mean_coe * float(upstream), B, K, D, Pn, m, N, cfg.act_id,
-              float(cfg.eps), float(cfg.ppc_cov_thresh), float(cfg.ppc_mean_thresh), 0, self.dZs_ppc,
-              self.dP_ppc)
-
         if ppc:   # branch: PPC loss || last layers (forked after the persistent similarity kernel so it cannot delay it)
             ev[2].record(main)
             side.wait_event(ev[2])
@@ -706,38 +695,28 @@ class FusedHeadStepV1:
                 c("pph_ppc_fwd", self.Zs, self.z2s, P, self.p2, self.idx32, labels, B, K, D, Pn, m, N, cfg.act_id,
                   float(cfg.eps), float(cfg.ppc_cov_thresh), float(cfg.ppc_mean_thresh), self.dslice, self.stats,
                   self.ppc_partial, self.ppc_counter, self.ppc_losses)
-                ev[3].record(side)
-                if sched1:
-                    ppc_bwd_side()
-                elif self.train:   # the token bins of the backward only need argmin: off the critical path
-                    c("pph_similarity_bwd", None, None, self.argmin, None, None, None, None, B, K, D, Pn, Pgn, self.ws,
-                      1, None, None, None, None, None, None)
-                    # ... and the PPC backward only needs the PPC forward: its contributions go to side buffers that
-                    # the gradient kernel adds while it writes dZs / dP
-                    self.dP_ppc.zero_()
-                    ppc_bwd_side()
-                    ev[4].record(side)
-            if sched1:   # token bins on a third branch
-                self.side2.wait_event(ev[2])
-                with torch.cuda.stream(self.side2):
-                    c("pph_similarity_bwd", None, None, self.argmin, None, None, None, None, B, K, D, Pn, Pgn, self.ws,
-                      1, None, None, None, None, None, None)
-                    ev[7].record(self.side2)
+                # the PPC backward only needs the PPC forward: its contributions go to side buffers that the gradient
+                # kernel adds while it writes dZs / dP
+                c("pph_ppc_bwd", self.Zs, P, self.idx32, labels, self.dslice, self.stats, None,
+                  self.cov_coe * float(upstream), self.mean_coe * float(upstream), B, K, D, Pn, m, N, cfg.act_id,
+                  float(cfg.eps), float(cfg.ppc_cov_thresh), float(cfg.ppc_mean_thresh), 0, self.dZs_ppc,
+                  self.dP_ppc)
+            # the token bins of the backward only need argmin: off the critical path, on a third branch
+            self.side2.wait_event(ev[2])
+            with torch.cuda.stream(self.side2):
+                c("pph_similarity_bwd", None, None, self.argmin, None, None, None, None, B, K, D, Pn, Pgn, self.ws,
+                  1, None, None, None, None, None, None)
+                ev[7].record(self.side2)
         c("pph_logits_fwd", self.act_l, self.act_g, Wl, Wg, B, Pn, Pgn, C, float(cfg.global_coe), self.logits,
           self.logits_g, self.logits_l)
-        if sched1:
-            c("pph_loss_tail", self.logits, labels, None, self.cov_coe, self.mean_coe, float(upstream), B, C,
-              self.ce_partial, self.ce_counter, self.losses_ce, self.dlogits)
+        c("pph_loss_tail", self.logits, labels, None, self.cov_coe, self.mean_coe, float(upstream), B, C,
+          self.ce_partial, self.ce_counter, self.losses_ce if ppc else self.losses, self.dlogits if self.train else None)
+        if ppc:
             ev[8].record(main)
             side.wait_event(ev[8])
             with torch.cuda.stream(side):
                 c("pph_loss_combine", self.losses_ce, self.ppc_losses, self.cov_coe, self.mean_coe, self.losses)
                 ev[4].record(side)
-        else:
-            if ppc:
-                main.wait_event(ev[3])
-            c("pph_loss_tail", self.logits, labels, self.ppc_losses if ppc else None, self.cov_coe, self.mean_coe,
-              float(upstream), B, C, self.ce_partial, self.ce_counter, self.losses, self.dlogits if self.train else None)
         if not self.train:
             return self.losses
         dWl, dWg = _last_layer_grad_targets(self.train, Wl, Wg, grads)
@@ -746,13 +725,11 @@ class FusedHeadStepV1:
               float(cfg.global_coe), dWl, dWg)
         c("pph_logits_bwd", self.dlogits, None, None, Wl, Wg, self.dmin_l, self.dmin_g, B, Pn, Pgn, C,
           float(cfg.global_coe), cfg.act_id, float(cfg.eps), self.g_l, self.g_g)
-        binned = ppc                                   # bins were produced on a side stream next to the PPC loss
-        if binned:
+        if ppc:                                        # bins were produced on a side branch next to the PPC loss
             main.wait_event(ev[4])
-            if sched1:
-                main.wait_event(ev[7])
+            main.wait_event(ev[7])
         c("pph_similarity_bwd", self.g_l, self.g_g, self.argmin, self.Zs, self.Zc, P, Pg, B, K, D, Pn, Pgn, self.ws,
-          2 if binned else 3, self.dZs_ppc if ppc else None, self.dP_ppc if ppc else None,
+          2 if ppc else 3, self.dZs_ppc if ppc else None, self.dP_ppc if ppc else None,
           self.dZs, self.dZc, grads["P"], grads["Pg"])
         # weight gradient || token gradient (independent GEMMs, 82 + 41 CTAs: they share the machine)
         ev[5].record(main)
@@ -814,7 +791,7 @@ class FusedHeadStep:
     grad; with both frozen, the default, the step is exactly the 11 launches above).  Reference: tools/engine_proto.py:49-76."""
 
     def __init__(self, cfg: HeadConfig, B, N, Din, D, P, Pg, C, m, device, heads: int = 0, ppc_cov_coe: float = 0.1,
-                 ppc_mean_coe: float = 0.5, train: bool = True, use_ppc: bool = True, schedule=None, variants=None,
+                 ppc_mean_coe: float = 0.5, train: bool = True, use_ppc: bool = True, variants=None,
                  token_dtype=torch.float32):
         token_entry("", token_dtype)
         if not fused_step_supported(B, N, Din, D, cfg.K, P, Pg, C, m, token_dtype):

@@ -15,8 +15,6 @@ case $stage in
     echo "== $k: rc=$? $(tail -1 gpurun_out/t_$k.log)" ;;
   times64)
     timeout 300 python scripts/step_times.py cub_b64 fp32 > gpurun_out/times_b64.json 2> gpurun_out/times_b64.err; tail -c 1500 gpurun_out/times_b64.json ;;
-  times64pdl)
-    PPH_PDL=1 timeout 300 python scripts/step_times.py cub_b64 fp32 > gpurun_out/times_b64_pdl.json 2> gpurun_out/times_b64_pdl.err; tail -c 1500 gpurun_out/times_b64_pdl.json ;;
   timeline)
     timeout 300 python scripts/timeline.py cub_b64 fp32 v2 > gpurun_out/timeline_v2.txt 2> gpurun_out/timeline_v2.err; tail -40 gpurun_out/timeline_v2.txt; tail -3 gpurun_out/timeline_v2.err
     timeout 300 python scripts/timeline.py cub_b64 fp32 v1 > gpurun_out/timeline_v1.txt 2> gpurun_out/timeline_v1.err ;;
@@ -64,9 +62,6 @@ case $stage in
     timeout 240 python -m torch.distributed.run --nnodes=1 --nproc-per-node $n --master-addr 127.0.0.1 --master-port 29512 \
         bench.py --gpus $n --steps 1000 --warmup 50 --no-extras --exchange nccl > gpurun_out/bench_n${n}_nccl.json 2> gpurun_out/bench_n${n}_nccl.err
     echo "== nccl rc=$?"; tail -c 1200 gpurun_out/bench_n${n}_nccl.json; tail -3 gpurun_out/bench_n${n}_nccl.err ;;
-  variants)   # A/B of the two variant switches: rollout normalisation (PPH_ROLLOUT=3) and staged class maps (PPH_CLASSMAP=2)
-    for v in 0 2; do echo "PPH_ROLLOUT=$v"; PPH_ROLLOUT=$v timeout 200 python scripts/rollout_bench.py "11,64,3,197;11,64,6,197" 2>&1 | cut -c1-160 | tail -2; done
-    for v in 1 2; do echo "PPH_CLASSMAP=$v"; PPH_CLASSMAP=$v timeout 200 python scripts/next_rows_bench.py 2>&1 | grep class_maps | cut -c1-200; done ;;
   e2e)
     for e in "" nocopy norows nod2h "nocopy,nosel" "nocopy,nosel,norows"; do EXP=$e timeout 200 python scripts/e2e_timeline.py 32 2 2>&1 | grep "^#"; done
     EXP=nocopy PPH_TIMELINE=1 timeout 200 python scripts/e2e_timeline.py 32 2 2>&1 | grep -v Warn | tail -30 ;;
@@ -75,9 +70,6 @@ case $stage in
   rollout)
     timeout 300 python -m pytest tests/test_rollout_gpu.py -q -m gpu --tb=short 2>&1 | tail -2
     timeout 200 python scripts/rollout_bench.py 2>&1 | cut -c1-150 | tail -4 ;;
-  pdlbench)
-    for v in 0 1; do echo "PPH_PDL=$v"; PPH_PDL=$v timeout 200 python bench.py --no-extras --no-cpu --steps 2000 --warmup 100 2>/dev/null | python -c "import sys,json; d=json.loads(sys.stdin.read().strip().splitlines()[-1]); print('value %.0f (%.1f us) e2e %.0f'%(d['value'],1e3*d['ms_per_step'],d['e2e']['value']))"; done
-    echo "bf16"; timeout 200 python bench.py --mode bf16 --no-extras --no-cpu 2>/dev/null | python -c "import sys,json; d=json.loads(sys.stdin.read().strip().splitlines()[-1]); print('value %.0f (%.1f us) e2e %.0f'%(d['value'],1e3*d['ms_per_step'],d['e2e']['value']))" ;;
   dogscheck)
     timeout 300 python bench.py --workload dogs_b256_eval --steps 200 --warmup 10 --no-extras 2> gpurun_out/dogs.err | python -c "import sys,json; d=json.loads(sys.stdin.read().strip().splitlines()[-1]); print('value %.0f (%.1f us) e2e %.0f'%(d['value'],1e3*d['ms_per_step'],d['e2e']['value']), d['oracle_check'], d['cpu_baseline'] and d['cpu_baseline']['value'])"; tail -2 gpurun_out/dogs.err ;;
   racecheck)  # shared-memory hazard check of the fused selection + add-on forward kernel and the dense PPC kernels (small shapes)
@@ -91,11 +83,7 @@ case $stage in
   execswitch)
     timeout 300 python scripts/exec_switch.py 2>&1 | tail -4 ;;
   gatherparts)
-    for v in 0 1; do echo "PPH_GATHER=$v"; PPH_GATHER=$v timeout 200 python scripts/gather_parts.py 2>&1 | tail -5; done ;;
-  bulktests)  # the sparse-backward tests with the bulk-copy gather selected
-    PPH_GATHER=1 timeout 600 python -m pytest tests/test_gpu_parity.py tests/test_step2_gpu.py tests/test_fused_step_gpu.py -q -m gpu --tb=short \
-        -k "bwd or backward or train_step or benchmarked or variants or fixture or reproducible" > gpurun_out/t_bulk.log 2>&1
-    echo "== bulktests rc=$? $(tail -1 gpurun_out/t_bulk.log)" ;;
+    timeout 200 python scripts/gather_parts.py 2>&1 | tail -5 ;;
   hostgather)
     timeout 200 python scripts/host_gather_times.py 2>&1 | tail -12 ;;
   mgtest)     # multi-GPU pytest group (gpurun --gpus 2)

@@ -102,16 +102,3 @@ def test_class_maps_full_size_against_materialised_map():
     _, act_map = ops.materialize_maps(cfg, tf, d["P"], d["Pg"])                    # (B,P,K) from the FP32-FMA kernel
     want = O.class_activation_maps(act_map.cpu(), idx.cpu().long(), case["labels"], shape.m, shape.N)
     assert rel_close(maps.flatten(2).cpu(), want, 1e-4), max_rel(maps.flatten(2).cpu(), want)
-
-
-@pytest.mark.gpu
-def test_class_maps_first_kernel_in_subprocess():
-    """The default is the staged-operand kernel; PPH_CLASSMAP=1 selects the first kernel (kept for A/B and for shapes whose
-    rows do not fit shared memory), read once per process -> run the same tests in a child."""
-    import os
-    import subprocess
-    import sys
-    env = dict(os.environ, PPH_CLASSMAP="1")
-    r = subprocess.run([sys.executable, "-m", "pytest", __file__, "-q", "-m", "gpu", "-x", "-k", "not subprocess"], env=env, capture_output=True,
-                       text=True, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert r.returncode == 0, r.stdout[-3000:]

@@ -33,7 +33,7 @@ def test_library_builds_loads_and_exports_every_declared_symbol():
         assert name in _lib.SIGNATURES, f"{name} has no ctypes signature"
         assert len(_lib.SIGNATURES[name]) == nargs, f"{name}: header has {nargs} args, binding {len(_lib.SIGNATURES[name])}"
     assert set(_lib.SIGNATURES) == set(decl)
-    assert lib.pph_version() == 202
+    assert lib.pph_version() == 203
 
 
 def test_sass_contains_blackwell_tensor_and_tma_instructions():
@@ -319,5 +319,7 @@ def test_round2_entry_points_validate_arguments_before_touching_the_device():
                                     None, None, None, None, None, None, None, None, None, None) == -1
     assert lib.pph_head_mid(*([None] * 8), 1, 81, 192, 2000, 2000, 200, 10, 196, 0.5, 0, 1e-4, 1.0, 1, 1, *([None] * 5),
                             1.0, 2.0, 0.1, 0.5, *([None] * 14)) == -1
-    assert lib.pph_set_option(b"no_such_option", 1) == -1 and lib.pph_set_option(b"pdl", 0) == 0
-    assert b"pph_" in lib.pph_last_error_string() or len(lib.pph_last_error_string()) > 0
+    assert lib.pph_rollout_ws_bytes(1, 1, 2, 0, None) == -1
+    assert b"pph_rollout_ws_bytes" in lib.pph_last_error_string()
+    # kernel choice is left to the shapes alone: no run-time switch is exported
+    assert not hasattr(lib, "pph_set_option")

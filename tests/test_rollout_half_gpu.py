@@ -4,9 +4,6 @@ Every half-precision value is exact in fp32, so the twins must give, bit for bit
 widened maps -- the result the rollout had on half maps when it made an fp32 copy of every layer first -- and must hold
 the oracle's bar on those widened maps."""
 import ctypes
-import os
-import subprocess
-import sys
 
 import pytest
 import torch
@@ -120,7 +117,7 @@ def test_half_maps_discard_ratios_start_row_and_odd_base_address(dt):
     v0 = torch.rand(3, 197, generator=torch.Generator().manual_seed(1))
     got = _assert_same_as_widened(maps, v0=v0.to(DEV), drop_first=False)
     assert rel_close(got.cpu(), R.rollout_cls_row(wide, v0=v0, drop_first=False), 1e-5, 1e-9)
-    for ratio in (0.0, 0.5, 1.0):
+    for ratio in (0.0, 0.2, 0.5, 1.0):           # 0.0 and 0.2: entry lists too long for the staged chain kernel
         got = _assert_same_as_widened(maps, discard_ratio=ratio, drop_first=False)
         assert rel_close(got.cpu(), R.rollout_cls_row(wide, ratio, "mean", drop_first=False), 1e-5, 1e-9), ratio
     # maps whose storage starts 2 bytes past a 4-byte boundary (a view at an odd element offset)
@@ -266,15 +263,3 @@ def test_backbone_loops_with_half_maps(dt):
             cait, cls_embed, x_embed, None, [(1, 16)],
             rollout_cait=lambda a, pre: ops.rollout_scores_cait(_widened(a), pre))
     assert torch.equal(score, score2) and torch.equal(x, x2)
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("variant", ["1", "2"])
-def test_half_maps_under_the_other_kernel_versions_in_subprocess(variant):
-    """PPH_ROLLOUT is read once per process: 1 runs the first version of the kernels, 2 the exact-division
-    normalisation (the default is one reciprocal per row)."""
-    env = dict(os.environ, PPH_ROLLOUT=variant)
-    r = subprocess.run([sys.executable, "-m", "pytest", __file__, "-q", "-m", "gpu", "-x", "-k", "not subprocess"],
-                       env=env, capture_output=True, text=True,
-                       cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    assert r.returncode == 0, r.stdout[-3000:]
